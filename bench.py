@@ -347,6 +347,7 @@ def wide_leg(ctx, D, key, steps, warmup, profile, e2e, sampler=None):
     D.barrier()
     dev_ms = D.max(e0.elapsed_time(e1))
     gpu_launches = ctx.launches - launches0
+    last = res[:2].cpu().numpy()        # what the last timed step returned, before the passes below overwrite `res`
     z_total = float(res[1].item())
     entries_rank = plan.union_entries
     entries_all = D.sum(entries_rank)
@@ -354,10 +355,11 @@ def wide_leg(ctx, D, key, steps, warmup, profile, e2e, sampler=None):
            "width_per_rank": width, "shard_vars": shard_vars, "n_launches": plan.n_launches,
            "entries_per_rank": entries_rank, "entries_all_ranks": entries_all, "entries_unsharded": full_entries,
            "redundant_work": entries_all / full_entries if full_entries else None,
-           "ms_per_step": dev_ms / steps, "value": entries_all * steps / (dev_ms / 1e3),
+           "steps": steps, "ms_per_step": dev_ms / steps, "value": entries_all * steps / (dev_ms / 1e3),
            "useful_value": full_entries * steps / (dev_ms / 1e3),
            "gpu_launches": gpu_launches, "Z": z_total, "Z_rank": z_local, "bytes_per_step": plan.bytes,
-           "peak_intermediate_GB": plan.peak_bytes / 1e9, "max_step_entries": plan.max_step_entries}
+           "peak_intermediate_GB": plan.peak_bytes / 1e9, "max_step_entries": plan.max_step_entries,
+           "outputs": {"result": last[:1], "partition": last[1:]}}
 
     # golden: the reference's own numbers (oracle/make_wide_golden.py), total and per slab
     gold = load_wide_golden().get("8" if key == "strong" else str(key))
@@ -481,6 +483,7 @@ def config5_leg(ctx, D, nsets, steps, warmup, cpu_arm):
         z = bn.partition_batch(observed, dev, "mf")
     e1.record(s)
     D.barrier()
+    z_last = z.cpu().numpy()            # `z` is the model's result buffer: the calls below write it again
     ms = D.max(e0.elapsed_time(e1)) / steps
     launches = (ctx.launches - l0) // steps
     plan = [p for k_, p in bn._plans.items()][0]
@@ -532,7 +535,7 @@ def config5_leg(ctx, D, nsets, steps, warmup, cpu_arm):
             "gpu_launches_per_batch": launches, "union_entries_per_s": plan.union_entries * nsets / ms * 1e3,
             "kernel": ("ve_fused: one launch, %d lanes per evidence set, %d doubles of shared memory per set, %d steps"
                        % (lanes, arena, n_steps)) if lanes else "contract_batched: one launch per bucket",
-            "sample_Z": z0, "cpu_baseline": cpu}
+            "sample_Z": z0, "cpu_baseline": cpu, "outputs": {"z": z_last}}
 
 
 def same_sample_leg(ctx, sample, steps):
@@ -564,7 +567,7 @@ def same_sample_leg(ctx, sample, steps):
     e2e_ms = (time.perf_counter() - t0) * 1e3 / steps
     ent = plan_entries = union_entries(bn.scopes, order)
     bn.close()
-    return {"sample_network": list(sample), "width": width, "entries": ent, "ms_per_query": ms, "value": plan_entries / ms * 1e3,
+    return {"sample_network": list(sample), "width": width, "entries": ent, "steps": steps, "ms_per_query": ms, "value": plan_entries / ms * 1e3,
             "unit": UNIT, "e2e": {"value": ent / e2e_ms * 1e3, "ms_per_query": e2e_ms}, "Z": z,
             "note": "L2-resident at this size (the tables are MBs): a same-config ratio against the reference arm, not a roofline number"}
 
@@ -614,7 +617,12 @@ def main():
     ap.add_argument("--no-config5", action="store_true", help="skip the PR-queries/sec legs (config 5)")
     ap.add_argument("--no-extra", action="store_true", help="skip the N = 1 legs shapes / configs_1_3 / multivalued / same_sample")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling leg (width-30 network)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each leg returned as DIR/<name>.npy (float64; at N > 1, rank "
+                         "0's): the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     D = Dist()
     sample = pick_cpu_sample(args.steps, args.warmup)
 
@@ -634,6 +642,7 @@ def main():
         print(json.dumps(line))
         return 0
 
+    import numpy as np
     import torch
     import torch.distributed as dist
     from bnpp_b200 import capi
@@ -654,7 +663,7 @@ def main():
     strong = None
     if not args.no_strong:
         try:
-            strong = wide_leg(ctx, D, "strong", max(2, args.steps // 2), 2, profile=False, e2e=False)
+            strong = wide_leg(ctx, D, "strong", args.steps, 2, profile=False, e2e=False)
             strong.pop("per_launch", None)
         except Exception as e:
             strong = {"error": "%s: %s" % (type(e).__name__, e)}
@@ -673,6 +682,15 @@ def main():
         if D.world > 1:
             dist.destroy_process_group()
         return 0
+
+    outputs = {"wide_" + k: v for k, v in weak.pop("outputs").items()}
+    outputs.update({"strong_" + k: v for k, v in (strong or {}).pop("outputs", {}).items()})
+    for nsets, leg in (config5 or {}).items():
+        outputs.update({"pr_queries_%s_%s" % (nsets, k): v for k, v in leg.pop("outputs", {}).items()})
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(arr, dtype=np.float64))
 
     # ---- roofline of the dominant kernel: the widest fused launch ---------------------------------
     peak, peak_kind = peaks()
@@ -709,9 +727,9 @@ def main():
     extra = {}
     if n_gpus == 1 and not args.no_extra:
         sys.path.insert(0, os.path.join(ROOT, "tools"))
-        for name, fn in (("same_sample", lambda: same_sample_leg(ctx, sample, max(3, args.steps))),
+        for name, fn in (("same_sample", lambda: same_sample_leg(ctx, sample, args.steps)),
                          ("multivalued", lambda: multivalued_leg(ctx)),
-                         ("configs_1_3", lambda: __import__("config_bench").run(ctx, reps=30)),
+                         ("configs_1_3", lambda: dict(__import__("config_bench").run(ctx, reps=30), reps=30)),
                          ("shapes", lambda: shapes_leg(ctx, peak))):
             try:
                 extra[name] = fn()
@@ -760,7 +778,7 @@ def shapes_leg(ctx, peak):
     rows = sb.run_binary(ctx, 28, 3, verbose=False, peak=peak)
     rows += sb.run_mixed(ctx, 3, verbose=False, peak=peak)
     rows += sb.run_mv(ctx, [3, 4, 5, 7, 8], 3, verbose=False, peak=peak)
-    return {"peak_GBs": peak, "rows": rows, "min_frac": min(r["frac"] for r in rows),
+    return {"peak_GBs": peak, "iters_per_row": 3, "rows": rows, "min_frac": min(r["frac"] for r in rows),
             "rows_below_0.70": [dict(kind=r["kind"], k=r["k"], frac=r["frac"], kernel=r["kernel"]) for r in rows if r["frac"] < 0.70]}
 
 

@@ -173,7 +173,7 @@ def orders():
     dump("orders.json", out, compress=True)
 
 
-# ---------------------------------------------------------------- ops.json
+# ---------------------------------------------------------------- ops_1.json, ops_2.json
 def rand_scope(rng, nvars, w):
     return rng.sample(range(nvars), w)
 
@@ -207,7 +207,8 @@ def ops():
         for nm, (scope, size, z, vals) in zip(names, facs):
             rec[nm] = {"scope": scope, "partition": z, "values": vals.tolist()}
         cases.append(rec)
-    dump("ops.json", cases, compress=True)
+    for i in range(2):                     # two halves: each file stays under 1 MB
+        dump("ops_%d.json" % (i + 1), cases[i * 80:(i + 1) * 80], compress=True)
 
 
 # ---------------------------------------------------------------- synthetic.json
@@ -267,8 +268,34 @@ def synthetic():
     dump("synthetic.json", out, compress=True)
 
 
+# ---------------------------------------------------------------- cli.json
+def cli():
+    """stdout of the reference's own `bn` / `mn` (oracle/_ref) on the command lines of
+    tests/test_gpu_host.py:cli_cases, `Executed in` and the directory of the input files masked"""
+    import pathlib
+    import subprocess
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_gpu_host import cli_cases, mask
+    with gzip.open(os.path.join(OUT, "models.json.gz"), "rt") as f:
+        golden_models = json.load(f)
+    d = pathlib.Path(TMP) / "cli"
+    d.mkdir(parents=True, exist_ok=True)
+    cases = []
+    for exe, args, stdin in cli_cases(d, golden_models):
+        p = subprocess.run([os.path.join(HERE, "_ref", exe)] + args, input=stdin, capture_output=True, text=True,
+                           timeout=300)
+        cases.append({"argv": [exe] + [mask(a, d) for a in args], "stdin": stdin, "returncode": p.returncode,
+                      "stdout": mask(p.stdout, d)})
+    with open(os.path.join(OUT, "cli.json"), "w") as f:
+        json.dump({"source": "stdout of the reference's bn / mn on the `make check` command lines (code/Makefile:47-56), "
+                             "written by `python oracle/make_golden.py cli`; `Executed in` and the directory of the input "
+                             "files masked", "cases": cases}, f, indent=1)
+        f.write("\n")
+    print("wrote cli.json", len(cases))
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
-    which = sys.argv[1:] or ["models", "orders", "ops", "synthetic"]
+    which = sys.argv[1:] or ["models", "orders", "ops", "synthetic", "cli"]
     for w in which:
         globals()[w]()

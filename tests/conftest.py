@@ -29,7 +29,7 @@ def golden_models():
 
 @pytest.fixture(scope="session")
 def golden_ops():
-    return load_golden("ops")
+    return load_golden("ops_1") + load_golden("ops_2")        # one list, stored in two halves of under 1 MB
 
 
 @pytest.fixture(scope="session")

@@ -3,8 +3,9 @@ mn CLIs) on top of the C ABI.
 
 `tests/bin/harness` (tests/harness/Makefile) is oracle/ref_harness.cpp -- the very source that drives the UNMODIFIED
 reference -- compiled against this repo's headers, so each test reads like a reference-side test:
-same commands, answers compared with the reference's (tests/golden, or oracle/_ref run side by side).
+same commands, answers compared with the reference's (tests/golden).
 """
+import json
 import math
 import os
 import re
@@ -137,26 +138,31 @@ def test_factor_ops_through_cpp_api(golden_ops):
         assert scal[2 * i] == c["max_p"] and math.isclose(scal[2 * i + 1], c["min_p"], rel_tol=1e-12)
 
 
-def mask(text):
+def mask(text, d=None):
     text = re.sub(r"Executed in [-+0-9.e]+ms", "Executed in Xms", text)
+    if d is not None:
+        text = text.replace(str(d), "<dir>")
     return text
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "bn")), reason="oracle/_ref not built")
-def test_cli_byte_compat(files, golden_models, tmp_path):
-    """the `make check` command lines of the reference (code/Makefile:47-56): same bytes on stdout,
-    `Executed in` masked.  Values print with 6-7 digits, where 1e-9 differences do not show."""
+def cli_cases(d, golden_models):
+    """the `make check` command lines of the reference (code/Makefile:47-56) as (exe, args, stdin), their
+    files written under `d`"""
+    files = {}
+    for name in ("asia", "cancer", "grid3x3"):
+        files[name] = str(d / (name + ".uai"))
+        (d / (name + ".uai")).write_text(golden_models[name]["uai"])
     m = golden_models["asia"]
-    evid = tmp_path / "asia.uai.evid"
+    evid = d / "asia.uai.evid"
     evid.write_text("1\n2 0 1 2 1")
-    ind = tmp_path / "asia.ind"
+    ind = d / "asia.ind"
     ind.write_text(m["ind"])
-    notind = tmp_path / "asia.not.ind"
+    notind = d / "asia.not.ind"
     notind.write_text(m["not_ind"])
     g = golden_models["grid3x3"]
-    gev = tmp_path / "g.evid"
+    gev = d / "g.evid"
     gev.write_text(g["shipped"]["PR_evid"])
-    cases = [
+    return [
         ("bn", [files["asia"], str(evid), "-pr"], ""),
         ("bn", [files["asia"], str(evid), "-pr", "-mf"], ""),
         ("bn", [files["asia"], str(evid), "-mar"], ""),
@@ -170,12 +176,21 @@ def test_cli_byte_compat(files, golden_models, tmp_path):
         ("bn", [files["asia"], "-v"], "width\nquit\n"),
         ("mn", [files["grid3x3"], str(gev)], "PR\nMAR\nquit\n"),
     ]
-    for exe, args, stdin in cases:
+
+
+def test_cli_byte_compat(golden_models, tmp_path):
+    """the `make check` command lines of the reference: same bytes on stdout as the unmodified reference
+    (tests/golden/cli.json), `Executed in` and the directory of the input files masked.  Values print with 6-7
+    digits, where 1e-9 differences do not show."""
+    with open(os.path.join(ROOT, "tests", "golden", "cli.json")) as f:
+        want = json.load(f)["cases"]
+    cases = cli_cases(tmp_path, golden_models)
+    assert len(cases) == len(want)
+    for (exe, args, stdin), ref in zip(cases, want):
+        assert [exe] + [mask(a, tmp_path) for a in args] == ref["argv"]
         ours = subprocess.run([os.path.join(BIN, exe)] + args, input=stdin, capture_output=True, text=True, timeout=300)
-        ref = subprocess.run([os.path.join(ROOT, "oracle", "_ref", exe)] + args, input=stdin, capture_output=True, text=True,
-                             timeout=300)
-        assert ours.returncode == ref.returncode, (exe, args, ours.stderr[-500:])
-        a, b = mask(ours.stdout), mask(ref.stdout)
+        assert ours.returncode == ref["returncode"], (exe, args, ours.stderr[-500:])
+        a, b = mask(ours.stdout, tmp_path), ref["stdout"]
         if "-v" in args:
             # unordered_set<const Variable*> print order is address-dependent in the reference: compare as multisets of lines
             assert sorted(a.splitlines()) == sorted(b.splitlines()) or len(a.splitlines()) == len(b.splitlines())
@@ -183,50 +198,47 @@ def test_cli_byte_compat(files, golden_models, tmp_path):
             assert a == b, (exe, args, a[:600], b[:600])
 
 
-MODELS = os.path.join(ROOT, "oracle", "_ref", "models")
-
-
-@pytest.mark.skipif(not os.path.isdir(MODELS) or not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "bn")),
-                    reason="oracle/_ref (reference binaries + shipped models) not built")
-def test_cli_all_shipped_networks_side_by_side():
-    """drop-in check on EVERY shipped Bayesian network: `bn <model> -pr -mf` (and -md / -wmf on the smaller
-    ones) prints the same partition line as the unmodified reference; the big multi-valued networks
-    (Link, Munin*, Barley, Mildew, Diabetes, pathfinder, Pigs) exercise the mixed-radix kernels end to end"""
-    import glob
+def test_cli_partition_lines_match_reference(files, golden_models):
+    """drop-in check on every shipped Bayesian network the golden fixtures carry: `bn <model> -pr -mf` (and -md / -wmf)
+    prints the same partition line as the unmodified reference (its value from tests/golden, printed as the reference
+    prints a double); the multi-valued networks (Water, andes, hepar2, ...) exercise the mixed-radix kernels end to end"""
     checked = 0
-    for path in sorted(glob.glob(os.path.join(MODELS, "bayesnets", "*.uai"))):
-        name = os.path.basename(path)
-        flags = [["-pr", "-mf"]]
-        if os.path.getsize(path) < 10000:
-            flags += [["-pr", "-md"], ["-pr", "-wmf"]]
-        for fl in flags:
-            try:
-                ref = subprocess.run([os.path.join(ROOT, "oracle", "_ref", "bn"), path] + fl, capture_output=True, text=True,
-                                     timeout=40)
-            except subprocess.TimeoutExpired:
-                ref = None       # Munin1: the reference needs minutes
-            ours = subprocess.run([os.path.join(BIN, "bn"), path] + fl, capture_output=True, text=True, timeout=300)
+    for name, m in sorted(golden_models.items()):
+        if m["uai"].split()[0] == "MARKOV":
+            continue
+        for case in m["pr"]:
+            if not case["flag"] or case["evidence"]:
+                continue
+            fl = ["-pr", "-" + case["flag"]]
+            ours = subprocess.run([os.path.join(BIN, "bn"), files[name]] + fl, capture_output=True, text=True, timeout=300)
             assert ours.returncode == 0, (name, fl, ours.stderr[-400:])
             line = ours.stdout.splitlines()[0]
-            assert line.startswith(">> Partition = ")
-            if ref is not None:
-                assert ref.stdout.splitlines()[0] == line, (name, fl, ref.stdout.splitlines()[0], line)
-                checked += 1
-    assert checked >= 22
+            assert line == ">> Partition = %g" % case["pr"], (name, fl, line, case["pr"])
+            checked += 1
+    assert checked >= 36
     # Markov net by VE (extension flags of `mn`): log10 Z of network.uai as shipped in network.uai.PR
-    net = os.path.join(MODELS, "markovnets", "network.uai")
-    out = subprocess.run([os.path.join(BIN, "mn"), net, os.path.join(MODELS, "markovnets", "network.uai.evid"), "-ve", "-mf"],
+    evid = os.path.join(os.path.dirname(files["network"]), "network.uai.evid")
+    with open(evid, "w") as f:
+        f.write(golden_models["network"]["shipped"]["evid"])
+    out = subprocess.run([os.path.join(BIN, "mn"), files["network"], evid, "-ve", "-mf"],
                          input="PR\nquit\n", capture_output=True, text=True, timeout=300)
     assert "Partition = 163.204" in out.stdout, out.stdout[-300:]
 
 
-def test_uai_solution_writers_round_trip(tmp_path):
+def test_uai_solution_writers_round_trip(tmp_path, golden_models):
     """SURVEY 8f row 3: `mn ... -o prefix` writes prefix.PR / prefix.MAR in the UAI solution format; token for token the
-    files shipped beside the reference's models (models/markovnets/grid3x3.uai.PR, grid3x3.uai.MAR, network.uai.PR and
-    network.uai.MAR -- the latter two through VE, the brute-force joint of 2^120 entries is out of reach)"""
-    mk = os.path.join(MODELS, "markovnets")
-    if not os.path.isdir(mk):
-        pytest.skip("oracle/_ref/models not present")
+    files shipped beside the reference's models (grid3x3.uai.PR, grid3x3.uai.MAR, network.uai.PR and network.uai.MAR,
+    kept in tests/golden -- the latter two through VE, the brute-force joint of 2^120 entries is out of reach)"""
+    mk = tmp_path / "markovnets"
+    mk.mkdir()
+    g, n = golden_models["grid3x3"], golden_models["network"]
+    for name, text in (("grid3x3.uai", g["uai"]), ("grid3x3-PR.uai.evid", g["shipped"]["PR_evid"]),
+                       ("grid3x3-MAR.uai.evid", g["shipped"]["MAR_evid"]), ("grid3x3.uai.PR", g["shipped"]["PR"]),
+                       ("grid3x3.uai.MAR", g["shipped"]["MAR"]), ("network.uai", n["uai"]),
+                       ("network.uai.evid", n["shipped"]["evid"]), ("network.uai.PR", n["shipped"]["PR"]),
+                       ("network.uai.MAR", n["shipped"]["MAR"])):
+        (mk / name).write_text(text)
+    mk = str(mk)
 
     def solve(model, evid, flags, command, suffix):
         prefix = str(tmp_path / (model + suffix))

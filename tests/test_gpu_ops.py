@@ -1,5 +1,5 @@
 """GPU parity tests proper: the CUDA path, called through the C ABI, against
-(1) per-op dumps of the unmodified reference (tests/golden/ops.json.gz) and
+(1) per-op dumps of the unmodified reference (tests/golden/ops_*.json.gz) and
 (2) the CPU oracle on seeded inputs.  Values are BIT-EXACT (same multiplication and
 summation order as the reference); partitions (tree-reduced on the GPU, sequential in
 the reference) agree to 1e-12 relative."""

@@ -155,7 +155,7 @@ def test_synthetic_bn_partition(golden_synth):
             assert math.isclose(z, case["pr"], rel_tol=1e-11)
 
 
-@pytest.mark.skipif(not orc.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
+@pytest.mark.skipif(not orc.have_ref(), reason="oracle/_ref not built (needs the reference's sources: make -C oracle ref REF=...)")
 def test_ref_harness_matches_fixture(golden_models):
     """the travelling binary still answers as when the fixtures were made"""
     import os, tempfile
