@@ -28,6 +28,7 @@ EXPORTS = [
     "bnpp_tuning_set", "bnpp_tuning_get", "bnpp_ve_plan_result_size", "bnpp_ve_plan_set_normalize",
     "bnpp_mar_plan_normalize", "bnpp_fg_reset", "bnpp_ve_plan_launches",
     "bnpp_sampler_create", "bnpp_sampler_destroy", "bnpp_sampler_logical", "bnpp_sampler_likelihood",
+    "bnpp_product_max_out", "bnpp_mpe_plan_create", "bnpp_mpe_plan_run",
 ]
 
 
@@ -85,6 +86,8 @@ def lib():
         L.bnpp_scope_size.argtypes = [ctypes.POINTER(Scope)]
         L.bnpp_product_sum_out.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(Operand), ctypes.POINTER(Scope),
                                            ctypes.c_int64, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
+        L.bnpp_product_max_out.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(Operand), ctypes.POINTER(Scope),
+                                           ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p]
         L.bnpp_product.argtypes = [ctypes.c_void_p, ctypes.POINTER(Scope), ctypes.c_void_p, ctypes.POINTER(Scope),
                                    ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
         L.bnpp_sum_out.argtypes = [ctypes.c_void_p, ctypes.POINTER(Scope), ctypes.c_void_p, ctypes.c_uint32,
@@ -164,11 +167,9 @@ class Context:
         return buf.value.decode(), g.value, b.value
 
     # ---- ops on raw device pointers (ints) ---------------------------------
-    def product_sum_out(self, operands, out_ids, out_cards, elim_var, out_ptr, z_ptr=None, divide=False):
-        """operands: list of (ptr, var_ids, cards, strides-or-None)"""
-        k = len(operands)
-        ops = (Operand * k)()
-        keep = []
+    @staticmethod
+    def _operands(operands, keep):
+        ops = (Operand * len(operands))()
         for i, (ptr, ids, cards, strides) in enumerate(operands):
             sc, ka = make_scope(ids, cards)
             keep.append(ka)
@@ -178,10 +179,25 @@ class Context:
                 keep.append(sa)
                 st = ctypes.cast(sa, c_i64p)
             ops[i] = Operand(ctypes.c_void_p(ptr), sc, st)
+        return ops
+
+    def product_sum_out(self, operands, out_ids, out_cards, elim_var, out_ptr, z_ptr=None, divide=False):
+        """operands: list of (ptr, var_ids, cards, strides-or-None)"""
+        k = len(operands)
+        keep = []
+        ops = self._operands(operands, keep)
         osc, ka = make_scope(out_ids, out_cards)
         self.check(self.L.bnpp_product_sum_out(self.h, k, ops, ctypes.byref(osc), -1 if elim_var is None else int(elim_var),
                                                int(divide), ctypes.c_void_p(out_ptr),
                                                ctypes.c_void_p(z_ptr) if z_ptr else None))
+
+    def product_max_out(self, operands, out_ids, out_cards, elim_var, out_ptr, arg_ptr):
+        """max-product step: out = max over elim_var of the product, arg (device uint8) = the first maximising value"""
+        keep = []
+        ops = self._operands(operands, keep)
+        osc, ka = make_scope(out_ids, out_cards)
+        self.check(self.L.bnpp_product_max_out(self.h, len(operands), ops, ctypes.byref(osc), int(elim_var),
+                                               ctypes.c_void_p(out_ptr), ctypes.c_void_p(arg_ptr)))
 
     def product(self, a_ptr, a_ids, a_cards, b_ptr, b_ids, b_cards, out_ptr, z_ptr=None, divide=False):
         sa, k1 = make_scope(a_ids, a_cards)

@@ -9,7 +9,7 @@
 
 namespace bnpp {
 int contract(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *out_scope, int64_t elim_var, int divide,
-             double *out_dev, double *z_dev);
+             double *out_dev, double *z_dev, bool max_mode = false, uint8_t *arg_dev = nullptr);
 int normalize(bnpp_ctx *ctx, uint64_t n, const double *in, const double *z_dev, double z_host, double *out);
 int reduce(bnpp_ctx *ctx, int op, uint64_t n, const double *in, double init, double *result);
 int fill(bnpp_ctx *ctx, double *out, uint64_t n, double value);
@@ -234,6 +234,12 @@ int bnpp_product_sum_out(bnpp_ctx *ctx, int k, const bnpp_operand *operands, con
                          int64_t elim_var, int divide, double *out_dev, double *z_dev)
 {
     return contract(ctx, k, operands, out_scope, elim_var, divide, out_dev, z_dev);
+}
+
+int bnpp_product_max_out(bnpp_ctx *ctx, int k, const bnpp_operand *operands, const bnpp_scope *out_scope,
+                         int64_t elim_var, double *out_dev, uint8_t *argmax_dev)
+{
+    return contract(ctx, k, operands, out_scope, elim_var, 0, out_dev, nullptr, true, argmax_dev);
 }
 
 int bnpp_product(bnpp_ctx *ctx, const bnpp_scope *sa, const double *a_dev, const bnpp_scope *sb, const double *b_dev,

@@ -392,7 +392,10 @@ __global__ void __launch_bounds__(kBlock) contract_fast_p2s(const __grid_constan
 // register shuffling -- per item K loads, 4(K-1) multiplies, 2+1 adds, one 16-byte store.
 // INVK >= 0 names an operand that does not depend on the two axes the plan placed at the
 // thread's unroll bits: its micro-tile is loaded once and reused for all U items.
-template <int K, unsigned MASK, int U, int INVK>
+// MAX: max-product instead -- r = the product at x = 0, replaced by x = 1's only if strictly
+// greater (ties keep the lower x, a NaN never replaces a number); the two argmax bytes of an
+// item go out as one 16-bit store at the (even) output index; no Z.
+template <int K, unsigned MASK, int U, int INVK, bool MAX = false>
 __global__ void __launch_bounds__(kBlock) contract_canon(const __grid_constant__ ParamsP2 p)
 {
     const ParamsHead &h = p.h;
@@ -431,12 +434,19 @@ __global__ void __launch_bounds__(kBlock) contract_canon(const __grid_constant__
                 cc = __dmul_rn(cc, tk.z);
                 d = __dmul_rn(d, tk.w);
             }
+            if (MAX) {
+                const bool x0 = b > a, x1 = d > cc;
+                const uint32_t o = ohi + olo[u];
+                *reinterpret_cast<double2 *>(h.out + o) = make_double2(x0 ? b : a, x1 ? d : cc);
+                *reinterpret_cast<uint16_t *>(h.arg + o) = (uint16_t)((uint32_t)x0 | ((uint32_t)x1 << 8));
+                continue;
+            }
             const double r0 = __dadd_rn(a, b), r1 = __dadd_rn(cc, d);
             zacc = __dadd_rn(zacc, __dadd_rn(r0, r1));
             *reinterpret_cast<double2 *>(h.out + (ohi + olo[u])) = make_double2(r0, r1);
         }
     }
-    if (h.z) grid_sum_to(zacc, h.partials, h.ticket, h.z);   // grid-uniform: intermediates of a VE plan need no partition
+    if (!MAX && h.z) grid_sum_to(zacc, h.partials, h.ticket, h.z);   // grid-uniform: intermediates of a VE plan need no partition
 }
 
 // Transposing variant: operand `st.sk` comes through a shared-memory tile (see StageInfo).
@@ -737,7 +747,8 @@ __global__ void __launch_bounds__(kBlock, 2) contract_staged_tma(const __grid_co
 }
 
 // Generic path: any cardinality of the eliminated variable, one output entry per item.
-template <class P, int K, bool DIV>
+// MAX: max-product (the rule of contract_canon<MAX>), arg[ooff] = the first maximising x; no Z.
+template <class P, int K, bool DIV, bool MAX = false>
 __global__ void __launch_bounds__(kBlock) contract_generic(const __grid_constant__ P p)
 {
     const ParamsHead &h = p.h;
@@ -748,6 +759,7 @@ __global__ void __launch_bounds__(kBlock) contract_generic(const __grid_constant
         uint32_t off[K], ooff;
         decompose<K>(p, (uint32_t)it, off, ooff);
         double acc = 0.0;
+        uint32_t best = 0;
         for (uint32_t x = 0; x < h.cx; ++x) {
             double v = ld1(h.in[0] + off[0] + x * h.sx[0]);
 #pragma unroll
@@ -756,13 +768,15 @@ __global__ void __launch_bounds__(kBlock) contract_generic(const __grid_constant
                 if (DIV) { zero_div |= (t == 0.0); v = __ddiv_rn(v, t); }
                 else v = __dmul_rn(v, t);
             }
-            acc = __dadd_rn(acc, v);
+            if (!MAX) acc = __dadd_rn(acc, v);
+            else if (x == 0 || v > acc) { acc = v; best = x; }
         }
         h.out[ooff] = acc;
-        zacc = __dadd_rn(zacc, acc);
+        if (MAX) h.arg[ooff] = (uint8_t)best;
+        else zacc = __dadd_rn(zacc, acc);
     }
     if (DIV && zero_div) atomicOr(h.status, BNPP_STATUS_ZERO_DIVISOR);
-    if (h.z) grid_sum_to(zacc, h.partials, h.ticket, h.z);   // grid-uniform: intermediates of a VE plan need no partition
+    if (!MAX && h.z) grid_sum_to(zacc, h.partials, h.ticket, h.z);   // grid-uniform: intermediates of a VE plan need no partition
 }
 
 // ---------------------------------------------------------------------------
@@ -777,6 +791,19 @@ struct Launch {
     {
         if (C == 1) return V == 2 ? contract_fast<P, K, 1, 2, U, false> : contract_fast<P, K, 1, 1, U, false>;
         return V == 2 ? contract_fast<P, K, 2, 2, U, false> : contract_fast<P, K, 2, 1, U, false>;
+    }
+
+    // max-product: one output entry per item, any cardinality and layout
+    static fn_t pick_max(int K)
+    {
+        switch (K) {
+        case 1: return contract_generic<P, 1, false, true>;
+        case 2: return contract_generic<P, 2, false, true>;
+        case 3: return contract_generic<P, 3, false, true>;
+        case 4: return contract_generic<P, 4, false, true>;
+        case 5: return contract_generic<P, 5, false, true>;
+        default: return contract_generic<P, 6, false, true>;
+        }
     }
 
     static fn_t pick(int K, int C, int V, bool div, bool generic, int &U)
@@ -831,34 +858,40 @@ typedef void (*p2s_fn)(const ParamsP2);
 
 constexpr int kCanonU = 4;
 
-template <int K, unsigned MASK>
+template <int K, unsigned MASK, bool MAX>
 static p2s_fn canon_inv(int invk)
 {
     switch (invk) {
-    case 0: return contract_canon<K, MASK, kCanonU, 0>;
-    case 1: return K > 1 ? contract_canon<K, MASK, kCanonU, (K > 1 ? 1 : -1)> : nullptr;
-    case 2: return K > 2 ? contract_canon<K, MASK, kCanonU, (K > 2 ? 2 : -1)> : nullptr;
-    default: return contract_canon<K, MASK, kCanonU, -1>;
+    case 0: return contract_canon<K, MASK, kCanonU, 0, MAX>;
+    case 1: return K > 1 ? contract_canon<K, MASK, kCanonU, (K > 1 ? 1 : -1), MAX> : nullptr;
+    case 2: return K > 2 ? contract_canon<K, MASK, kCanonU, (K > 2 ? 2 : -1), MAX> : nullptr;
+    default: return contract_canon<K, MASK, kCanonU, -1, MAX>;
     }
 }
 
-static p2s_fn pick_canon(int K, unsigned mask, int invk)
+template <int K, unsigned MASK>
+static p2s_fn canon_inv(int invk, bool max)
+{
+    return max ? canon_inv<K, MASK, true>(invk) : canon_inv<K, MASK, false>(invk);
+}
+
+static p2s_fn pick_canon(int K, unsigned mask, int invk, bool max)
 {
     switch (K * 8 + (int)mask) {
-    case 1 * 8 + 0: return canon_inv<1, 0>(-1);
-    case 1 * 8 + 1: return canon_inv<1, 1>(-1);
-    case 2 * 8 + 0: return canon_inv<2, 0>(invk);
-    case 2 * 8 + 1: return canon_inv<2, 1>(invk);
-    case 2 * 8 + 2: return canon_inv<2, 2>(invk);
-    case 2 * 8 + 3: return canon_inv<2, 3>(invk);
-    case 3 * 8 + 0: return canon_inv<3, 0>(invk);
-    case 3 * 8 + 1: return canon_inv<3, 1>(invk);
-    case 3 * 8 + 2: return canon_inv<3, 2>(invk);
-    case 3 * 8 + 3: return canon_inv<3, 3>(invk);
-    case 3 * 8 + 4: return canon_inv<3, 4>(invk);
-    case 3 * 8 + 5: return canon_inv<3, 5>(invk);
-    case 3 * 8 + 6: return canon_inv<3, 6>(invk);
-    case 3 * 8 + 7: return canon_inv<3, 7>(invk);
+    case 1 * 8 + 0: return canon_inv<1, 0>(-1, max);
+    case 1 * 8 + 1: return canon_inv<1, 1>(-1, max);
+    case 2 * 8 + 0: return canon_inv<2, 0>(invk, max);
+    case 2 * 8 + 1: return canon_inv<2, 1>(invk, max);
+    case 2 * 8 + 2: return canon_inv<2, 2>(invk, max);
+    case 2 * 8 + 3: return canon_inv<2, 3>(invk, max);
+    case 3 * 8 + 0: return canon_inv<3, 0>(invk, max);
+    case 3 * 8 + 1: return canon_inv<3, 1>(invk, max);
+    case 3 * 8 + 2: return canon_inv<3, 2>(invk, max);
+    case 3 * 8 + 3: return canon_inv<3, 3>(invk, max);
+    case 3 * 8 + 4: return canon_inv<3, 4>(invk, max);
+    case 3 * 8 + 5: return canon_inv<3, 5>(invk, max);
+    case 3 * 8 + 6: return canon_inv<3, 6>(invk, max);
+    case 3 * 8 + 7: return canon_inv<3, 7>(invk, max);
     default: return nullptr;
     }
 }
@@ -968,6 +1001,7 @@ static void describe(LaunchDesc *d, const ParamsHead &h, const void *fn, uint64_
     d->U = U;
     d->div = div;
     d->generic = generic;
+    d->max = false;
     d->R = R;
     (void)h;
 }
@@ -980,6 +1014,9 @@ std::string LaunchDesc::name()
                       mvtp.T, mvtp.g, mvtp.n_tiles, R, mvtp.stage_doubles * 8u);
     else if (mv) snprintf(nm, sizeof nm, "contract_mv<%s,K=%d,U=%d> cx=%u T=%u E=%u g=%u tiles=%u R=%u", variant, k, U, h.cx, mvp.T, mvp.E,
                      mvp.g, mvp.n_tiles, R);
+    else if (max && generic) snprintf(nm, sizeof nm, "contract_generic_max<%s,K=%d> cx=%u R=%u", variant, k, h.cx, R);
+    else if (max) snprintf(nm, sizeof nm, "contract_canon_max<%s,K=%d,U=%d> R=%u cls=%d,%d,%d", variant, k, U, R, h.cls[0],
+                           k > 1 ? h.cls[1] : -1, k > 2 ? h.cls[2] : -1);
     else if (generic) snprintf(nm, sizeof nm, "contract_generic<%s,K=%d,div=%d> cx=%u R=%u", variant, k, div, h.cx, R);
     else snprintf(nm, sizeof nm, "contract_fast<%s,K=%d,C=%d,V=%d,U=%d,div=%d> R=%u cls=%d,%d,%d", variant, k, C, V, U, div, R,
                   h.cls[0], k > 1 ? h.cls[1] : -1, k > 2 ? h.cls[2] : -1);
@@ -988,19 +1025,22 @@ std::string LaunchDesc::name()
 
 template <class P>
 static int plan_launch(bnpp_ctx *ctx, LaunchDesc *d, const P &p, int k, int C, int V, bool div, bool generic, const char *mode,
-                       uint32_t R)
+                       uint32_t R, bool max = false)
 {
     int U = 1;
-    typename Launch<P>::fn_t fn = Launch<P>::pick(k, C, V, div, generic, U);
+    typename Launch<P>::fn_t fn = max ? Launch<P>::pick_max(k) : Launch<P>::pick(k, C, V, div, generic, U);
     uint64_t blocks = (p.h.n_items + (uint64_t)kBlock * U - 1) / ((uint64_t)kBlock * U);
     const uint64_t cap = resident_ctas(ctx, fn);
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
     describe(d, p.h, reinterpret_cast<const void *>(fn), blocks, mode, k, C, V, U, div, generic, R);
+    d->max = max;
     return BNPP_OK;
 }
 
-static bool plan_launch_p2s(bnpp_ctx *ctx, LaunchDesc *d, const ParamsP2 &p, int k, int C, int V, bool div, uint32_t R)
+// max: only the canonical layout has a max-product variant here (false otherwise: contract_generic<MAX> takes the step)
+static bool plan_launch_p2s(bnpp_ctx *ctx, LaunchDesc *d, const ParamsP2 &p, int k, int C, int V, bool div, uint32_t R,
+                            bool max = false)
 {
     int U = 1;
     p2s_fn fn = nullptr;
@@ -1023,11 +1063,12 @@ static bool plan_launch_p2s(bnpp_ctx *ctx, LaunchDesc *d, const ParamsP2 &p, int
                     touches |= (((uint64_t)p.f[q][f].mask << p.f[q][f].sh) & (uint64_t)(kBlock * (kCanonU - 1))) != 0;
                 if (!touches && (invk < 0 || (((mask >> q) & 1u) && !((mask >> invk) & 1u)))) invk = q;
             }
-            fn = pick_canon(k, mask, invk);
+            fn = pick_canon(k, mask, invk, max);
             U = kCanonU;
             variant = invk < 0 ? "canon" : (invk == 0 ? "canon/inv0" : (invk == 1 ? "canon/inv1" : "canon/inv2"));
         }
     }
+    if (max && (!fn || !aligned(p.h.arg, 2))) return false;
     if (!fn) fn = pick_p2s(k, C, V, div, U);
     const uint64_t ch = (uint64_t)kBlock * U;
     if (p.h.n_items < ch || p.h.n_items % ch) return false;   // tiny problem: per-item kernel
@@ -1035,6 +1076,7 @@ static bool plan_launch_p2s(bnpp_ctx *ctx, LaunchDesc *d, const ParamsP2 &p, int
     const uint64_t cap = resident_ctas(ctx, fn);
     if (blocks > cap) blocks = cap;
     describe(d, p.h, reinterpret_cast<const void *>(fn), blocks, variant, k, C, V, U, div, false, R);
+    d->max = max;
     return true;
 }
 
@@ -1056,10 +1098,10 @@ int contract_launch(bnpp_ctx *ctx, LaunchDesc &d, const double *const *in, doubl
 }
 
 int contract(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *out_scope, int64_t elim_var, int divide,
-             double *out_dev, double *z_dev)
+             double *out_dev, double *z_dev, bool max_mode, uint8_t *arg_dev)
 {
     LaunchDesc d;
-    const int rc = contract_plan(ctx, k, ops, out_scope, elim_var, divide, out_dev, z_dev, &d);
+    const int rc = contract_plan(ctx, k, ops, out_scope, elim_var, divide, out_dev, z_dev, &d, max_mode, arg_dev);
     if (rc != BNPP_OK) return rc;
     const double *in[kMaxK];
     for (int q = 0; q < k; ++q) in[q] = ops[q].data;
@@ -1070,10 +1112,27 @@ int contract(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *ou
     return rc2;
 }
 
+// max_mode: 0 = sum-product; 1 = max-product, canon<MAX> where the sum-mode plan takes canon; 2 = max-product, generic<MAX>
+static int plan_impl(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *out_scope, int64_t elim_var,
+                     int divide, double *out_dev, double *z_dev, LaunchDesc *desc, int max_mode, uint8_t *arg_dev);
+
 int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *out_scope, int64_t elim_var,
-                  int divide, double *out_dev, double *z_dev, LaunchDesc *desc)
+                  int divide, double *out_dev, double *z_dev, LaunchDesc *desc, bool max_mode, uint8_t *arg_dev)
 {
     if (!ctx || !desc) return BNPP_EINVAL;
+    if (max_mode) {
+        if (elim_var < 0) return fail(ctx, BNPP_EINVAL, "product_max_out: a max-product step eliminates a variable");
+        if (divide) return fail(ctx, BNPP_EINVAL, "product_max_out: no divide");
+        if (!arg_dev) return fail(ctx, BNPP_EINVAL, "product_max_out: argmax buffer missing");
+    }
+    return plan_impl(ctx, k, ops, out_scope, elim_var, divide, out_dev, z_dev, desc, max_mode ? 1 : 0, arg_dev);
+}
+
+static int plan_impl(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *out_scope, int64_t elim_var,
+                     int divide, double *out_dev, double *z_dev, LaunchDesc *desc, int max_mode, uint8_t *arg_dev)
+{
+    // the generic max-product kernel: one output entry per item (V = 1), planned again from scratch
+    auto generic_max = [&]() { return plan_impl(ctx, k, ops, out_scope, elim_var, divide, out_dev, z_dev, desc, 2, arg_dev); };
     if (k < 1 || k > kMaxK) return fail(ctx, BNPP_ERANK, "product_sum_out: operand count must be 1..BNPP_MAX_OPERANDS");
     if (divide && k != 2) return fail(ctx, BNPP_EINVAL, "divide needs exactly two operands");
     if (!out_scope || out_scope->rank < 0 || out_scope->rank > BNPP_MAX_RANK)
@@ -1128,6 +1187,8 @@ int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scop
         if (maxoff >= (1ull << 32)) return fail(ctx, BNPP_ETOOBIG, "operand table has >= 2^32 entries");
         op_bytes[q] = 8 * dense;
     }
+    if (max_mode && cx > 255)
+        return fail(ctx, BNPP_EINVAL, "product_max_out: the eliminated variable has more than 255 values (uint8 argmax)");
 
     // ---- iteration order -------------------------------------------------------
     // keep the output's fastest axes (>= kTileOutputs entries) in place; above them iterate
@@ -1262,7 +1323,7 @@ int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scop
         m.push_back(it[i]);
     }
 
-    const bool generic = (cx > 2);
+    const bool generic = (cx > 2) || max_mode == 2;
     // The tiled multi-valued kernels stream: they pay per union entry for bringing operand entries to the SM.  A step
     // whose operands are all much smaller than its union table (an outer product of small tables) re-reads them from
     // L1/L2 either way, and there the one-entry-per-thread kernel with its cached gathers is as fast or faster
@@ -1271,7 +1332,7 @@ int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scop
     uint64_t heaviest = 0;
     for (int q = 0; q < k; ++q) heaviest = std::max(heaviest, op_bytes[q]);
     const bool streams = heaviest * 16 >= 8 * n_out * cx || mv_min_entries() == 0;
-    if (generic && !divide && streams && n_out * cx >= mv_min_entries()) {
+    if (generic && !divide && !max_mode && streams && n_out * cx >= mv_min_entries()) {
         // multi-valued elimination: the table-driven tile kernel (contract_mv.cu), in the output's own axis order
         std::vector<MVAxis> mva;
         for (int i = 0; i < wr; ++i) {
@@ -1323,6 +1384,7 @@ int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scop
     h.n_items = n_out / V;
     h.cx = cx;
     h.out = out_dev;
+    h.arg = max_mode ? arg_dev : nullptr;
     h.out_vec = (V == 2 && h.sol == 1 && aligned(out_dev, 16)) ? 1 : 0;
     for (uint32_t a = 0; a < R && h.out_vec; ++a)
         if (m[a].so % 2) h.out_vec = 0;
@@ -1519,6 +1581,7 @@ int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scop
                     if (!((pt.mask >> q) & 1u) && op_bytes[q] * 8 >= total_bytes) all_big = false;
                 tma_fn fn = pick_staged_tma(k, C);
                 if (fn && all_big && 2u * off * 8u <= budget) {
+                    if (max_mode) return generic_max();
                     pt.b = p;
                     desc->p2 = true;
                     desc->tma = true;
@@ -1537,6 +1600,7 @@ int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scop
             st.pair = (even && st.tile >= 2 * kBlock) ? 1 : 0;
             staged_fn fn = ok ? pick_staged(k, C) : nullptr;
             if (fn) {
+                if (max_mode) return generic_max();
                 desc->p2 = true;
                 desc->staged = true;
                 const uint64_t cap = resident_ctas(ctx, fn);
@@ -1549,11 +1613,13 @@ int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scop
         if (fits) {
             desc->p2 = true;
             desc->staged = false;
-            if (!generic && plan_launch_p2s(ctx, desc, p, k, C, V, divide != 0, R)) return BNPP_OK;
-            return plan_launch(ctx, desc, p, k, C, V, divide != 0, generic, "p2", R);
+            if (!generic && plan_launch_p2s(ctx, desc, p, k, C, V, divide != 0, R, max_mode != 0)) return BNPP_OK;
+            if (max_mode && !generic) return generic_max();
+            return plan_launch(ctx, desc, p, k, C, V, divide != 0, generic, "p2", R, max_mode != 0);
         }
     }
 
+    if (max_mode && !generic) return generic_max();
     if ((int)R > kMaxR) return fail(ctx, BNPP_ERANK, "more than BNPP_MAX_AXES non-mergeable axes");
     ParamsMR &p = desc->mrp;
     memset(&p, 0, sizeof p);
@@ -1565,7 +1631,7 @@ int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scop
         for (int q = 0; q < k; ++q) p.s[q][a] = (uint32_t)m[a].s[q];
     }
     desc->p2 = false;
-    return plan_launch(ctx, desc, p, k, C, V, divide != 0, generic, "mr", R);
+    return plan_launch(ctx, desc, p, k, C, V, divide != 0, generic, "mr", R, max_mode != 0);
 }
 
 }  // namespace bnpp

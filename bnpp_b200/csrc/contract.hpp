@@ -27,6 +27,7 @@ struct ParamsHead {
     uint32_t sol;               // output stride between the V entries of an item
     uint8_t cls[kMaxK];
     uint8_t out_vec;            // 16-byte store allowed
+    uint8_t *arg;               // max-product steps: the first maximising x per output entry, at the output's index
 };
 
 // Mixed-radix iteration space: digits by multiply-high division, outermost axis first.
@@ -150,14 +151,19 @@ struct LaunchDesc {
     const char *variant = "";
     int C = 0, V = 0, U = 0;
     bool div = false, generic = false;
+    bool max = false;           // max-product step: contract_canon_max / contract_generic_max
     uint32_t R = 0;
     std::string name();
     ParamsHead &head() { return tma ? p2t.b.h : (mvt ? mvtp.h : (mv ? mvp.h : (p2 ? p2p.b.h : mrp.h))); }
     void *params() { return tma ? static_cast<void *>(&p2t) : mvt ? static_cast<void *>(&mvtp) : mv ? static_cast<void *>(&mvp) : (p2 ? (staged ? static_cast<void *>(&p2p) : static_cast<void *>(&p2p.b)) : static_cast<void *>(&mrp)); }
 };
 
+// max_mode: out[o] = max_x prod_k F_k[pi_k(o, x)] and arg_dev[o] = the first x attaining it (no Z); elim_var must be
+// >= 0 with at most 255 values.  The step takes contract_canon<MAX> where the sum-mode plan would take contract_canon,
+// else contract_generic<MAX>.  arg_dev is fixed at planning time: contract_launch does not patch it.
 int contract_plan(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *out_scope, int64_t elim_var,
-                  int divide, double *out_dev, double *z_dev, LaunchDesc *desc);
+                  int divide, double *out_dev, double *z_dev, LaunchDesc *desc, bool max_mode = false,
+                  uint8_t *arg_dev = nullptr);
 // in / out / z replace the pointers the descriptor was planned with; they must be at least as
 // aligned (a descriptor planned for 32-byte aligned operands may use 256-bit loads)
 int contract_launch(bnpp_ctx *ctx, LaunchDesc &desc, const double *const *in, double *out, double *z);

@@ -34,7 +34,7 @@
 
 namespace bnpp {
 int contract(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *out_scope, int64_t elim_var, int divide,
-             double *out_dev, double *z_dev);
+             double *out_dev, double *z_dev, bool max_mode = false, uint8_t *arg_dev = nullptr);
 int fill(bnpp_ctx *ctx, double *out, uint64_t n, double value);
 int normalize_segments(bnpp_ctx *ctx, double *buf, const uint32_t *off_dev, const uint32_t *size_dev, int n);
 
@@ -98,6 +98,39 @@ struct FusedProgram {
     uint32_t *prog_dev = nullptr, *offtab_dev = nullptr;
     bool offtab_uploaded = false;
 };
+// MPE decode (bnpp_mpe_plan_run): one thread walks the eliminating steps in reverse.  rec: the n_obs observed ids,
+// then per eliminating step, last first: elim var, argmax table offset (bytes, lo, hi), rank, rank x (var, stride)
+// over the step's output scope -- every variable there is eliminated later, so it is already decoded.  The evidence
+// values travel in the parameters (a replay re-parameterises the node), in device memory beyond kDecodeInlineObs.
+constexpr uint32_t kDecodeInlineObs = 896;
+struct MpeDecodeParams {
+    const uint32_t *rec;
+    const uint8_t *arg;
+    const uint32_t *obs_val_dev;
+    uint32_t *assign;
+    double *value;
+    uint32_t nvars, n_obs, n_rec, set_one;      // set_one: the plan has no result step, the value is the empty product
+    uint32_t obs_val[kDecodeInlineObs];
+};
+
+__global__ void mpe_decode(const __grid_constant__ MpeDecodeParams p)
+{
+    if (threadIdx.x || blockIdx.x) return;
+    for (uint32_t v = 0; v < p.nvars; ++v) p.assign[v] = 0;
+    const uint32_t *r = p.rec;
+    const uint32_t *val = p.n_obs <= kDecodeInlineObs ? p.obs_val : p.obs_val_dev;
+    for (uint32_t i = 0; i < p.n_obs; ++i) p.assign[r[i]] = val[i];
+    r += p.n_obs;
+    for (uint32_t s = 0; s < p.n_rec; ++s) {
+        const uint64_t off = (uint64_t)r[1] | ((uint64_t)r[2] << 32);
+        const uint32_t rank = r[3];
+        uint64_t idx = 0;
+        for (uint32_t j = 0; j < rank; ++j) idx += (uint64_t)p.assign[r[4 + 2 * j]] * r[5 + 2 * j];
+        p.assign[r[0]] = p.arg[off + idx];
+        r += 4 + 2 * rank;
+    }
+    if (p.set_one) *p.value = 1.0;
+}
 }  // namespace bnpp
 
 struct bnpp_ve_plan {
@@ -174,6 +207,18 @@ struct bnpp_ve_plan {
     bool is_mar = false;
     std::vector<uint32_t> mar_off, mar_size;
     uint32_t *mar_off_dev = nullptr, *mar_size_dev = nullptr;
+    // MPE plan (max-product): every eliminating step also writes its argmax table into a byte arena that is never
+    // reused within a run (the decode reads all of them); K9 / K10 stay off (their interpreters only sum)
+    bool is_mpe = false;
+    uint32_t mpe_nvars = 0;
+    std::vector<uint64_t> arg_off;          // per step: byte offset of its argmax table (eliminating steps only)
+    uint64_t arg_bytes = 0;
+    uint8_t *arg_arena = nullptr;
+    std::vector<uint32_t> decode_rec;       // see MpeDecodeParams; uploaded once
+    uint32_t *decode_rec_dev = nullptr, *obs_val_dev = nullptr;
+    uint32_t n_decode_rec = 0;
+    bnpp::MpeDecodeParams decode;           // parameters of the decode's node in the replay graph
+    cudaGraphNode_t decode_node = nullptr;
     bool profiling = false;
     std::vector<cudaEvent_t> ev;
     std::vector<float> step_ms;
@@ -470,7 +515,9 @@ bool plan_step(bnpp_ve_plan *pl, size_t s)
     }
     pl->exec_planned[s] = 1;
     if (!pl->exec[s]) pl->exec[s].reset(new LaunchDesc());
-    return contract_plan(pl->ctx, (int)st.operands.size(), ops, &os, st.elim, 0, dst, nullptr, pl->exec[s].get()) == BNPP_OK;
+    const bool max_mode = pl->is_mpe && st.elim >= 0;
+    return contract_plan(pl->ctx, (int)st.operands.size(), ops, &os, st.elim, 0, dst, nullptr, pl->exec[s].get(), max_mode,
+                         max_mode ? pl->arg_arena + pl->arg_off[s] : nullptr) == BNPP_OK;
 }
 
 
@@ -1265,8 +1312,11 @@ int run_fused(bnpp_ve_plan *pl, FusedProgram &fp, int G, const double *const *ta
 
 extern "C" {
 
-int bnpp_ve_plan_create(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_obs, const uint32_t *obs_var,
-                        int n_order, const uint32_t *order, bnpp_ve_plan **out)
+static int mpe_finish(bnpp_ve_plan *pl, int nvars, int n_obs, const uint32_t *obs_var);
+
+// the bucket schedule of bnpp_ve_plan_create; mpe_card != NULL: an MPE plan over that many variables (bnpp_mpe_plan_create)
+static int create_plan(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_obs, const uint32_t *obs_var, int n_order,
+                       const uint32_t *order, int mpe_nvars, const uint32_t *mpe_card, bnpp_ve_plan **out)
 {
     if (!out || nfac < 0 || n_obs < 0 || n_order < 0) return BNPP_EINVAL;   // ctx == NULL: a dry plan (inspect, never run)
     *out = nullptr;
@@ -1293,6 +1343,20 @@ int bnpp_ve_plan_create(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n
     if (int rc = add_inputs(pl, nfac, scopes, obs_index, rank)) {
         delete pl;
         return fail(ctx, rc, "bad factor scope");
+    }
+    if (mpe_card) {
+        // MPE eliminates every unobserved variable; its argmax tables are uint8
+        for (const PlanFactor &pf : pl->f)
+            for (size_t a = 0; a < pf.var.size(); ++a) {
+                const char *why = nullptr;
+                if (pf.var[a] >= (uint32_t)mpe_nvars) why = "MPE plan: a scope names a variable id >= nvars";
+                else if (rank.at(pf.var[a]) >= (uint64_t)n_order) why = "MPE plan: the order misses an unobserved variable";
+                else if (pf.card[a] > 255) why = "MPE plan: a variable has more than 255 values (uint8 argmax tables)";
+                if (why) {
+                    delete pl;
+                    return fail(ctx, BNPP_EINVAL, why);
+                }
+            }
     }
 
     // bucket = factors whose earliest-eliminated variable is order[i] (code/model.cpp:390-406)
@@ -1339,6 +1403,12 @@ int bnpp_ve_plan_create(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n
     const auto tc2 = std::chrono::steady_clock::now();
     build_exec(pl);
     const auto tc3 = std::chrono::steady_clock::now();
+    if (mpe_card) {
+        if (int rc = mpe_finish(pl, mpe_nvars, n_obs, obs_var)) {
+            delete pl;
+            return fail(ctx, rc, "MPE plan: bad observed variable");
+        }
+    }
     if (pl->segments_mode) build_levels(pl);
     if (getenv("BNPP_TIMING")) {
         auto ms = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
@@ -1348,6 +1418,64 @@ int bnpp_ve_plan_create(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n
                 ms(tc0, tc1), ms(tc1, tc2), ms(tc2, tc3), ms(tc3, std::chrono::steady_clock::now()));
     }
     *out = pl;
+    return BNPP_OK;
+}
+
+int bnpp_ve_plan_create(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_obs, const uint32_t *obs_var,
+                        int n_order, const uint32_t *order, bnpp_ve_plan **out)
+{
+    return create_plan(ctx, nfac, scopes, n_obs, obs_var, n_order, order, 0, nullptr, out);
+}
+
+int bnpp_mpe_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfac, const bnpp_scope *scopes, int n_obs,
+                         const uint32_t *obs_var, int n_order, const uint32_t *order, bnpp_ve_plan **out)
+{
+    if (!out || nvars < 0 || !card) return BNPP_EINVAL;
+    for (int i = 0; i < n_order; ++i)
+        if (order[i] >= (uint32_t)nvars) return fail(ctx, BNPP_EINVAL, "MPE plan: an order entry is >= nvars");
+    return create_plan(ctx, nfac, scopes, n_obs, obs_var, n_order, order, nvars, card, out);
+}
+
+// Argmax arena and decode records of an MPE plan; the K9 / K10 paths off
+static int mpe_finish(bnpp_ve_plan *pl, int nvars, int n_obs, const uint32_t *obs_var)
+{
+    pl->is_mpe = true;
+    pl->mpe_nvars = (uint32_t)nvars;
+    pl->fused_mode = 0;
+    pl->segments_mode = 0;
+    pl->arg_off.assign(pl->steps.size(), 0);
+    for (size_t s = 0; s < pl->steps.size(); ++s) {
+        const PlanStep &st = pl->steps[s];
+        if (st.elim < 0) continue;
+        pl->arg_off[s] = (pl->arg_bytes + 255) & ~(uint64_t)255;
+        pl->arg_bytes = pl->arg_off[s] + pl->f[st.out].size;
+    }
+    pl->peak_bytes += pl->arg_bytes;
+    std::vector<uint32_t> &r = pl->decode_rec;
+    for (int i = 0; i < n_obs; ++i) {
+        if (obs_var[i] >= (uint32_t)nvars) return BNPP_EINVAL;
+        r.push_back(obs_var[i]);
+    }
+    for (size_t s = pl->steps.size(); s-- > 0;) {
+        const PlanStep &st = pl->steps[s];
+        if (st.elim < 0) continue;
+        const PlanFactor &of = pl->f[st.out];
+        r.push_back((uint32_t)st.elim);
+        r.push_back((uint32_t)pl->arg_off[s]);
+        r.push_back((uint32_t)(pl->arg_off[s] >> 32));
+        r.push_back((uint32_t)of.var.size());
+        uint64_t stride = 1;
+        std::vector<uint32_t> st_of(of.var.size());
+        for (size_t a = of.var.size(); a-- > 0;) {
+            st_of[a] = (uint32_t)stride;
+            stride *= of.card[a];
+        }
+        for (size_t a = 0; a < of.var.size(); ++a) {
+            r.push_back(of.var[a]);
+            r.push_back(st_of[a]);
+        }
+        pl->n_decode_rec++;
+    }
     return BNPP_OK;
 }
 
@@ -1510,6 +1638,9 @@ int bnpp_ve_plan_destroy(bnpp_ve_plan *pl)
     if (pl->graph_exec) cudaGraphExecDestroy(pl->graph_exec);
     if (pl->graph) cudaGraphDestroy(pl->graph);
     if (pl->arena) bnpp_free(pl->ctx, pl->arena);
+    if (pl->arg_arena) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->arg_arena));
+    if (pl->decode_rec_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->decode_rec_dev));
+    if (pl->obs_val_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->obs_val_dev));
     for (auto &d : pl->exec)
         if (d) {
             contract_release(pl->ctx, *d);
@@ -1583,6 +1714,7 @@ int bnpp_ve_plan_set_profiling(bnpp_ve_plan *pl, int on)
 int bnpp_ve_plan_set_fused(bnpp_ve_plan *pl, int on)
 {
     if (!pl) return BNPP_EINVAL;
+    if (pl->is_mpe && on) return fail(pl->ctx, BNPP_EINVAL, "MPE plans run one launch per bucket (ve_fused only sums)");
     pl->fused_mode = on != 0;
     return BNPP_OK;
 }
@@ -1660,6 +1792,7 @@ int bnpp_ve_plan_describe(const bnpp_ve_plan *pl, uint64_t *buf, uint64_t cap, u
 int bnpp_ve_plan_set_segments(bnpp_ve_plan *pl, int on, uint32_t max_steps)
 {
     if (!pl) return BNPP_EINVAL;
+    if (pl->is_mpe && on) return fail(pl->ctx, BNPP_EINVAL, "MPE plans run one launch per bucket (ve_tasks only sums)");
     pl->segments_mode = on != 0 ? 1 : 0;
     if (pl->graph_exec && pl->graph_groups != (on != 0)) {      // the replay graph was built the other way
         cudaGraphExecDestroy(pl->graph_exec);
@@ -1777,6 +1910,7 @@ int bnpp_ve_plan_step_kernel(const bnpp_ve_plan *pl, uint64_t step, char *name, 
     return BNPP_OK;
 }
 
+// MPE plans: eliminating steps are max-product steps writing their argmax tables into the plan's byte arena
 static int run_dynamic(bnpp_ve_plan *pl, const std::vector<const double *> &ptr_in, double *result_dev, double *z_dev)
 {
     bnpp_ctx *ctx = pl->ctx;
@@ -1812,7 +1946,9 @@ static int run_dynamic(bnpp_ve_plan *pl, const std::vector<const double *> &ptr_
             dst = owned[st.out];
             ptr[st.out] = dst;
         }
-        rc = contract(ctx, (int)st.operands.size(), ops, &os, st.elim, 0, dst, (st.out == -2 && st.want_z) ? z_dev : nullptr);
+        const bool max_mode = pl->is_mpe && st.elim >= 0;
+        rc = contract(ctx, (int)st.operands.size(), ops, &os, st.elim, 0, dst, (st.out == -2 && st.want_z) ? z_dev : nullptr,
+                      max_mode, max_mode ? pl->arg_arena + pl->arg_off[s] : nullptr);
         if (pl->profiling) {
             pl->step_kernel.resize(pl->steps.size());
             pl->step_kernel[s] = ctx->last_kernel;   // set by contract() below
@@ -1828,8 +1964,64 @@ static int run_dynamic(bnpp_ve_plan *pl, const std::vector<const double *> &ptr_
     return rc;
 }
 
+// the parameters of an MPE run's decode (a launch, or the last node of the replay graph, set again on every replay:
+// the evidence values travel in them); the decode records go to the device on the first run
+static int mpe_decode_prepare(bnpp_ve_plan *pl, const uint32_t *obs_val, double *value_dev, uint32_t *assign_dev)
+{
+    bnpp_ctx *ctx = pl->ctx;
+    if (!pl->decode_rec_dev && !pl->decode_rec.empty()) {
+        double *store = nullptr;
+        int rc = bnpp_alloc(ctx, (pl->decode_rec.size() + 1) / 2, &store);
+        if (rc != BNPP_OK) return rc;
+        pl->decode_rec_dev = reinterpret_cast<uint32_t *>(store);
+        BNPP_CUDA(ctx, cudaMemcpyAsync(pl->decode_rec_dev, pl->decode_rec.data(), 4 * pl->decode_rec.size(),
+                                       cudaMemcpyHostToDevice, ctx->stream));
+    }
+    MpeDecodeParams &p = pl->decode;
+    p.rec = pl->decode_rec_dev;
+    p.arg = pl->arg_arena;
+    p.assign = assign_dev;
+    p.value = value_dev;
+    p.nvars = pl->mpe_nvars;
+    p.n_obs = (uint32_t)pl->n_obs;
+    p.n_rec = pl->n_decode_rec;
+    p.set_one = (pl->steps.empty() || pl->steps.back().out != -2) ? 1u : 0u;
+    if (p.n_obs <= kDecodeInlineObs) {
+        for (uint32_t i = 0; i < p.n_obs; ++i) p.obs_val[i] = obs_val[i];
+    } else {
+        if (!pl->obs_val_dev) {
+            double *store = nullptr;
+            int rc = bnpp_alloc(ctx, (p.n_obs + 1) / 2, &store);
+            if (rc != BNPP_OK) return rc;
+            pl->obs_val_dev = reinterpret_cast<uint32_t *>(store);
+        }
+        BNPP_CUDA(ctx, cudaMemcpyAsync(pl->obs_val_dev, obs_val, 4ull * p.n_obs, cudaMemcpyHostToDevice, ctx->stream));
+        p.obs_val_dev = pl->obs_val_dev;
+    }
+    return BNPP_OK;
+}
+
+static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uint32_t *obs_val, double *result_dev,
+                    double *z_dev, uint32_t *assign_dev);
+
 int bnpp_ve_plan_run(bnpp_ve_plan *pl, const double *const *tables_dev, const uint32_t *obs_val, double *result_dev,
                      double *z_dev)
+{
+    if (pl && pl->is_mpe) return fail(pl->ctx, BNPP_EINVAL, "MPE plan: run it with bnpp_mpe_plan_run");
+    return run_plan(pl, tables_dev, obs_val, result_dev, z_dev, nullptr);
+}
+
+int bnpp_mpe_plan_run(bnpp_ve_plan *pl, const double *const *tables_dev, const uint32_t *obs_val, double *value_dev,
+                      uint32_t *assignment_dev)
+{
+    if (!pl) return BNPP_EINVAL;
+    if (!pl->is_mpe || !assignment_dev) return fail(pl->ctx, BNPP_EINVAL, "bnpp_mpe_plan_run: not an MPE plan, or no assignment buffer");
+    return run_plan(pl, tables_dev, obs_val, value_dev, nullptr, assignment_dev);
+}
+
+// assign_dev != NULL: an MPE run (result_dev is the value)
+static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uint32_t *obs_val, double *result_dev,
+                    double *z_dev, uint32_t *assign_dev)
 {
     if (!pl || !pl->ctx || !result_dev) return BNPP_EINVAL;
     bnpp_ctx *ctx = pl->ctx;
@@ -1848,7 +2040,7 @@ int bnpp_ve_plan_run(bnpp_ve_plan *pl, const double *const *tables_dev, const ui
         ptr[i] = tables_dev[pf.src] + base;
         aligned32 = aligned32 && (reinterpret_cast<uintptr_t>(tables_dev[pf.src]) % 32 == 0);
     }
-    if (!pl->is_mar && (pl->steps.empty() || pl->steps.back().out != -2)) {
+    if (!pl->is_mar && !pl->is_mpe && (pl->steps.empty() || pl->steps.back().out != -2)) {
         int rc = fill(ctx, result_dev, 1, 1.0);   // no factor left: the scalar 1 (code/model.cpp:355)
         if (rc != BNPP_OK) return rc;
         if (z_dev) rc = fill(ctx, z_dev, 1, 1.0);
@@ -1858,7 +2050,17 @@ int bnpp_ve_plan_run(bnpp_ve_plan *pl, const double *const *tables_dev, const ui
     int fused_g = 0;
     bool ev_inline = pl->n_obs <= kFusedInlineEv;      // the evidence values travel in the kernel parameters as bytes
     for (int i = 0; i < pl->n_obs && ev_inline; ++i) ev_inline = obs_val[i] <= 255;
-    if (ev_inline) fused_g = fused_pick(pl, 1);
+    if (ev_inline && !pl->is_mpe) fused_g = fused_pick(pl, 1);
+    if (pl->is_mpe) {
+        if (!pl->arg_arena && pl->arg_bytes) {
+            double *store = nullptr;
+            rc = bnpp_alloc(ctx, (pl->arg_bytes + 7) / 8, &store);
+            if (rc != BNPP_OK) return rc;
+            pl->arg_arena = reinterpret_cast<uint8_t *>(store);
+        }
+        rc = mpe_decode_prepare(pl, obs_val, result_dev, assign_dev);
+        if (rc != BNPP_OK) return rc;
+    }
     if (getenv("BNPP_TIMING") && pl->runs == 0)
         fprintf(stderr, "bnpp timing: up to the choice of the path %.3f ms\n",
                 std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_run0).count());
@@ -1867,6 +2069,11 @@ int bnpp_ve_plan_run(bnpp_ve_plan *pl, const double *const *tables_dev, const ui
         rc = run_fused(pl, fused_g, tables_dev, 1, nullptr, obs_val, result_dev, z_dev);
     } else if (!pl->exec_ok || !aligned32) {
         rc = run_dynamic(pl, ptr, result_dev, z_dev);
+        if (rc == BNPP_OK && pl->is_mpe) {
+            mpe_decode<<<1, 32, 0, ctx->stream>>>(pl->decode);
+            BNPP_CUDA(ctx, cudaGetLastError());
+            ctx->launches++;
+        }
     } else {
         if (!pl->arena && pl->arena_doubles) {
             const auto t_a0 = std::chrono::steady_clock::now();
@@ -1884,7 +2091,7 @@ int bnpp_ve_plan_run(bnpp_ve_plan *pl, const double *const *tables_dev, const ui
         for (size_t i = 0; i < pl->f.size(); ++i)
             if (pl->f[i].src < 0) ptr[i] = pl->arena + pl->arena_off[i];
         // K10: the small tasks of every dependency level as ONE ve_tasks launch (a node of the replay graph like any other)
-        const bool seg_on = pl->segments_mode && pl->levels_built && ev_inline && !pl->profiling;
+        const bool seg_on = pl->segments_mode && pl->levels_built && ev_inline && !pl->profiling && !pl->is_mpe;
         static const bool timing = getenv("BNPP_TIMING") != nullptr;
         const auto t_0 = std::chrono::steady_clock::now();
         if (seg_on && !pl->segments_built) build_segments(pl);
@@ -1981,6 +2188,26 @@ int bnpp_ve_plan_run(bnpp_ve_plan *pl, const double *const *tables_dev, const ui
             if (e != cudaSuccess) return cuda_fail(ctx, e, "CUDA graph node");
             if (fresh) prev = pl->nodes[s];
         }
+        if (pl->is_mpe && rc == BNPP_OK) {
+            ++n_launched;
+            if (!(graphed && pl->use_graph)) {
+                mpe_decode<<<1, 32, 0, ctx->stream>>>(pl->decode);
+                BNPP_CUDA(ctx, cudaGetLastError());
+                ctx->launches++;
+            } else {
+                void *args[1] = {&pl->decode};
+                cudaKernelNodeParams kp;
+                memset(&kp, 0, sizeof kp);
+                kp.func = reinterpret_cast<void *>(mpe_decode);
+                kp.gridDim = dim3(1);
+                kp.blockDim = dim3(32);
+                kp.kernelParams = args;
+                cudaError_t e;
+                if (fresh) e = cudaGraphAddKernelNode(&pl->decode_node, pl->graph, prev ? &prev : nullptr, prev ? 1 : 0, &kp);
+                else e = cudaGraphExecKernelNodeSetParams(pl->graph_exec, pl->decode_node, &kp);
+                if (e != cudaSuccess) return cuda_fail(ctx, e, "CUDA graph node (MPE decode)");
+            }
+        }
         if (timing && pl->runs == 0)
             fprintf(stderr, "bnpp timing: resolving the wide steps' launches (contract_plan) %.3f ms, %llu launches, launch loop %.3f ms\n",
                     t_plan_steps, (unsigned long long)n_launched,
@@ -2021,6 +2248,7 @@ int bnpp_ve_plan_run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, 
                              const uint8_t *ev_dev, double *result_dev)
 {
     if (!pl || !pl->ctx || !result_dev || nb == 0) return BNPP_EINVAL;
+    if (pl->is_mpe) return fail(pl->ctx, BNPP_EINVAL, "MPE plan: batched runs are not supported");
     bnpp_ctx *ctx = pl->ctx;
     if ((int)n_obs != pl->n_obs) return fail(ctx, BNPP_EINVAL, "batched VE: n_obs differs from the plan's");
     if (n_obs && !ev_dev) return fail(ctx, BNPP_EINVAL, "batched VE: evidence matrix missing");

@@ -132,3 +132,17 @@ def fused_product_sum_out(ctx, factors, out_scope, elim_var):
     ctx.product_sum_out([(f.ptr, f.scope, f.cards, None) for f in factors], out.scope, out.cards, elim_var,
                         out.ptr, out.zptr)
     return out
+
+
+def fused_product_max_out(ctx, factors, out_scope, elim_var):
+    """One max-product step (MPE) in one kernel -> (factor over `out_scope` holding max_x of the product, device uint8
+    tensor of the first maximising x per entry).  The factor's partition slot is not written."""
+    cards = {}
+    for f in factors:
+        cards.update(zip(f.scope, f.cards))
+    out = DeviceFactor.empty(ctx, out_scope, [cards[v] for v in out_scope])
+    with torch.cuda.stream(ctx.torch_stream):
+        arg = torch.empty(max(1, out.size), dtype=torch.uint8, device=out.buf.device)
+    ctx.product_max_out([(f.ptr, f.scope, f.cards, None) for f in factors], out.scope, out.cards, elim_var,
+                        out.ptr, arg.data_ptr())
+    return out, arg[:out.size]

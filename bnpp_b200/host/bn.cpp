@@ -26,6 +26,7 @@ struct Flag { const char *text; const char *key; const char *help; };
 static const Flag kTasks[] = {
     {"-pr", "partition", "solve partition task"},
     {"-mar", "marginals", "solve marginals task"},
+    {"-mpe", "mpe", "solve most probable explanation task"},
 };
 static const Flag kOptions[] = {
     {"-ls", "logical-sampling", "compute partition using logical sampling"},
@@ -82,6 +83,18 @@ static void execute_partition()
     if (options["verbose"]) cout << ">> Computing partition for evidence ..." << endl;
     const double p = model->partition(evidence, options, uptime);
     cout << ">> Partition = " << p << endl;
+    cout << ">> Executed in " << uptime << "ms." << endl << endl;
+}
+
+static void execute_mpe()
+{
+    double uptime;
+    vector<unsigned> assignment;
+    const double p = model->mpe(evidence, options, assignment, uptime);
+    cout << ">> MPE = " << p << endl;
+    cout << ">> Assignment =";
+    for (unsigned x : assignment) cout << " " << x;
+    cout << endl;
     cout << ">> Executed in " << uptime << "ms." << endl << endl;
 }
 
@@ -278,9 +291,10 @@ int main(int argc, char *argv[])
         if (read_uai_evidence(evidence_filename, evidence)) return -2;
         if (options["verbose"] && !evidence.empty()) print_evidence(",\t");
     }
-    if (options["partition"] || options["marginals"]) {
+    if (options["partition"] || options["marginals"] || options["mpe"]) {
         if (options["partition"]) execute_partition();
         if (options["marginals"]) execute_marginals();
+        if (options["mpe"]) execute_mpe();
     } else {
         prompt();
     }

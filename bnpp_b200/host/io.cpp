@@ -156,6 +156,16 @@ int write_uai_pr(const std::string &filename, double partition)
     return out.good() ? 0 : -1;
 }
 
+int write_uai_mpe(const std::string &filename, const std::vector<unsigned> &assignment)
+{
+    std::ofstream out(filename);
+    if (!out.is_open()) return -1;
+    out << "MPE" << std::endl << 1 << std::endl << assignment.size();
+    for (unsigned x : assignment) out << " " << x;
+    out << std::endl;
+    return out.good() ? 0 : -1;
+}
+
 int write_uai_mar(const std::string &filename, const std::vector<const Factor*> &marginals,
                   const std::vector<unsigned> &cardinalities, const std::unordered_map<unsigned,unsigned> &evidence)
 {

@@ -26,6 +26,8 @@ void read_factors(std::ifstream &input_file, std::vector<Variable*> &variables, 
 // ..."), the form read_uai_evidence honours (code/io.cpp:157-180).  Numbers carry 6 significant digits like the
 // shipped files.  0 on success, -1 if the file cannot be written.
 int write_uai_pr(const std::string &filename, double partition);
+// UAI MPE solution file: "MPE", 1, then the number of variables and their values (extension: the reference writes none)
+int write_uai_mpe(const std::string &filename, const std::vector<unsigned> &assignment);
 int write_uai_mar(const std::string &filename, const std::vector<const Factor*> &marginals,
                   const std::vector<unsigned> &cardinalities, const std::unordered_map<unsigned,unsigned> &evidence);
 int write_uai_evidence(const std::string &filename, const std::unordered_map<unsigned,unsigned> &evidence);

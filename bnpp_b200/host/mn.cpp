@@ -2,6 +2,8 @@
 // output of the reference tool (code/mn.cpp:37-155).  Extension: the ordering flags
 // -ve [-mf|-wmf|-md] switch PR / MAR from the brute-force joint to device-resident
 // variable elimination (the reference offers VE on Markov nets only through its library).
+// Extension: the prompt command MPE|mpe prints the most probable explanation (log10 of its value
+// and the assignment) and, with -o, writes <prefix>.MPE.
 #include "io.hh"
 using namespace bn;
 
@@ -48,6 +50,19 @@ static void execute_partition()
     cout << ">> Executed in " << uptime << "ms." << endl << endl;
 }
 
+static void execute_mpe()
+{
+    double uptime;
+    vector<unsigned> assignment;
+    const double p = model->mpe(evidence, options, assignment, uptime);
+    cout << "MPE = " << log10(p) << endl;
+    cout << "Assignment =";
+    for (unsigned x : assignment) cout << " " << x;
+    cout << endl << endl;
+    if (!solution_prefix.empty() && write_uai_mpe(solution_prefix + ".MPE", assignment)) cerr << "Error: cannot write " << solution_prefix << ".MPE" << endl;
+    cout << ">> Executed in " << uptime << "ms." << endl << endl;
+}
+
 static void execute_marginals()
 {
     cout << ">> Marginals:" << endl;
@@ -73,7 +88,7 @@ static void prompt()
         for (const auto &e : evidence) cout << "Variable = " << e.first << ", Value = " << e.second << endl;
         cout << endl;
     }
-    const regex quit("quit"), pr("PR|pr|partition"), mar("MAR|mar|marginals");
+    const regex quit("quit"), pr("PR|pr|partition"), mar("MAR|mar|marginals"), mpe("MPE|mpe");
     cout << ">> Query prompt:" << endl;
     while (cin) {
         cout << "? ";
@@ -81,6 +96,7 @@ static void prompt()
         getline(cin, line);
         if (regex_match(line, pr)) execute_partition();
         else if (regex_match(line, mar)) execute_marginals();
+        else if (regex_match(line, mpe)) execute_mpe();
         else if (regex_match(line, quit)) break;
         else cout << "Error: not a valid query." << endl;
     }

@@ -6,6 +6,7 @@
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
+#include <cstring>
 #include <iostream>
 
 namespace bn {
@@ -244,6 +245,62 @@ std::vector<const Factor*> Model::marginals_ve(const std::unordered_map<unsigned
         marg.push_back(new Factor(new Domain(sc), values, 1.0));
     }
     return marg;
+}
+
+double Model::mpe(const std::unordered_map<unsigned,unsigned> &evidence, std::unordered_map<std::string,bool> &options,
+                  std::vector<unsigned> &assignment, double &uptime) const
+{
+    Stopwatch sw;
+    std::vector<const Factor*> factors(_factors.begin(), _factors.end());
+    std::vector<unsigned> ids, card;
+    for (const Variable *pv : _variables)
+        if (evidence.find(pv->id()) == evidence.end()) ids.push_back(pv->id());
+    for (const Variable *pv : _variables) card.push_back(pv->size());
+    if (options["min-fill"] || options["weighted-min-fill"] || options["min-degree"]) {
+        std::vector<std::vector<unsigned>> scopes;
+        for (const Factor *pf : factors) {
+            std::vector<unsigned> sc;
+            for (uint32_t id : pf->domain().ids())
+                if (evidence.find(id) == evidence.end()) sc.push_back(id);
+            scopes.push_back(sc);
+        }
+        bnpp::Heuristic h = bnpp::H_MIN_FILL;
+        if (options["min-degree"]) h = bnpp::H_MIN_DEGREE;
+        else if (options["weighted-min-fill"]) h = bnpp::H_WEIGHTED_MIN_FILL;
+        unsigned width = 0;
+        ids = bnpp::FastOrderer(scopes, card).ordering(ids, h, width);
+    }
+    std::vector<bnpp_scope> scopes(factors.size());
+    std::vector<const double*> tables(factors.size());
+    for (size_t i = 0; i < factors.size(); ++i) {
+        const Domain &d = factors[i]->domain();
+        scopes[i].rank = (int32_t)d.width();
+        scopes[i].var_id = d.ids().data();
+        scopes[i].card = d.cards().data();
+        tables[i] = factors[i]->device_data();
+    }
+    std::vector<uint32_t> obs_var, obs_val;
+    for (const auto &e : evidence) {
+        obs_var.push_back(e.first);
+        obs_val.push_back(e.second);
+    }
+    bnpp_ctx *ctx = gpu::ctx();
+    bnpp_ve_plan *plan = nullptr;
+    const int nvars = (int)_variables.size();
+    gpu::check(bnpp_mpe_plan_create(ctx, nvars, card.data(), (int)factors.size(), scopes.data(), (int)obs_var.size(),
+                                    obs_var.data(), (int)ids.size(), ids.data(), &plan), "bnpp_mpe_plan_create");
+    // [value, assignment as uint32 words]: one buffer, one download
+    double *res = nullptr;
+    gpu::check(bnpp_alloc(ctx, 1 + ((uint64_t)nvars + 1) / 2, &res), "bnpp_alloc");
+    gpu::check(bnpp_mpe_plan_run(plan, tables.data(), obs_val.data(), res, reinterpret_cast<uint32_t *>(res + 1)), "bnpp_mpe_plan_run");
+    std::vector<double> host(1 + ((size_t)nvars + 1) / 2);
+    gpu::check(bnpp_download(ctx, host.data(), res, host.size()), "bnpp_download");
+    bnpp_free(ctx, res);
+    bnpp_ve_plan_destroy(plan);
+    assignment.assign(nvars, 0);
+    std::memcpy(assignment.data(), host.data() + 1, sizeof(unsigned) * nvars);
+    uptime = sw.ms();
+    return host[0];
 }
 
 // ------------------------------------------------------------------------------------------

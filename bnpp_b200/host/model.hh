@@ -54,6 +54,12 @@ public:
     // Markov nets only through its library API, SURVEY §8c)
     double partition_ve(const std::unordered_map<unsigned,unsigned> &evidence, std::unordered_map<std::string,bool> &options) const;
     std::vector<const Factor*> marginals_ve(const std::unordered_map<unsigned,unsigned> &evidence, std::unordered_map<std::string,bool> &options) const;
+    // MPE (no reference counterpart): the most probable assignment of the unobserved variables given the evidence
+    // (assignment[id]; observed variables keep their evidence value) and its value max_x prod_f f(x, e), by
+    // max-product variable elimination on the device.  The order follows the -mf / -wmf / -md flags as in
+    // partition_ve, else variables in id order.  Ties go to the lowest values.
+    double mpe(const std::unordered_map<unsigned,unsigned> &evidence, std::unordered_map<std::string,bool> &options,
+               std::vector<unsigned> &assignment, double &uptime) const;
 
 protected:
     std::string _name;

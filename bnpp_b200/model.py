@@ -45,6 +45,9 @@ def _declare(L):
     L.bnpp_ve_plan_step_stats.argtypes = [ctypes.c_void_p, ctypes.c_uint64, P(ctypes.c_float), capi.c_u64p, capi.c_u64p,
                                           P(ctypes.c_int32)]
     L.bnpp_ve_plan_step_kernel.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_char_p, ctypes.c_size_t]
+    L.bnpp_mpe_plan_create.argtypes = [ctypes.c_void_p, ctypes.c_int, capi.c_u32p, ctypes.c_int, P(capi.Scope), ctypes.c_int,
+                                       capi.c_u32p, ctypes.c_int, capi.c_u32p, P(ctypes.c_void_p)]
+    L.bnpp_mpe_plan_run.argtypes = [ctypes.c_void_p, P(ctypes.c_void_p), capi.c_u32p, ctypes.c_void_p, ctypes.c_void_p]
     L._ve_declared = True
 
 
@@ -209,6 +212,36 @@ class MarPlan(VEPlan):
         self.n_launches, self.union_entries, self.bytes, self.peak_bytes, self.max_step_entries = [v.value for v in vals]
 
 
+class MPEPlan(VEPlan):
+    """bnpp_mpe_plan: max-product variable elimination over the schedule of a VEPlan, then an on-device decode of the
+    most probable assignment.  `order` must cover every unobserved variable.  ctx.h may be None: a dry plan."""
+
+    def __init__(self, ctx, cards, scopes, observed, order, _arr=None):
+        self.ctx = ctx
+        L = ctx.L
+        _declare(L)
+        arr, self._keep = (_arr, None) if _arr is not None else _scopes(scopes, cards)
+        self.observed = list(observed)
+        self.nvars = len(cards)
+        c, ov, od = capi._u32(cards), capi._u32(self.observed), capi._u32(order)
+        h = ctypes.c_void_p()
+        ctx.check(L.bnpp_mpe_plan_create(ctx.h, len(cards), ctypes.cast(c, capi.c_u32p), len(scopes), arr,
+                                         len(self.observed), ctypes.cast(ov, capi.c_u32p), len(order),
+                                         ctypes.cast(od, capi.c_u32p), ctypes.byref(h)))
+        self.h = h
+        self.result_size = 1
+        vals = [ctypes.c_uint64() for _ in range(5)]
+        ctx.check(L.bnpp_ve_plan_info(h, None, None, None, *[ctypes.byref(v) for v in vals]))
+        self.n_launches, self.union_entries, self.bytes, self.peak_bytes, self.max_step_entries = [v.value for v in vals]
+
+    def run_mpe(self, table_ptrs, obs_val, value_ptr, assignment_ptr):
+        """value_ptr: device double; assignment_ptr: device uint32 [nvars].  Asynchronous."""
+        tp = (ctypes.c_void_p * max(1, len(table_ptrs)))(*table_ptrs)
+        ov = capi._u32(obs_val)
+        self.ctx.check(self.ctx.L.bnpp_mpe_plan_run(self.h, tp, ctypes.cast(ov, capi.c_u32p), ctypes.c_void_p(value_ptr),
+                                                    ctypes.c_void_p(assignment_ptr)))
+
+
 class BN:
     """Model(name, variables, factors) with the factors resident in HBM (code/model.cpp:14-19)."""
 
@@ -267,7 +300,9 @@ class BN:
     MAX_PLANS = 64      # every plan keeps its device arena, offset tables and replay graph: the cache is bounded (oldest out)
 
     def plan(self, observed, order):
-        key = (tuple(observed), tuple(order))
+        return self._cached_plan((tuple(observed), tuple(order)), VEPlan, observed, order)
+
+    def _cached_plan(self, key, cls, observed, order):
         p = self._plans.get(key)
         if p is None:
             while len(self._plans) >= self.MAX_PLANS:
@@ -275,7 +310,7 @@ class BN:
                 old = self._plans.pop(old_key)
                 self._batch_plans = {k: v for k, v in self._batch_plans.items() if v is not old}
                 old.close()
-            p = VEPlan(self.ctx, self.cards, self.scopes, observed, order, _arr=self._scope_arr)
+            p = cls(self.ctx, self.cards, self.scopes, observed, order, _arr=self._scope_arr)
             self._plans[key] = p
         return p
 
@@ -349,6 +384,42 @@ class BN:
         assert z0 == z1 or (comm is not None and abs(z0 - z1) <= 1e-12 * abs(z1))     # code/model.cpp:288
         self.last_timing = {"order_ms": (t1 - t0) * 1e3, "plan_ms": (t2 - t1) * 1e3, "run_ms": (t3 - t2) * 1e3}
         return z1, (time.perf_counter() - t0) * 1e3
+
+    def mpe(self, evidence=None, heuristic=None):
+        """Most probable explanation (no reference counterpart) -> (value, assignment list, uptime_ms).
+        value = max over the unobserved variables of the product of every CPT conditioned on the evidence, i.e.
+        P(x*, e), not normalised; assignment[v] is the evidence value of an observed v.  Ties go to the lowest values.
+        The order is the one `partition` uses (heuristic None: variables in id order)."""
+        t0 = time.perf_counter()
+        evidence = dict(evidence or {})
+        observed = sorted(evidence)
+        okey = (tuple(observed), heuristic)
+        order = self._order_cache.get(okey)
+        if order is None:
+            variables = [v for v in range(self.nvars) if v not in evidence]
+            order, _ = self.order(variables, evidence, heuristic)
+            if len(self._order_cache) >= self.MAX_PLANS:
+                self._order_cache.pop(next(iter(self._order_cache)))
+            self._order_cache[okey] = order
+        t1 = time.perf_counter()
+        p = self._cached_plan(("mpe", tuple(observed), tuple(order)), MPEPlan, observed, order)
+        t2 = time.perf_counter()
+        n = self.nvars
+        if getattr(self, "_mpe_buf", None) is None or self._mpe_buf.numel() != 2 + n:
+            # [value (two uint32 words), assignment[nvars]]: one device-to-host copy of 1 + nvars words
+            with torch.cuda.stream(self.ctx.torch_stream):
+                self._mpe_buf = torch.empty(2 + n, dtype=torch.int32, device=self._dev.device)
+                self._mpe_host = torch.empty(2 + n, dtype=torch.int32).pin_memory()
+        p.run_mpe(self.table_ptrs, [evidence[v] for v in observed], self._mpe_buf.data_ptr(), self._mpe_buf.data_ptr() + 8)
+        with torch.cuda.stream(self.ctx.torch_stream):
+            self._mpe_host.copy_(self._mpe_buf, non_blocking=True)
+        self.ctx.sync()
+        t3 = time.perf_counter()
+        host = self._mpe_host.numpy()
+        value = float(host[:2].view(np.float64)[0])
+        assignment = [int(x) for x in host[2:].view(np.uint32)]
+        self.last_timing = {"order_ms": (t1 - t0) * 1e3, "plan_ms": (t2 - t1) * 1e3, "run_ms": (t3 - t2) * 1e3}
+        return value, assignment, (time.perf_counter() - t0) * 1e3
 
     def partition_batch(self, observed, values, heuristic="mf", host_values=None):
         """PR for a batch of evidence sets sharing the observed ids (config 5).

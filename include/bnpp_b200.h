@@ -119,6 +119,15 @@ int bnpp_product_sum_out(bnpp_ctx *ctx, int k, const bnpp_operand *operands,
                          const bnpp_scope *out_scope, int64_t elim_var, int divide,
                          double *out_dev, double *z_dev);
 
+/* Max-product step (MPE; no reference counterpart):
+ *   out[o] = max_x prod_k operand_k[pi_k(o, x)],  arg[o] = the first x attaining it (uint8)
+ * Products are formed as in bnpp_product_sum_out.  The maximum starts at x = 0 and x replaces it
+ * only if its product is strictly greater: ties keep the lowest x and a NaN never replaces a
+ * number.  argmax_dev is dense over out_scope like out_dev.  elim_var < 0 or an eliminated
+ * variable with more than 255 values returns BNPP_EINVAL.  No partition is computed. */
+int bnpp_product_max_out(bnpp_ctx *ctx, int k, const bnpp_operand *operands, const bnpp_scope *out_scope,
+                         int64_t elim_var, double *out_dev, uint8_t *argmax_dev);
+
 /* ---- reference-shaped single ops ---------------------------------------------- */
 /* Factor::product / Factor::divide, code/factor.cpp:117-180. out is dense over
  * bnpp_union_scope(a, b). */
@@ -194,6 +203,23 @@ int bnpp_ve_plan_info(const bnpp_ve_plan *plan, int32_t *result_rank, uint32_t *
  * Factor::operator[], code/factor.cpp:83-95). */
 int bnpp_ve_plan_run(bnpp_ve_plan *plan, const double *const *tables_dev, const uint32_t *obs_val,
                      double *result_dev, double *z_dev);
+/* MPE (no reference counterpart): the most probable assignment of every unobserved variable given
+ * the evidence, and its value  max_x prod_f f(x, e)  -- P(x*, e) for a Bayesian network, not
+ * normalised.  The steps are those bnpp_ve_plan_create builds for the same inputs with every sum
+ * replaced by a max (rule of bnpp_product_max_out); each eliminating step keeps its argmax table
+ * (one byte per output entry, counted in peak_bytes) and a one-thread decode walks them backwards.
+ * `order` must cover every unobserved variable that some scope mentions, and an eliminated
+ * variable may have at most 255 values; else BNPP_EINVAL.  ctx may be NULL (a dry plan).
+ * Runs are launch-per-bucket (never the K9 / K10 paths); from the second run on a run is one
+ * replay of a CUDA graph that includes the decode.
+ * run: assignment_dev[nvars] receives one uint32 per variable id: the evidence value for an
+ * observed variable, 0 for a variable no factor mentions; value_dev one double.  Zero-probability
+ * evidence gives value 0 and the lowest values.  An evidence value out of range returns
+ * BNPP_EINVAL.  bnpp_ve_plan_run / _run_batched / _run_sharded return BNPP_EINVAL on an MPE plan. */
+int bnpp_mpe_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfac, const bnpp_scope *scopes,
+                         int n_obs, const uint32_t *obs_var, int n_order, const uint32_t *order, bnpp_ve_plan **out);
+int bnpp_mpe_plan_run(bnpp_ve_plan *plan, const double *const *tables_dev, const uint32_t *obs_val,
+                      double *value_dev, uint32_t *assignment_dev);
 /* entries of the result table a run writes (PR: 1; marginals plan: the layout's total) */
 int bnpp_ve_plan_result_size(const bnpp_ve_plan *plan, uint64_t *n);
 /* BN::marginals (code/model.cpp:320-339) for EVERY variable in one plan: two passes over the
