@@ -9,6 +9,7 @@
 //     base_k(b) = sum_j stride_kj * value[b][obs_kj]
 // which is the whole of Factor::conditioning (code/factor.cpp:214-242) here.  One launch
 // per bucket for the entire batch; nothing is materialised per evidence set.
+#include <algorithm>
 #include <cstring>
 #include <vector>
 
@@ -16,8 +17,6 @@
 #include "common.cuh"
 
 namespace bnpp {
-
-constexpr int kMaxObsPerOperand = 8;
 
 struct BOperand {
     const double *ptr;
@@ -240,6 +239,53 @@ int sanitize_evidence_launch(bnpp_ctx *ctx, const uint8_t *in, uint8_t *out, uin
     BNPP_CUDA(ctx, cudaGetLastError());
     ctx->launches++;
     return BNPP_OK;
+}
+
+// The evidence base of a CPT with more observed axes than a K8 operand holds, sum_j stride_j * value[obs_j], for
+// every set: up to kMaxObsPerOperand axes per launch, added to `acc`; the last launch (digits != 0) writes the sum as
+// `digits` base-256 digits into the evidence columns digit_col, digit_col + 1, ... of the column-major matrix `ev`.
+struct ObsAxes {
+    uint32_t n;
+    uint32_t stride[kMaxObsPerOperand];
+    uint32_t col[kMaxObsPerOperand];
+};
+
+__global__ void evidence_digits(const __grid_constant__ ObsAxes a, uint8_t *ev, uint32_t nb, uint32_t *__restrict__ acc, int first,
+                                uint32_t digit_col, uint32_t digits)
+{
+    for (uint32_t b = blockIdx.x * blockDim.x + threadIdx.x; b < nb; b += gridDim.x * blockDim.x) {
+        uint32_t e = first ? 0 : acc[b];
+        for (uint32_t j = 0; j < a.n; ++j) e += a.stride[j] * ev[(uint64_t)a.col[j] * nb + b];
+        if (!digits) acc[b] = e;
+        for (uint32_t d = 0; d < digits; ++d) ev[(uint64_t)(digit_col + d) * nb + b] = (uint8_t)(e >> (8 * d));
+    }
+}
+
+int evidence_digits_launch(bnpp_ctx *ctx, const std::vector<std::pair<int64_t, int>> &obs, uint8_t *ev_dev, uint32_t nb,
+                           uint32_t digit_col, uint32_t digits)
+{
+    if (!nb || obs.empty() || !digits) return BNPP_OK;
+    double *acc = nullptr;
+    if (obs.size() > (size_t)kMaxObsPerOperand) {
+        const int rc = bnpp_alloc(ctx, nb / 2 + 1, &acc);
+        if (rc != BNPP_OK) return rc;
+    }
+    const unsigned blocks = (unsigned)std::min<uint64_t>((nb + 255) / 256, 4096);
+    for (size_t j0 = 0; j0 < obs.size(); j0 += kMaxObsPerOperand) {
+        ObsAxes a;
+        memset(&a, 0, sizeof a);
+        a.n = (uint32_t)std::min<size_t>(kMaxObsPerOperand, obs.size() - j0);
+        for (uint32_t j = 0; j < a.n; ++j) {
+            a.stride[j] = (uint32_t)obs[j0 + j].first;
+            a.col[j] = (uint32_t)obs[j0 + j].second;
+        }
+        const bool last = j0 + a.n == obs.size();
+        evidence_digits<<<blocks, 256, 0, ctx->stream>>>(a, ev_dev, nb, reinterpret_cast<uint32_t *>(acc), j0 == 0, digit_col,
+                                                         last ? digits : 0);
+        BNPP_CUDA(ctx, cudaGetLastError());
+        ctx->launches++;
+    }
+    return bnpp_free(ctx, acc);
 }
 
 typedef void (*batched_fn)(const BParams);

@@ -8,6 +8,8 @@ struct bnpp_ctx;
 
 namespace bnpp {
 
+constexpr int kMaxObsPerOperand = 8;    // observed axes one K8 operand reads its evidence base through
+
 // One operand of a batched elimination step: an intermediate [entries][batch] or a resident
 // CPT view read through a per-evidence-set base offset.
 struct BatchedOperandDesc {
@@ -27,5 +29,10 @@ int contract_batched_step(bnpp_ctx *ctx, int k, const BatchedOperandDesc *ops, c
 // variable's cardinality (card_dev[n_obs]) by 0 and raising BNPP_STATUS_BAD_EVIDENCE
 int sanitize_evidence_launch(bnpp_ctx *ctx, const uint8_t *in, uint8_t *out, uint32_t nb, uint32_t n_obs, const uint32_t *card_dev,
                              bool transpose);
+// a CPT with more than kMaxObsPerOperand observed axes: its evidence base per set, sum of stride * value over `obs`
+// (stride, column), written as `digits` base-256 digits into columns digit_col.. of the column-major [cols][nb]
+// matrix ev_dev, so that K8 reads the CPT through those columns with strides 1, 256, ...
+int evidence_digits_launch(bnpp_ctx *ctx, const std::vector<std::pair<int64_t, int>> &obs, uint8_t *ev_dev, uint32_t nb,
+                           uint32_t digit_col, uint32_t digits);
 
 }  // namespace bnpp

@@ -2340,9 +2340,21 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
     static const std::vector<int64_t> dense;
     static const std::vector<std::pair<int64_t, int>> no_obs;
     int rc = BNPP_OK;
+    // a CPT with more observed axes than a K8 operand holds is read through the base-256 digits of its evidence base,
+    // extra evidence columns after the plan's own: (stride, column) per digit instead of its observed axes
+    std::vector<std::vector<std::pair<int64_t, int>>> digit_obs(pl->f.size());
+    uint32_t n_cols = n_obs;
+    for (size_t i = 0; i < pl->f.size(); ++i) {
+        const PlanFactor &pf = pl->f[i];
+        if (pf.src < 0 || pf.obs.size() <= (size_t)kMaxObsPerOperand) continue;
+        uint64_t max_base = 0;
+        for (auto &o : pf.obs) max_base += (uint64_t)o.first * (pl->obs_card[o.second] - 1);
+        if (max_base >> 32) return fail(ctx, BNPP_ETOOBIG, "batched VE: evidence base of a table beyond 32 bits");
+        for (uint32_t d = 0; d == 0 || (d < 4 && (max_base >> (8 * d))); ++d) digit_obs[i].push_back({1ll << (8 * d), (int)n_cols++});
+    }
     // evidence columns contiguous over the sets: every thread of a warp then reads neighbouring bytes
     double *evt_store = nullptr;
-    rc = bnpp_alloc(ctx, ((uint64_t)nb * (n_obs ? n_obs : 1) + 7) / 8 + 1, &evt_store);
+    rc = bnpp_alloc(ctx, ((uint64_t)nb * (n_cols ? n_cols : 1) + 7) / 8 + 1, &evt_store);
     if (rc != BNPP_OK) return rc;
     uint8_t *evt = reinterpret_cast<uint8_t *>(evt_store);
     if (pl->offtab_host.size() != pl->steps.size()) {
@@ -2350,6 +2362,9 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
         pl->offtab_dev.assign(pl->steps.size(), nullptr);
     }
     rc = sanitize_evidence_launch(ctx, ev_dev, evt, nb, n_obs, pl->obs_card_dev, true);
+    for (size_t i = 0; i < pl->f.size() && rc == BNPP_OK; ++i)
+        if (!digit_obs[i].empty())
+            rc = evidence_digits_launch(ctx, pl->f[i].obs, evt, nb, (uint32_t)digit_obs[i][0].second, (uint32_t)digit_obs[i].size());
     for (uint32_t b0 = 0; b0 < nb && rc == BNPP_OK; b0 += slice) {
         const uint32_t cur = std::min(slice, nb - b0);
         std::vector<double *> owned(pl->f.size(), nullptr);
@@ -2363,7 +2378,7 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
                 ops[q].var = &pf.var;
                 ops[q].card = &pf.card;
                 ops[q].stride = pf.src < 0 ? &dense : &pf.stride;
-                ops[q].obs = pf.src < 0 ? &no_obs : &pf.obs;
+                ops[q].obs = pf.src < 0 ? &no_obs : digit_obs[st.operands[q]].empty() ? &pf.obs : &digit_obs[st.operands[q]];
             }
             double *dst;
             const std::vector<uint32_t> *ov, *oc;
@@ -2379,7 +2394,7 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
                 if (rc != BNPP_OK) break;
                 dst = owned[st.out];
             }
-            rc = contract_batched_step(ctx, (int)st.operands.size(), ops, *ov, *oc, st.elim, cur, evt + b0, nb, n_obs, dst,
+            rc = contract_batched_step(ctx, (int)st.operands.size(), ops, *ov, *oc, st.elim, cur, evt + b0, nb, n_cols, dst,
                                        &pl->offtab_host[s], &pl->offtab_dev[s]);
             for (int id : st.operands)
                 if (owned[id] && pl->f[id].last_use == (int)s) {
