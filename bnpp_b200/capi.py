@@ -28,7 +28,7 @@ EXPORTS = [
     "bnpp_tuning_set", "bnpp_tuning_get", "bnpp_ve_plan_result_size", "bnpp_ve_plan_set_normalize",
     "bnpp_mar_plan_normalize", "bnpp_fg_reset", "bnpp_ve_plan_launches",
     "bnpp_sampler_create", "bnpp_sampler_destroy", "bnpp_sampler_logical", "bnpp_sampler_likelihood",
-    "bnpp_product_max_out", "bnpp_mpe_plan_create", "bnpp_mpe_plan_run",
+    "bnpp_product_max_out", "bnpp_mpe_plan_create", "bnpp_mpe_plan_run", "bnpp_mpe_plan_run_batched",
 ]
 
 

@@ -38,13 +38,20 @@ struct BParams {
     FastDiv nbdiv;
 };
 
+// the max-product variant (MPE): out = the maximum over the eliminated variable (start at x = 0, a later x replaces it
+// only if its product is strictly greater -- contract.cu's rule), arg = [n_out][nb] bytes, the first maximising x
+struct BMaxParams {
+    BParams p;
+    uint8_t *arg;
+};
+
 // A thread owns VB evidence sets (2 when the slice is even: 16-byte accesses on the batched
 // tables) and walks `oc` consecutive output entries for them.  What depends only on the sets
 // -- the evidence base of every resident CPT -- is computed once per thread, what depends only
 // on the output entry -- operand offsets -- comes from a small table that a warp reads as one
 // broadcast (all lanes share the entry, the batch being the fastest axis).
-template <int K, int VB>
-__global__ void __launch_bounds__(kBlock) contract_batched(const __grid_constant__ BParams p)
+template <int K, int VB, bool MAX>
+__device__ __forceinline__ void batched_entries(const BParams &p, uint8_t *arg)
 {
     const uint32_t nbv = p.nb / VB;
     const uint64_t total = (uint64_t)p.n_chunks * nbv;
@@ -90,6 +97,9 @@ __global__ void __launch_bounds__(kBlock) contract_batched(const __grid_constant
                 for (int v = 0; v < VB; ++v) src[k][v] = base[k][v] + off;
             }
             double acc[VB];
+            uint32_t best[VB];
+#pragma unroll
+            for (int w = 0; w < VB; ++w) best[w] = 0;
             for (uint32_t x = 0; x < p.cx; ++x) {
                 double v[VB];
 #pragma unroll
@@ -107,21 +117,44 @@ __global__ void __launch_bounds__(kBlock) contract_batched(const __grid_constant
                     for (int w = 0; w < VB; ++w) v[w] = (k == 0) ? t[w] : __dmul_rn(v[w], t[w]);
                 }
 #pragma unroll
-                for (int w = 0; w < VB; ++w) acc[w] = (x == 0) ? v[w] : __dadd_rn(acc[w], v[w]);
+                for (int w = 0; w < VB; ++w) {
+                    if (!MAX) {
+                        acc[w] = (x == 0) ? v[w] : __dadd_rn(acc[w], v[w]);
+                    } else if (x == 0 || v[w] > acc[w]) {
+                        acc[w] = v[w];
+                        best[w] = x;
+                    }
+                }
             }
             double *dst = p.out + ((uint64_t)o * p.nb + b);
             if (VB == 2) *reinterpret_cast<double2 *>(dst) = make_double2(acc[0], acc[VB - 1]);
             else dst[0] = acc[0];
+            if (MAX) {
+#pragma unroll
+                for (int w = 0; w < VB; ++w) arg[(uint64_t)o * p.nb + b + w] = (uint8_t)best[w];
+            }
         }
     }
+}
+
+template <int K, int VB>
+__global__ void __launch_bounds__(kBlock) contract_batched(const __grid_constant__ BParams p)
+{
+    batched_entries<K, VB, false>(p, nullptr);
+}
+
+template <int K, int VB>
+__global__ void __launch_bounds__(kBlock) contract_batched_max(const __grid_constant__ BMaxParams q)
+{
+    batched_entries<K, VB, true>(q.p, q.arg);
 }
 
 // Binary eliminated variable (every BASELINE network): UO output entries of a thread are
 // processed together -- all their loads are issued before the first multiply, so one wave of
 // CTAs moves UO times the bytes per memory round trip (the launch is a handful of waves long,
 // each paying a full DRAM latency).
-template <int K, int VB, int UO>
-__global__ void __launch_bounds__(kBlock) contract_batched_bin(const __grid_constant__ BParams p)
+template <int K, int VB, int UO, bool MAX>
+__device__ __forceinline__ void batched_bin_entries(const BParams &p, uint8_t *arg)
 {
     const uint32_t nbv = p.nb / VB;
     const uint64_t total = (uint64_t)p.n_chunks * nbv;
@@ -191,7 +224,13 @@ __global__ void __launch_bounds__(kBlock) contract_batched_bin(const __grid_cons
                         v0 = __dmul_rn(v0, t[i][k][0][w]);
                         v1 = __dmul_rn(v1, t[i][k][1][w]);
                     }
-                    acc[w] = __dadd_rn(v0, v1);
+                    if (MAX) {
+                        const bool gt = v1 > v0;
+                        acc[w] = gt ? v1 : v0;
+                        arg[(uint64_t)(o0 + i) * p.nb + b + w] = (uint8_t)gt;
+                    } else {
+                        acc[w] = __dadd_rn(v0, v1);
+                    }
                 }
                 double *dst = p.out + ((uint64_t)(o0 + i) * p.nb + b);
                 if (VB == 2) *reinterpret_cast<double2 *>(dst) = make_double2(acc[0], acc[VB - 1]);
@@ -199,6 +238,18 @@ __global__ void __launch_bounds__(kBlock) contract_batched_bin(const __grid_cons
             }
         }
     }
+}
+
+template <int K, int VB, int UO>
+__global__ void __launch_bounds__(kBlock) contract_batched_bin(const __grid_constant__ BParams p)
+{
+    batched_bin_entries<K, VB, UO, false>(p, nullptr);
+}
+
+template <int K, int VB, int UO>
+__global__ void __launch_bounds__(kBlock) contract_batched_bin_max(const __grid_constant__ BMaxParams q)
+{
+    batched_bin_entries<K, VB, UO, true>(q.p, q.arg);
 }
 
 // [nb][n_obs] (one row per evidence set, as the caller has it) -> [n_obs][nb] (transpose != 0) or a copy in place
@@ -289,6 +340,7 @@ int evidence_digits_launch(bnpp_ctx *ctx, const std::vector<std::pair<int64_t, i
 }
 
 typedef void (*batched_fn)(const BParams);
+typedef void (*batched_max_fn)(const BMaxParams);
 
 template <int VB>
 static batched_fn pick_batched_bin(int K, int &uo)
@@ -315,10 +367,35 @@ static batched_fn pick_batched_v(int K)
     }
 }
 
+template <int VB>
+static batched_max_fn pick_batched_bin_max(int K, int &uo)
+{
+    switch (K) {
+    case 1: uo = 4; return contract_batched_bin_max<1, VB, 4>;
+    case 2: uo = 4; return contract_batched_bin_max<2, VB, 4>;
+    case 3: uo = 2; return contract_batched_bin_max<3, VB, 2>;
+    case 4: uo = 2; return contract_batched_bin_max<4, VB, 2>;
+    default: uo = 0; return nullptr;
+    }
+}
+
+template <int VB>
+static batched_max_fn pick_batched_v_max(int K)
+{
+    switch (K) {
+    case 1: return contract_batched_max<1, VB>;
+    case 2: return contract_batched_max<2, VB>;
+    case 3: return contract_batched_max<3, VB>;
+    case 4: return contract_batched_max<4, VB>;
+    case 5: return contract_batched_max<5, VB>;
+    default: return contract_batched_max<6, VB>;
+    }
+}
+
 int contract_batched_step(bnpp_ctx *ctx, int k, const BatchedOperandDesc *ops, const std::vector<uint32_t> &out_var,
                           const std::vector<uint32_t> &out_card, int64_t elim, uint32_t nb, const uint8_t *ev_dev,
                           uint32_t ev_stride, uint32_t n_obs, double *out_dev, std::vector<uint32_t> *offtab_host,
-                          uint32_t **offtab_dev)
+                          uint32_t **offtab_dev, uint8_t *arg_dev)
 {
     if (k < 1 || k > kMaxK) return fail(ctx, BNPP_ERANK, "batched step: operand count");
     BParams p;
@@ -400,8 +477,15 @@ int contract_batched_step(bnpp_ctx *ctx, int k, const BatchedOperandDesc *ops, c
     // binary eliminated variable with at most 4 operands: the unrolled variant
     int uo = 0;
     batched_fn fn = nullptr;
-    if (cx == 2) fn = (vb == 2) ? pick_batched_bin<2>(k, uo) : pick_batched_bin<1>(k, uo);
-    if (!fn) fn = (vb == 2) ? pick_batched_v<2>(k) : pick_batched_v<1>(k);
+    batched_max_fn fn_max = nullptr;
+    const bool max_mode = arg_dev && elim >= 0;
+    if (max_mode) {
+        if (cx == 2) fn_max = (vb == 2) ? pick_batched_bin_max<2>(k, uo) : pick_batched_bin_max<1>(k, uo);
+        if (!fn_max) fn_max = (vb == 2) ? pick_batched_v_max<2>(k) : pick_batched_v_max<1>(k);
+    } else {
+        if (cx == 2) fn = (vb == 2) ? pick_batched_bin<2>(k, uo) : pick_batched_bin<1>(k, uo);
+        if (!fn) fn = (vb == 2) ? pick_batched_v<2>(k) : pick_batched_v<1>(k);
+    }
     // about one resident wave of threads, each walking `oc` consecutive output entries
     const uint64_t want_threads = (uint64_t)ctx->sm_count * (uo ? 768 : 2048);
     uint64_t oc = (n_out * (nb / vb) + want_threads - 1) / want_threads;
@@ -414,7 +498,14 @@ int contract_batched_step(bnpp_ctx *ctx, int k, const BatchedOperandDesc *ops, c
     uint64_t blocks = (total + kBlock - 1) / kBlock;
     const uint64_t cap = (uint64_t)ctx->sm_count * 8;
     if (blocks > cap) blocks = cap;
-    fn<<<(unsigned)blocks, kBlock, 0, ctx->stream>>>(p);
+    if (max_mode) {
+        BMaxParams q;
+        q.p = p;
+        q.arg = arg_dev;
+        fn_max<<<(unsigned)blocks, kBlock, 0, ctx->stream>>>(q);
+    } else {
+        fn<<<(unsigned)blocks, kBlock, 0, ctx->stream>>>(p);
+    }
     BNPP_CUDA(ctx, cudaGetLastError());
     ctx->launches++;
     return BNPP_OK;

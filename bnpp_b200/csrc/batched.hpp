@@ -23,7 +23,9 @@ struct BatchedOperandDesc {
 int contract_batched_step(bnpp_ctx *ctx, int k, const BatchedOperandDesc *ops, const std::vector<uint32_t> &out_var,
                           const std::vector<uint32_t> &out_card, int64_t elim, uint32_t nb, const uint8_t *ev_dev,
                           uint32_t ev_stride, uint32_t n_obs, double *out_dev, std::vector<uint32_t> *offtab_host,
-                          uint32_t **offtab_dev);
+                          uint32_t **offtab_dev, uint8_t *arg_dev = nullptr);
+// arg_dev != nullptr and elim >= 0: a max-product step (MPE), the first maximising value of the eliminated variable for
+// output entry o and set b at arg_dev[o * nb + b]
 // ev_dev above is COLUMN-major ([n_obs][ev_stride], first set of the slice at ev_dev[0]); this turns the
 // caller's row-major [nb][n_obs] matrix into it (transpose) or copies it, replacing values outside their
 // variable's cardinality (card_dev[n_obs]) by 0 and raising BNPP_STATUS_BAD_EVIDENCE

@@ -18,6 +18,10 @@
 // Per entry the arithmetic is that of contract.cu / batched.cu -- operands multiplied in bucket
 // order with __dmul_rn, values of the eliminated variable added in index order with __dadd_rn
 // -- so a result is bit-identical to the launch-per-bucket paths.
+// MAX (ve_fused_max, the batch engine of MPE plans): the same products, the maximum over the eliminated variable by the
+// rule of contract.cu's max-product kernels (start at x = 0, a later x replaces it only if its product is strictly
+// greater: ties keep the lowest x, a NaN never replaces a number), and the argmax byte of every output entry of a
+// kFusedMax step in global memory -- ~14 KB of argmax per set of config 5 would not fit in shared memory.
 #include <cstdlib>
 #include <map>
 #include <mutex>
@@ -57,22 +61,25 @@ struct Dest {
     uint64_t stride;
     uint32_t out_off;   // arena destination: element offset
     bool store;
+    uint8_t *arg;       // MAX, != nullptr: the argmax of entry o goes to arg[o * arg_stride]
+    uint32_t arg_stride;
 };
 
-template <int SPW>
-__device__ __forceinline__ void put(const SetView<SPW> &v, const Dest &d, uint32_t o, double val)
+template <int SPW, bool MAX = false>
+__device__ __forceinline__ void put(const SetView<SPW> &v, const Dest &d, uint32_t o, double val, uint32_t best = 0)
 {
     if (d.result) {
         if (d.store) d.result[(uint64_t)o * d.stride] = val;
     } else {
         arena_smem[v.at(d.out_off + o)] = val;
     }
+    if (MAX && d.arg && d.store) d.arg[(uint64_t)o * d.arg_stride] = (uint8_t)best;
 }
 
 // Binary eliminated variable, every arena operand with the variable at stride 1 on an even
 // offset (a 16-byte pair), AMASK = which operands are arena tables -- the shape of every bucket
 // of an all-binary network.  Two output entries per trip, all loads of both before the math.
-template <int K, unsigned AMASK, int G, int SPW>
+template <int K, unsigned AMASK, int G, int SPW, bool MAX>
 __device__ __forceinline__ double entries_pairs(const SetView<SPW> &v, const Operands &op, const uint32_t *__restrict__ tab,
                                                 uint32_t n_out, uint32_t lane, const Dest &d)
 {
@@ -109,6 +116,12 @@ __device__ __forceinline__ double entries_pairs(const SetView<SPW> &v, const Ope
             y0 = __dmul_rn(y0, b0[q]);
             y1 = __dmul_rn(y1, b1[q]);
         }
+        if (MAX) {
+            const bool ga = x1 > x0, gb = y1 > y0;
+            put<SPW, true>(v, d, o0, ga ? x1 : x0, ga);
+            if (two) put<SPW, true>(v, d, o1, gb ? y1 : y0, gb);
+            continue;
+        }
         const double ra = __dadd_rn(x0, x1), rb = __dadd_rn(y0, y1);
         put<SPW>(v, d, o0, ra);
         zacc = __dadd_rn(zacc, ra);
@@ -121,7 +134,7 @@ __device__ __forceinline__ double entries_pairs(const SetView<SPW> &v, const Ope
 }
 
 // any cardinality, any operand layout; amask: which operands are arena tables
-template <int K, int G, int SPW>
+template <int K, int G, int SPW, bool MAX>
 __device__ __forceinline__ double entries_any(const SetView<SPW> &v, const Operands &op, uint32_t amask,
                                               const uint32_t *__restrict__ tab, uint32_t n_out, uint32_t cx, uint32_t lane,
                                               const Dest &d)
@@ -132,6 +145,7 @@ __device__ __forceinline__ double entries_any(const SetView<SPW> &v, const Opera
 #pragma unroll
         for (int q = 0; q < K; ++q) off[q] = __ldg(tab + (size_t)q * n_out + o);
         double acc = 0.0;
+        uint32_t best = 0;
         for (uint32_t x = 0; x < cx; ++x) {
             double val = 0.0;
 #pragma unroll
@@ -140,7 +154,16 @@ __device__ __forceinline__ double entries_any(const SetView<SPW> &v, const Opera
                 const double t = ((amask >> q) & 1u) ? arena_smem[v.at(op.base[q] + e)] : __ldg(op.cpt[q] + e);
                 val = (q == 0) ? t : __dmul_rn(val, t);
             }
-            acc = (x == 0) ? val : __dadd_rn(acc, val);
+            if (!MAX) {
+                acc = (x == 0) ? val : __dadd_rn(acc, val);
+            } else if (x == 0 || val > acc) {
+                acc = val;
+                best = x;
+            }
+        }
+        if (MAX) {
+            put<SPW, true>(v, d, o, acc, best);
+            continue;
         }
         put<SPW>(v, d, o, acc);
         zacc = __dadd_rn(zacc, acc);
@@ -148,25 +171,25 @@ __device__ __forceinline__ double entries_any(const SetView<SPW> &v, const Opera
     return zacc;
 }
 
-template <int K, int G, int SPW>
+template <int K, int G, int SPW, bool MAX>
 __device__ __forceinline__ double entries_dispatch(const SetView<SPW> &v, const Operands &op, uint32_t amask, bool pairs,
                                                    const uint32_t *tab, uint32_t n_out, uint32_t cx, uint32_t lane, const Dest &d)
 {
     if (pairs && K <= 3) {
         // compile-time arena mask for the common operand counts
         switch (amask) {
-        case 0: return entries_pairs<K, 0u, G, SPW>(v, op, tab, n_out, lane, d);
-        case 1: return entries_pairs<K, 1u, G, SPW>(v, op, tab, n_out, lane, d);
-        case 2: if (K >= 2) return entries_pairs<K, (K >= 2 ? 2u : 0u), G, SPW>(v, op, tab, n_out, lane, d); break;
-        case 3: if (K >= 2) return entries_pairs<K, (K >= 2 ? 3u : 0u), G, SPW>(v, op, tab, n_out, lane, d); break;
-        case 4: if (K >= 3) return entries_pairs<K, (K >= 3 ? 4u : 0u), G, SPW>(v, op, tab, n_out, lane, d); break;
-        case 5: if (K >= 3) return entries_pairs<K, (K >= 3 ? 5u : 0u), G, SPW>(v, op, tab, n_out, lane, d); break;
-        case 6: if (K >= 3) return entries_pairs<K, (K >= 3 ? 6u : 0u), G, SPW>(v, op, tab, n_out, lane, d); break;
-        case 7: if (K >= 3) return entries_pairs<K, (K >= 3 ? 7u : 0u), G, SPW>(v, op, tab, n_out, lane, d); break;
+        case 0: return entries_pairs<K, 0u, G, SPW, MAX>(v, op, tab, n_out, lane, d);
+        case 1: return entries_pairs<K, 1u, G, SPW, MAX>(v, op, tab, n_out, lane, d);
+        case 2: if (K >= 2) return entries_pairs<K, (K >= 2 ? 2u : 0u), G, SPW, MAX>(v, op, tab, n_out, lane, d); break;
+        case 3: if (K >= 2) return entries_pairs<K, (K >= 2 ? 3u : 0u), G, SPW, MAX>(v, op, tab, n_out, lane, d); break;
+        case 4: if (K >= 3) return entries_pairs<K, (K >= 3 ? 4u : 0u), G, SPW, MAX>(v, op, tab, n_out, lane, d); break;
+        case 5: if (K >= 3) return entries_pairs<K, (K >= 3 ? 5u : 0u), G, SPW, MAX>(v, op, tab, n_out, lane, d); break;
+        case 6: if (K >= 3) return entries_pairs<K, (K >= 3 ? 6u : 0u), G, SPW, MAX>(v, op, tab, n_out, lane, d); break;
+        case 7: if (K >= 3) return entries_pairs<K, (K >= 3 ? 7u : 0u), G, SPW, MAX>(v, op, tab, n_out, lane, d); break;
         default: break;
         }
     }
-    return entries_any<K, G, SPW>(v, op, amask, tab, n_out, cx, lane, d);
+    return entries_any<K, G, SPW, MAX>(v, op, amask, tab, n_out, cx, lane, d);
 }
 
 // the steps of one program for one evidence set (b), on the G lanes that own it.
@@ -174,11 +197,11 @@ __device__ __forceinline__ double entries_dispatch(const SetView<SPW> &v, const 
 // words for every lane of the warp) is fetched with ONE coalesced load, lane i word i, while the PREVIOUS step runs, and
 // read field by field with warp shuffles; the evidence values of the set sit in registers the same way (lane l of the
 // set holds values 4l .. 4l+3).  Records longer than 32 words and plans with more than 32 observed variables read the
-// rest from memory.  `prog` must be readable 32 words past the last record.
-template <int G, int SPW>
+// rest from memory.  `prog` must be readable 32 words past the last record.  MAX: see ve_fused_max.
+template <int G, int SPW, bool MAX = false>
 __device__ __forceinline__ void run_steps(const uint32_t *__restrict__ prog, const uint32_t *__restrict__ offtab, uint32_t n_steps,
                                           const uint8_t *ev, uint32_t n_obs, double *result, double *zout, uint32_t nb, uint32_t b,
-                                          bool live, const SetView<SPW> &v, uint32_t lane, double *s_red)
+                                          bool live, const SetView<SPW> &v, uint32_t lane, double *s_red, uint8_t *arg = nullptr)
 {
     const uint32_t tw = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     constexpr uint32_t kEvLanes = G < 8 ? G : 8;                // lanes of a set inside one warp that hold evidence values
@@ -212,6 +235,10 @@ __device__ __forceinline__ void run_steps(const uint32_t *__restrict__ prog, con
         } else {
             d.result = nullptr;
             d.stride = 0;
+        }
+        if (MAX) {
+            d.arg = (flags & kFusedMax) ? arg + ((uint64_t)word(7) * nb + b) : nullptr;
+            d.arg_stride = nb;
         }
         // operand records (the k of a step is uniform over its lanes)
         uint32_t at = kFusedHeaderWords;
@@ -248,14 +275,14 @@ __device__ __forceinline__ void run_steps(const uint32_t *__restrict__ prog, con
         const bool pairs = (flags & kFusedPairs) != 0;
         double zacc;
         switch (k) {
-        case 1: zacc = entries_dispatch<1, G, SPW>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        case 2: zacc = entries_dispatch<2, G, SPW>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        case 3: zacc = entries_dispatch<3, G, SPW>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        case 4: zacc = entries_dispatch<4, G, SPW>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        case 5: zacc = entries_dispatch<5, G, SPW>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        default: zacc = entries_dispatch<6, G, SPW>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
+        case 1: zacc = entries_dispatch<1, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
+        case 2: zacc = entries_dispatch<2, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
+        case 3: zacc = entries_dispatch<3, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
+        case 4: zacc = entries_dispatch<4, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
+        case 5: zacc = entries_dispatch<5, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
+        default: zacc = entries_dispatch<6, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
         }
-        if ((flags & kFusedWantZ) && zout) {      // uniform over the lanes of the set; only single queries ask for it
+        if (!MAX && (flags & kFusedWantZ) && zout) {      // uniform over the lanes of the set; only single queries ask for it
             double z = zacc;
             if (G <= 32) {
                 // the lanes of a set are the threads l * SPW + s of the warp
@@ -276,12 +303,12 @@ __device__ __forceinline__ void run_steps(const uint32_t *__restrict__ prog, con
     }
 }
 
-template <int G>
-__global__ void __launch_bounds__(kFusedThreads) ve_fused(const __grid_constant__ FusedLaunch p)
+// the evidence sets of a launch, a group of G lanes each
+template <int G, bool MAX>
+__device__ __forceinline__ void run_sets(const FusedLaunch &p, double *s_red, uint8_t *arg)
 {
     constexpr int SPW = G >= 32 ? 1 : 32 / G;       // sets per warp, interleaved in the warp's slice of the arena
     constexpr int SPC = kFusedThreads / G;          // sets per CTA
-    __shared__ double s_red[kFusedThreads / 32];
     const uint32_t tw = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     uint32_t lane, set_in_cta;
     SetView<SPW> v;
@@ -304,8 +331,22 @@ __global__ void __launch_bounds__(kFusedThreads) ve_fused(const __grid_constant_
         const bool live = b < p.nb;      // lanes of a missing set repeat the last one (they take part in the syncs), stores off
         if (!live) b = p.nb - 1;
         const uint8_t *ev = p.ev ? p.ev + (uint64_t)b * p.n_obs : p.ev_inline;
-        run_steps<G, SPW>(p.prog, p.offtab, p.n_steps, ev, p.n_obs, p.result, p.z, p.nb, b, live, v, lane, s_red);
+        run_steps<G, SPW, MAX>(p.prog, p.offtab, p.n_steps, ev, p.n_obs, p.result, p.z, p.nb, b, live, v, lane, s_red, arg);
     }
+}
+
+template <int G>
+__global__ void __launch_bounds__(kFusedThreads) ve_fused(const __grid_constant__ FusedLaunch p)
+{
+    __shared__ double s_red[kFusedThreads / 32];
+    run_sets<G, false>(p, s_red, nullptr);
+}
+
+// an MPE program over a batch: the value of every set to p.f.result, the argmax rows to p.arg (fused.hpp)
+template <int G>
+__global__ void __launch_bounds__(kFusedThreads) ve_fused_max(const __grid_constant__ FusedMaxLaunch p)
+{
+    run_sets<G, true>(p.f, nullptr, p.arg);
 }
 
 // K10 -- TASKS: one launch runs many independent programs of one query, a CTA each.  A mixed plan (hundreds of tiny
@@ -333,6 +374,10 @@ size_t fused_smem_bytes(int G, uint32_t arena)
 }
 
 typedef void (*fused_fn)(const FusedLaunch);
+typedef void (*fused_max_fn)(const FusedMaxLaunch);
+
+// fn: the kernel for G (nullptr: no such variant), args: its parameter block
+static int launch_sets(bnpp_ctx *ctx, int G, const void *fn, void *args_block, const FusedLaunch &p, const char *const names[6]);
 
 int fused_launch(bnpp_ctx *ctx, int G, const FusedLaunch &p)
 {
@@ -344,8 +389,32 @@ int fused_launch(bnpp_ctx *ctx, int G, const FusedLaunch &p)
     case 16: fn = ve_fused<16>; break;
     case 32: fn = ve_fused<32>; break;
     case 128: fn = ve_fused<128>; break;
-    default: return fail(ctx, BNPP_EINVAL, "fused VE: lanes per set must be 8, 16, 32 or 128");
+    default: break;
     }
+    static const char *const names[6] = {"ve_fused<G=2>", "ve_fused<G=4>", "ve_fused<G=8>", "ve_fused<G=16>", "ve_fused<G=32>", "ve_fused<G=128>"};
+    return launch_sets(ctx, G, reinterpret_cast<const void *>(fn), const_cast<FusedLaunch *>(&p), p, names);
+}
+
+int fused_max_launch(bnpp_ctx *ctx, int G, const FusedMaxLaunch &p)
+{
+    fused_max_fn fn = nullptr;
+    switch (G) {
+    case 2: fn = ve_fused_max<2>; break;
+    case 4: fn = ve_fused_max<4>; break;
+    case 8: fn = ve_fused_max<8>; break;
+    case 16: fn = ve_fused_max<16>; break;
+    case 32: fn = ve_fused_max<32>; break;
+    case 128: fn = ve_fused_max<128>; break;
+    default: break;
+    }
+    static const char *const names[6] = {"ve_fused_max<G=2>", "ve_fused_max<G=4>", "ve_fused_max<G=8>", "ve_fused_max<G=16>",
+                                         "ve_fused_max<G=32>", "ve_fused_max<G=128>"};
+    return launch_sets(ctx, G, reinterpret_cast<const void *>(fn), const_cast<FusedMaxLaunch *>(&p), p.f, names);
+}
+
+static int launch_sets(bnpp_ctx *ctx, int G, const void *fn, void *args_block, const FusedLaunch &p, const char *const names[6])
+{
+    if (!fn) return fail(ctx, BNPP_EINVAL, "fused VE: lanes per set must be 8, 16, 32 or 128");
     if (p.arena & 1u) return fail(ctx, BNPP_EINVAL, "fused VE: the arena of a set must be an even number of doubles");
     const size_t smem = fused_smem_bytes(G, p.arena);
     {
@@ -368,12 +437,11 @@ int fused_launch(bnpp_ctx *ctx, int G, const FusedLaunch &p)
     const uint64_t resident = (uint64_t)ctx->sm_count * per_sm;
     if (blocks > resident) blocks = resident;
     if (blocks < 1) blocks = 1;
-    void *args[1] = {const_cast<FusedLaunch *>(&p)};
-    BNPP_CUDA(ctx, cudaLaunchKernel(reinterpret_cast<const void *>(fn), dim3((unsigned)blocks), dim3(kFusedThreads), args, smem,
-                                    ctx->stream));
+    void *args[1] = {args_block};
+    BNPP_CUDA(ctx, cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(kFusedThreads), args, smem, ctx->stream));
     ctx->launches++;
     ctx->last_desc = nullptr;
-    ctx->last_kernel = G == 2 ? "ve_fused<G=2>" : G == 4 ? "ve_fused<G=4>" : G == 8 ? "ve_fused<G=8>" : (G == 16 ? "ve_fused<G=16>" : (G == 32 ? "ve_fused<G=32>" : "ve_fused<G=128>"));
+    ctx->last_kernel = names[G == 2 ? 0 : G == 4 ? 1 : G == 8 ? 2 : G == 16 ? 3 : G == 32 ? 4 : 5];
     ctx->last_grid = (uint32_t)blocks;
     ctx->last_block = kFusedThreads;
     return BNPP_OK;

@@ -131,6 +131,38 @@ __global__ void mpe_decode(const __grid_constant__ MpeDecodeParams p)
     }
     if (p.set_one) *p.value = 1.0;
 }
+
+// MPE decode of a batch (bnpp_mpe_plan_run_batched): one thread per set of a slice walks the records of mpe_decode with
+// the FIRST ARGMAX ROW of the step in words 1-2: the argmax of output entry o of a step for set t of the slice is
+// arg[(row + o) * cur + t].  The records are the same for every set, so the threads of a warp always touch one
+// variable's row of assign[v][nb] (coalesced); only the argmax byte a set's own assignment selects is scattered.
+struct MpeBatchDecodeParams {
+    const uint32_t *rec;
+    const uint8_t *arg;             // [rows][cur]
+    const uint8_t *ev;              // evidence value j of set t: ev[j * ev_col + t * ev_row] (already range-checked)
+    uint64_t ev_col, ev_row;
+    uint8_t *assign;                // [nvars][nb]: the column of the slice's first set
+    uint32_t nb, cur, nvars, n_obs, n_rec;
+};
+
+__global__ void mpe_decode_batched(const __grid_constant__ MpeBatchDecodeParams p)
+{
+    for (uint32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < p.cur; t += gridDim.x * blockDim.x) {
+        uint8_t *a = p.assign + t;
+        for (uint32_t v = 0; v < p.nvars; ++v) a[(uint64_t)v * p.nb] = 0;
+        const uint32_t *r = p.rec;
+        for (uint32_t i = 0; i < p.n_obs; ++i) a[(uint64_t)__ldg(r + i) * p.nb] = p.ev[i * p.ev_col + t * p.ev_row];
+        r += p.n_obs;
+        for (uint32_t s = 0; s < p.n_rec; ++s) {
+            const uint64_t row = (uint64_t)__ldg(r + 1) | ((uint64_t)__ldg(r + 2) << 32);
+            const uint32_t rank = __ldg(r + 3);
+            uint64_t idx = 0;
+            for (uint32_t j = 0; j < rank; ++j) idx += (uint64_t)a[(uint64_t)__ldg(r + 4 + 2 * j) * p.nb] * __ldg(r + 5 + 2 * j);
+            a[(uint64_t)__ldg(r) * p.nb] = p.arg[(row + idx) * p.cur + t];
+            r += 4 + 2 * rank;
+        }
+    }
+}
 }  // namespace bnpp
 
 struct bnpp_ve_plan {
@@ -208,7 +240,8 @@ struct bnpp_ve_plan {
     std::vector<uint32_t> mar_off, mar_size;
     uint32_t *mar_off_dev = nullptr, *mar_size_dev = nullptr;
     // MPE plan (max-product): every eliminating step also writes its argmax table into a byte arena that is never
-    // reused within a run (the decode reads all of them); K9 / K10 stay off (their interpreters only sum)
+    // reused within a run (the decode reads all of them); single runs are launch-per-bucket (K10 only sums), batched
+    // runs take K9 in max mode (ve_fused_max) or K8's max variants
     bool is_mpe = false;
     uint32_t mpe_nvars = 0;
     std::vector<uint64_t> arg_off;          // per step: byte offset of its argmax table (eliminating steps only)
@@ -219,6 +252,14 @@ struct bnpp_ve_plan {
     uint32_t n_decode_rec = 0;
     bnpp::MpeDecodeParams decode;           // parameters of the decode's node in the replay graph
     cudaGraphNode_t decode_node = nullptr;
+    // batched MPE: eliminating step s (plan order) owns argmax rows [arg_row[s], arg_row[s] + its output entries) of a
+    // byte scratch of arg_rows rows x slice sets, entry o of set b at (arg_row[s] + o) * slice + b
+    std::vector<uint64_t> arg_row;
+    uint64_t arg_rows = 0;
+    std::vector<uint32_t> batch_rec;        // decode records of mpe_decode_batched (rows for byte offsets); uploaded once
+    uint32_t *batch_rec_dev = nullptr;
+    uint8_t *batch_arg = nullptr;
+    uint64_t batch_arg_bytes = 0;
     bool profiling = false;
     std::vector<cudaEvent_t> ev;
     std::vector<float> step_ms;
@@ -867,8 +908,13 @@ void fused_encode(bnpp_ve_plan *pl, const std::vector<int> &order, bool segment,
             for (uint64_t o = 0; o < n_out && pairs; ++o) pairs = (fp.offtab[tab_off + (size_t)q * n_out + o] & 1u) == 0;
         }
         uint32_t flags = pairs ? kFusedPairs : 0u, out_off;
+        const bool argmax = pl->is_mpe && st.elim >= 0;
+        if (argmax) {
+            if (pl->arg_row[order[i]] >= (1ull << 32)) return;
+            flags |= kFusedMax;
+        }
         if (st.out == -2) {
-            flags |= kFusedToResult | (st.want_z ? kFusedWantZ : 0u);
+            flags |= kFusedToResult | (st.want_z && !pl->is_mpe ? kFusedWantZ : 0u);
             if (st.roff >= (1ull << 32)) return;
             out_off = (uint32_t)st.roff;
         } else if (in_smem[st.out]) {
@@ -877,7 +923,8 @@ void fused_encode(bnpp_ve_plan *pl, const std::vector<int> &order, bool segment,
             flags |= kFusedToGlobal;      // a later launch reads it: absolute address in header words 5-6
             out_off = 0;
         }
-        const uint32_t head[kFusedHeaderWords] = {(uint32_t)n_out, cx, (uint32_t)k | (flags << 8), out_off, tab_off, 0, 0, 0};
+        const uint32_t head[kFusedHeaderWords] = {(uint32_t)n_out, cx, (uint32_t)k | (flags << 8), out_off, tab_off, 0, 0,
+                                                  argmax ? (uint32_t)pl->arg_row[order[i]] : 0u};
         if (flags & kFusedToGlobal) {
             const uint32_t at = (uint32_t)fp.prog.size();
             fp.ptr_slots.push_back({at + 5, at + 6, 1, st.out});
@@ -1249,16 +1296,17 @@ int upload_tasks(bnpp_ve_plan *pl, const double *const *tables_dev)
 }
 
 int run_fused(bnpp_ve_plan *pl, FusedProgram &fp, int G, const double *const *tables_dev, uint32_t nb, const uint8_t *ev_dev,
-              const uint32_t *obs_val, double *result_dev, double *z_dev);
+              const uint32_t *obs_val, double *result_dev, double *z_dev, uint8_t *arg_dev = nullptr);
 
+// arg_dev != nullptr: an MPE program over a batch (ve_fused_max), argmax rows [rows][nb] there
 int run_fused(bnpp_ve_plan *pl, int G, const double *const *tables_dev, uint32_t nb, const uint8_t *ev_dev,
-              const uint32_t *obs_val, double *result_dev, double *z_dev)
+              const uint32_t *obs_val, double *result_dev, double *z_dev, uint8_t *arg_dev = nullptr)
 {
-    return run_fused(pl, pl->fused, G, tables_dev, nb, ev_dev, obs_val, result_dev, z_dev);
+    return run_fused(pl, pl->fused, G, tables_dev, nb, ev_dev, obs_val, result_dev, z_dev, arg_dev);
 }
 
 int run_fused(bnpp_ve_plan *pl, FusedProgram &fp, int G, const double *const *tables_dev, uint32_t nb, const uint8_t *ev_dev,
-              const uint32_t *obs_val, double *result_dev, double *z_dev)
+              const uint32_t *obs_val, double *result_dev, double *z_dev, uint8_t *arg_dev)
 {
     bnpp_ctx *ctx = pl->ctx;
     auto address = [&](const FusedProgram::Slot &slot) {
@@ -1305,6 +1353,12 @@ int run_fused(bnpp_ve_plan *pl, FusedProgram &fp, int G, const double *const *ta
     p.arena = fp.arena;
     if (!ev_dev && obs_val)
         for (int i = 0; i < pl->n_obs && i < kFusedInlineEv; ++i) p.ev_inline[i] = (uint8_t)obs_val[i];
+    if (arg_dev) {
+        FusedMaxLaunch q;
+        q.f = p;
+        q.arg = arg_dev;
+        return fused_max_launch(ctx, G, q);
+    }
     return fused_launch(ctx, G, p);
 }
 
@@ -1436,19 +1490,21 @@ int bnpp_mpe_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfa
     return create_plan(ctx, nfac, scopes, n_obs, obs_var, n_order, order, nvars, card, out);
 }
 
-// Argmax arena and decode records of an MPE plan; the K9 / K10 paths off
+// Argmax arena, argmax rows of batched runs and decode records of an MPE plan; the K10 path off
 static int mpe_finish(bnpp_ve_plan *pl, int nvars, int n_obs, const uint32_t *obs_var)
 {
     pl->is_mpe = true;
     pl->mpe_nvars = (uint32_t)nvars;
-    pl->fused_mode = 0;
     pl->segments_mode = 0;
     pl->arg_off.assign(pl->steps.size(), 0);
+    pl->arg_row.assign(pl->steps.size(), 0);
     for (size_t s = 0; s < pl->steps.size(); ++s) {
         const PlanStep &st = pl->steps[s];
         if (st.elim < 0) continue;
         pl->arg_off[s] = (pl->arg_bytes + 255) & ~(uint64_t)255;
         pl->arg_bytes = pl->arg_off[s] + pl->f[st.out].size;
+        pl->arg_row[s] = pl->arg_rows;
+        pl->arg_rows += pl->f[st.out].size;
     }
     pl->peak_bytes += pl->arg_bytes;
     std::vector<uint32_t> &r = pl->decode_rec;
@@ -1475,6 +1531,15 @@ static int mpe_finish(bnpp_ve_plan *pl, int nvars, int n_obs, const uint32_t *ob
             r.push_back(st_of[a]);
         }
         pl->n_decode_rec++;
+    }
+    // the same records with the step's first argmax row in place of its byte offset
+    pl->batch_rec = r;
+    uint32_t *w = pl->batch_rec.data() + n_obs;
+    for (size_t s = pl->steps.size(); s-- > 0;) {
+        if (pl->steps[s].elim < 0) continue;
+        w[1] = (uint32_t)pl->arg_row[s];
+        w[2] = (uint32_t)(pl->arg_row[s] >> 32);
+        w += 4 + 2 * w[3];
     }
     return BNPP_OK;
 }
@@ -1641,6 +1706,8 @@ int bnpp_ve_plan_destroy(bnpp_ve_plan *pl)
     if (pl->arg_arena) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->arg_arena));
     if (pl->decode_rec_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->decode_rec_dev));
     if (pl->obs_val_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->obs_val_dev));
+    if (pl->batch_rec_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->batch_rec_dev));
+    if (pl->batch_arg) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->batch_arg));
     for (auto &d : pl->exec)
         if (d) {
             contract_release(pl->ctx, *d);
@@ -1714,7 +1781,6 @@ int bnpp_ve_plan_set_profiling(bnpp_ve_plan *pl, int on)
 int bnpp_ve_plan_set_fused(bnpp_ve_plan *pl, int on)
 {
     if (!pl) return BNPP_EINVAL;
-    if (pl->is_mpe && on) return fail(pl->ctx, BNPP_EINVAL, "MPE plans run one launch per bucket (ve_fused only sums)");
     pl->fused_mode = on != 0;
     return BNPP_OK;
 }
@@ -2238,17 +2304,101 @@ static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uin
 // ids are the plan's, ev_dev[b][j] is the value of obs_var[j] in set b.  result_dev receives
 // [result_size][nb] (batch fastest).  Sets are processed in slices that keep the widest
 // intermediate below ~1 GiB.
+// assign_dev != nullptr: an MPE run (result_dev receives the values, assign_dev [nvars][nb] the assignments)
 static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, uint32_t nb, uint32_t n_obs,
-                            const uint8_t *ev_dev, double *result_dev);
+                            const uint8_t *ev_dev, double *result_dev, uint8_t *assign_dev);
+static int run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32_t nb, uint32_t n_obs, const uint8_t *ev_dev,
+                       double *result_dev, uint8_t *assign_dev);
 
-// The launches of a batched run are tiny when the batch is sharded over many GPUs, so from the
-// third run with the same buffers on, the whole run (stream-ordered allocations included) is
-// replayed as one captured CUDA graph.
 int bnpp_ve_plan_run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32_t nb, uint32_t n_obs,
                              const uint8_t *ev_dev, double *result_dev)
 {
     if (!pl || !pl->ctx || !result_dev || nb == 0) return BNPP_EINVAL;
-    if (pl->is_mpe) return fail(pl->ctx, BNPP_EINVAL, "MPE plan: batched runs are not supported");
+    if (pl->is_mpe) return fail(pl->ctx, BNPP_EINVAL, "MPE plan: run a batch with bnpp_mpe_plan_run_batched");
+    return run_batched(pl, tables_dev, nb, n_obs, ev_dev, result_dev, nullptr);
+}
+
+int bnpp_mpe_plan_run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32_t nb, uint32_t n_obs,
+                              const uint8_t *ev_dev, double *value_dev, uint8_t *assignment_dev)
+{
+    if (!pl || !pl->ctx || !value_dev || !assignment_dev || nb == 0) return BNPP_EINVAL;
+    if (!pl->is_mpe) return fail(pl->ctx, BNPP_EINVAL, "bnpp_mpe_plan_run_batched: not an MPE plan");
+    return run_batched(pl, tables_dev, nb, n_obs, ev_dev, value_dev, assignment_dev);
+}
+
+// Sets per slice of a batched run: K8 keeps its widest intermediate within ~1 GiB (k8 = true), and an MPE run its
+// argmax rows (arg_rows bytes per set) within 1 GiB on either engine.
+static uint32_t batch_slice(const bnpp_ve_plan *pl, uint32_t nb, bool k8)
+{
+    uint64_t slice = nb;
+    if (k8) {
+        uint64_t widest = 1;
+        for (const PlanFactor &pf : pl->f)
+            if (pf.src < 0) widest = std::max(widest, pf.size);
+        widest = std::max(widest, pl->result_size);
+        slice = std::min<uint64_t>(nb, std::max<uint64_t>(1, (1ull << 27) / widest));
+        if (pl->result_size > 1) slice = nb;     // a multi-entry result is laid out [entries][nb]: no slicing
+    }
+    if (pl->is_mpe && pl->arg_rows) slice = std::min<uint64_t>(slice, std::max<uint64_t>(1, (1ull << 30) / pl->arg_rows));
+    return (uint32_t)slice;
+}
+
+// the argmax rows of an MPE batch of `slice` sets, and the decode records on the device (before any capture)
+static int mpe_batch_prepare(bnpp_ve_plan *pl, uint32_t slice)
+{
+    bnpp_ctx *ctx = pl->ctx;
+    if (!pl->batch_rec_dev && !pl->batch_rec.empty()) {
+        double *store = nullptr;
+        const int rc = bnpp_alloc(ctx, (pl->batch_rec.size() + 1) / 2, &store);
+        if (rc != BNPP_OK) return rc;
+        pl->batch_rec_dev = reinterpret_cast<uint32_t *>(store);
+        BNPP_CUDA(ctx, cudaMemcpyAsync(pl->batch_rec_dev, pl->batch_rec.data(), 4 * pl->batch_rec.size(), cudaMemcpyHostToDevice,
+                                       ctx->stream));
+    }
+    const uint64_t need = pl->arg_rows * slice;
+    if (need > pl->batch_arg_bytes) {
+        if (pl->batch_arg) bnpp_free(ctx, reinterpret_cast<double *>(pl->batch_arg));
+        pl->batch_arg = nullptr;
+        pl->batch_arg_bytes = 0;
+        double *store = nullptr;
+        const int rc = bnpp_alloc(ctx, (need + 7) / 8, &store);
+        if (rc != BNPP_OK) return rc;
+        pl->batch_arg = reinterpret_cast<uint8_t *>(store);
+        pl->batch_arg_bytes = need;
+    }
+    return BNPP_OK;
+}
+
+// the decode of the sets [b0, b0 + cur) of an MPE batch; ev: evidence value j of set b0 + t at ev[j * ev_col + t * ev_row]
+static int mpe_decode_batch_launch(bnpp_ve_plan *pl, uint32_t nb, uint32_t b0, uint32_t cur, const uint8_t *ev, uint64_t ev_col,
+                                   uint64_t ev_row, uint8_t *assign_dev)
+{
+    bnpp_ctx *ctx = pl->ctx;
+    MpeBatchDecodeParams p;
+    memset(&p, 0, sizeof p);
+    p.rec = pl->batch_rec_dev;
+    p.arg = pl->batch_arg;
+    p.ev = ev;
+    p.ev_col = ev_col;
+    p.ev_row = ev_row;
+    p.assign = assign_dev + b0;
+    p.nb = nb;
+    p.cur = cur;
+    p.nvars = pl->mpe_nvars;
+    p.n_obs = (uint32_t)pl->n_obs;
+    p.n_rec = pl->n_decode_rec;
+    mpe_decode_batched<<<(cur + 127) / 128, 128, 0, ctx->stream>>>(p);
+    BNPP_CUDA(ctx, cudaGetLastError());
+    ctx->launches++;
+    return BNPP_OK;
+}
+
+// The launches of a batched run are tiny when the batch is sharded over many GPUs, so from the
+// third run with the same buffers on, the whole run (stream-ordered allocations included) is
+// replayed as one captured CUDA graph.
+static int run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32_t nb, uint32_t n_obs, const uint8_t *ev_dev,
+                       double *result_dev, uint8_t *assign_dev)
+{
     bnpp_ctx *ctx = pl->ctx;
     if ((int)n_obs != pl->n_obs) return fail(ctx, BNPP_EINVAL, "batched VE: n_obs differs from the plan's");
     if (n_obs && !ev_dev) return fail(ctx, BNPP_EINVAL, "batched VE: evidence matrix missing");
@@ -2282,14 +2432,32 @@ int bnpp_ve_plan_run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, 
                 if (rc != BNPP_OK) return rc;
                 ev = pl->ev_clean;
             }
-            return run_fused(pl, G, tables_dev, nb, ev, nullptr, result_dev, nullptr);
+            if (!assign_dev) return run_fused(pl, G, tables_dev, nb, ev, nullptr, result_dev, nullptr);
+            // MPE: slices whose argmax rows fit the scratch, each one ve_fused_max launch and its decode
+            const uint32_t slice = batch_slice(pl, nb, false);
+            int rc = mpe_batch_prepare(pl, slice);
+            for (uint32_t b0 = 0; b0 < nb && rc == BNPP_OK; b0 += slice) {
+                const uint32_t cur = std::min(slice, nb - b0);
+                const uint8_t *ev_b = n_obs ? ev + (uint64_t)b0 * n_obs : ev;
+                rc = run_fused(pl, G, tables_dev, cur, ev_b, nullptr, result_dev + b0, nullptr, pl->batch_arg);
+                if (rc == BNPP_OK) rc = mpe_decode_batch_launch(pl, nb, b0, cur, ev_b, 1, n_obs, assign_dev);
+            }
+            return rc;
         }
+    }
+    if (assign_dev) {
+        const int rc = mpe_batch_prepare(pl, batch_slice(pl, nb, true));
+        if (rc != BNPP_OK) return rc;
     }
     std::vector<const void *> key;
     key.push_back(ev_dev);
     key.push_back(result_dev);
     key.push_back(reinterpret_cast<const void *>(static_cast<uintptr_t>(nb)));
     for (int q = 0; q < pl->n_inputs; ++q) key.push_back(tables_dev[q]);
+    if (assign_dev) {
+        key.push_back(assign_dev);
+        key.push_back(pl->batch_arg);       // a captured run writes the argmax rows there
+    }
     if (pl->batch_exec && key == pl->batch_key) {
         BNPP_CUDA(ctx, cudaGraphLaunch(pl->batch_exec, ctx->stream));
         ctx->launches += pl->steps.size() + 1;
@@ -2306,7 +2474,7 @@ int bnpp_ve_plan_run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, 
         cudaGraph_t g = nullptr;
         if (cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
             const uint64_t before = ctx->launches;
-            const int rc = run_batched_once(pl, tables_dev, nb, n_obs, ev_dev, result_dev);
+            const int rc = run_batched_once(pl, tables_dev, nb, n_obs, ev_dev, result_dev, assign_dev);
             const cudaError_t e = cudaStreamEndCapture(ctx->stream, &g);
             ctx->launches = before;
             if (rc == BNPP_OK && e == cudaSuccess && cudaGraphInstantiate(&pl->batch_exec, g, 0) == cudaSuccess) {
@@ -2323,19 +2491,18 @@ int bnpp_ve_plan_run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, 
     }
     pl->batch_key = key;
     pl->batch_runs++;
-    return run_batched_once(pl, tables_dev, nb, n_obs, ev_dev, result_dev);
+    return run_batched_once(pl, tables_dev, nb, n_obs, ev_dev, result_dev, assign_dev);
 }
 
 static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, uint32_t nb, uint32_t n_obs,
-                            const uint8_t *ev_dev, double *result_dev)
+                            const uint8_t *ev_dev, double *result_dev, uint8_t *assign_dev)
 {
     bnpp_ctx *ctx = pl->ctx;
     uint64_t widest = 1;
     for (const PlanFactor &pf : pl->f)
         if (pf.src < 0) widest = std::max(widest, pf.size);
     widest = std::max(widest, pl->result_size);
-    uint32_t slice = (uint32_t)std::min<uint64_t>(nb, std::max<uint64_t>(1, (1ull << 27) / widest));
-    if (pl->result_size > 1) slice = nb;     // a multi-entry result is laid out [entries][nb]: no slicing
+    const uint32_t slice = batch_slice(pl, nb, true);
     if ((uint64_t)widest * slice >= (1ull << 32)) return fail(ctx, BNPP_ETOOBIG, "batched VE: intermediate too large");
     static const std::vector<int64_t> dense;
     static const std::vector<std::pair<int64_t, int>> no_obs;
@@ -2394,8 +2561,9 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
                 if (rc != BNPP_OK) break;
                 dst = owned[st.out];
             }
+            uint8_t *arg = assign_dev && st.elim >= 0 ? pl->batch_arg + pl->arg_row[s] * cur : nullptr;   // MPE: the step's rows
             rc = contract_batched_step(ctx, (int)st.operands.size(), ops, *ov, *oc, st.elim, cur, evt + b0, nb, n_cols, dst,
-                                       &pl->offtab_host[s], &pl->offtab_dev[s]);
+                                       &pl->offtab_host[s], &pl->offtab_dev[s], arg);
             for (int id : st.operands)
                 if (owned[id] && pl->f[id].last_use == (int)s) {
                     bnpp_free(ctx, owned[id]);
@@ -2405,6 +2573,7 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
         for (double *p : owned)
             if (p) bnpp_free(ctx, p);
         if (pl->steps.empty() || pl->steps.back().out != -2) rc = fill(ctx, result_dev + b0, cur, 1.0);
+        if (rc == BNPP_OK && assign_dev) rc = mpe_decode_batch_launch(pl, nb, b0, cur, evt + b0, nb, 1, assign_dev);
     }
     bnpp_free(ctx, evt_store);
     return rc;

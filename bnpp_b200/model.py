@@ -48,6 +48,8 @@ def _declare(L):
     L.bnpp_mpe_plan_create.argtypes = [ctypes.c_void_p, ctypes.c_int, capi.c_u32p, ctypes.c_int, P(capi.Scope), ctypes.c_int,
                                        capi.c_u32p, ctypes.c_int, capi.c_u32p, P(ctypes.c_void_p)]
     L.bnpp_mpe_plan_run.argtypes = [ctypes.c_void_p, P(ctypes.c_void_p), capi.c_u32p, ctypes.c_void_p, ctypes.c_void_p]
+    L.bnpp_mpe_plan_run_batched.argtypes = [ctypes.c_void_p, P(ctypes.c_void_p), ctypes.c_uint32, ctypes.c_uint32,
+                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
     L._ve_declared = True
 
 
@@ -240,6 +242,18 @@ class MPEPlan(VEPlan):
         ov = capi._u32(obs_val)
         self.ctx.check(self.ctx.L.bnpp_mpe_plan_run(self.h, tp, ctypes.cast(ov, capi.c_u32p), ctypes.c_void_p(value_ptr),
                                                     ctypes.c_void_p(assignment_ptr)))
+
+    def run_mpe_batched(self, table_ptrs, nb, ev_ptr, value_ptr, assignment_ptr):
+        """ev_ptr: device uint8 [nb][len(observed)]; value_ptr: device double [nb]; assignment_ptr: device uint8
+        [nvars][nb].  Asynchronous."""
+        tp = (ctypes.c_void_p * max(1, len(table_ptrs)))(*table_ptrs)
+        self.ctx.check(self.ctx.L.bnpp_mpe_plan_run_batched(self.h, tp, int(nb), len(self.observed), ctypes.c_void_p(ev_ptr),
+                                                            ctypes.c_void_p(value_ptr), ctypes.c_void_p(assignment_ptr)))
+
+    def set_fused(self, on=True):
+        """the engine of batched runs: the whole plan in one launch per slice when every step is small (default), or one
+        launch per bucket; single runs are always one launch per bucket"""
+        super().set_fused(on)
 
 
 class BN:
@@ -447,6 +461,34 @@ class BN:
             if out is None:
                 out = self._batch_out[nb] = torch.empty(nb, dtype=torch.float64, device=self._dev.device)
         p.run_batched(self.table_ptrs, nb, values.data_ptr(), out.data_ptr())
+        self._keep_alive = values
+        return out
+
+    def mpe_batch(self, observed, values, heuristic="mf", host_values=None):
+        """MPE for a batch of evidence sets sharing the observed ids, the batched counterpart of `mpe`.
+        observed: sorted variable ids; values: torch.uint8 CUDA tensor [nb][len(observed)] (or pass host_values, a pinned
+        uint8 tensor, to include the H2D copy).  -> (value [nb] float64, assignment [nvars][nb] uint8), device tensors;
+        every set's value and assignment equal `mpe` for its evidence (an out-of-range value is read as 0 and raises
+        BNPP_STATUS_BAD_EVIDENCE, see ctx.status()).
+        The returned tensors are the model's result buffers for batches of nb sets, written on the context's stream:
+        synchronise (`ctx.sync()`) before reading them on another stream, and clone them if they must survive the next
+        call with the same nb (stable pointers are what lets the library replay the run as a graph)."""
+        observed = list(observed)
+        bkey = ("mpe", tuple(observed), heuristic)
+        p = self._batch_plans.get(bkey)
+        if p is None:
+            variables = [v for v in range(self.nvars) if v not in set(observed)]
+            order, _ = self.order(variables, observed, heuristic)
+            p = self._batch_plans[bkey] = self._cached_plan(("mpe", tuple(observed), tuple(order)), MPEPlan, observed, order)
+        with torch.cuda.stream(self.ctx.torch_stream):
+            if host_values is not None:
+                values = host_values.to(self._dev.device, non_blocking=True)
+            nb = values.shape[0]
+            out = self._batch_out.get(("mpe", nb))
+            if out is None:
+                out = self._batch_out[("mpe", nb)] = (torch.empty(nb, dtype=torch.float64, device=self._dev.device),
+                                                       torch.empty((self.nvars, nb), dtype=torch.uint8, device=self._dev.device))
+        p.run_mpe_batched(self.table_ptrs, nb, values.data_ptr(), out[0].data_ptr(), out[1].data_ptr())
         self._keep_alive = values
         return out
 

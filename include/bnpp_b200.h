@@ -210,8 +210,8 @@ int bnpp_ve_plan_run(bnpp_ve_plan *plan, const double *const *tables_dev, const 
  * (one byte per output entry, counted in peak_bytes) and a one-thread decode walks them backwards.
  * `order` must cover every unobserved variable that some scope mentions, and an eliminated
  * variable may have at most 255 values; else BNPP_EINVAL.  ctx may be NULL (a dry plan).
- * Runs are launch-per-bucket (never the K9 / K10 paths); from the second run on a run is one
- * replay of a CUDA graph that includes the decode.
+ * Single runs are launch-per-bucket (never the K9 / K10 paths); from the second run on a run is one
+ * replay of a CUDA graph that includes the decode.  Batches: bnpp_mpe_plan_run_batched.
  * run: assignment_dev[nvars] receives one uint32 per variable id: the evidence value for an
  * observed variable, 0 for a variable no factor mentions; value_dev one double.  Zero-probability
  * evidence gives value 0 and the lowest values.  An evidence value out of range returns
@@ -220,6 +220,23 @@ int bnpp_mpe_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfa
                          int n_obs, const uint32_t *obs_var, int n_order, const uint32_t *order, bnpp_ve_plan **out);
 int bnpp_mpe_plan_run(bnpp_ve_plan *plan, const double *const *tables_dev, const uint32_t *obs_val,
                       double *value_dev, uint32_t *assignment_dev);
+/* MPE for a BATCH of evidence sets over one MPE plan: ev_dev [nb][n_obs] uint8 as for
+ * bnpp_ve_plan_run_batched; value_dev receives [nb] doubles, assignment_dev [nvars][nb] uint8 (batch
+ * fastest).  Every set's value and assignment equal, bit for bit, what bnpp_mpe_plan_run returns for its
+ * evidence: the observed variables report the values the set was computed with, a variable no factor
+ * mentions reports 0.  A value >= its variable's cardinality is read as 0 (and reported as 0) and raises
+ * BNPP_STATUS_BAD_EVIDENCE.  Engines as for batched PR: the whole plan in one launch per slice (K9,
+ * ve_fused_max) when fused_info accepts the plan for nb > 1 sets, else one launch per bucket (K8's
+ * max-product variants, replayed as a captured graph from the third run with the same buffers on);
+ * bnpp_ve_plan_set_fused(plan, 0) forces K8.  A decode launch per slice, one thread per set, follows.
+ * Argmax layout, shared by both engines: eliminating step s (plan order, bnpp_ve_plan_describe) owns the
+ * rows [R_s, R_s + n_out_s) of a plan-owned byte scratch, R_s = the sum of n_out over the eliminating steps
+ * before it; the argmax of its output entry o for set b of a slice of `slice` sets is at byte
+ * (R_s + o) * slice + b.  Batches are cut into slices so that the scratch stays within 1 GiB (K8: also its
+ * widest intermediate).  A non-MPE plan, an n_obs other than the plan's, a NULL buffer or nb == 0 returns
+ * BNPP_EINVAL. */
+int bnpp_mpe_plan_run_batched(bnpp_ve_plan *plan, const double *const *tables_dev, uint32_t nb, uint32_t n_obs,
+                              const uint8_t *ev_dev, double *value_dev, uint8_t *assignment_dev);
 /* entries of the result table a run writes (PR: 1; marginals plan: the layout's total) */
 int bnpp_ve_plan_result_size(const bnpp_ve_plan *plan, uint64_t *n);
 /* BN::marginals (code/model.cpp:320-339) for EVERY variable in one plan: two passes over the
@@ -250,7 +267,9 @@ int bnpp_ve_plan_run_batched(bnpp_ve_plan *plan, const double *const *tables_dev
  * lanes owns an evidence set and walks the bucket loop of code/model.cpp:409-439 with the
  * intermediates of the set in shared memory; results are bit-identical to the launch-per-bucket
  * path.  On by default (environment BNPP_FUSED=0 turns it off for new plans); set_fused(plan, 0)
- * forces one launch per bucket.  fused_info: lanes per evidence set a run over nb sets would use
+ * forces one launch per bucket.  On an MPE plan it selects the engine of bnpp_mpe_plan_run_batched
+ * only (single MPE runs are always launch-per-bucket), and fused_info / fused_program describe the
+ * max-mode program (fused.hpp: kFusedMax steps carry their first argmax row R_s in header word 7).  fused_info: lanes per evidence set a run over nb sets would use
  * (0 = not fused), shared-memory doubles per set, steps in the launch. */
 int bnpp_ve_plan_set_fused(bnpp_ve_plan *plan, int on);
 int bnpp_ve_plan_fused_info(bnpp_ve_plan *plan, uint32_t nb, int32_t *lanes_per_set, uint32_t *arena_doubles,
