@@ -143,6 +143,14 @@ public:
     std::vector<unsigned> ordering(const std::vector<unsigned> &vars, Heuristic h, unsigned &width) const
     {
         InteractionGraph g(*this);
+        return g.ordering_in_place(vars, h, width);
+    }
+
+    // the same on this graph itself: the eliminated nodes are gone and the fill edges stay, so a second call orders
+    // the rest of the variables after the first ones (constrained orders: summed variables, then MAP variables)
+    std::vector<unsigned> ordering_in_place(const std::vector<unsigned> &vars, Heuristic h, unsigned &width)
+    {
+        InteractionGraph &g = *this;
         NodeSet cand;
         for (unsigned v : vars) cand.insert(v);
         std::vector<unsigned> order;
@@ -265,7 +273,8 @@ public:
     // The one case where the scan is NOT that minimum -- plain min-fill seeds its best
     // score with |nodes|+1 (code/graph.cpp:122-153), so when no candidate scores below
     // the seed the first candidate survives unless a later one ties the seed with a smaller
-    // degree -- falls back to the literal scan for that round.
+    // degree -- falls back to the literal scan for that round.  The graph is eliminated in place: a second call orders
+    // the rest of the variables with the fill edges of the first in place.
     std::vector<unsigned> ordering(const std::vector<unsigned> &vars, Heuristic h, unsigned &width)
     {
         std::unordered_set<unsigned> cand;

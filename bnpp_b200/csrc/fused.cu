@@ -22,6 +22,8 @@
 // rule of contract.cu's max-product kernels (start at x = 0, a later x replaces it only if its product is strictly
 // greater: ties keep the lowest x, a NaN never replaces a number), and the argmax byte of every output entry of a
 // kFusedMax step in global memory -- ~14 KB of argmax per set of config 5 would not fit in shared memory.
+// MIXED (ve_fused_mixed, the batch engine of MAP plans that also sum): a kFusedMax step takes the MAX path above, every
+// other step the sum path of ve_fused (same products, same order of additions; no partition).
 #include <cstdlib>
 #include <map>
 #include <mutex>
@@ -192,13 +194,29 @@ __device__ __forceinline__ double entries_dispatch(const SetView<SPW> &v, const 
     return entries_any<K, G, SPW, MAX>(v, op, amask, tab, n_out, cx, lane, d);
 }
 
+// the entries of one step, k operands
+template <int G, int SPW, bool MAX>
+__device__ __forceinline__ double step_entries(uint32_t k, const SetView<SPW> &v, const Operands &op, uint32_t amask, bool pairs,
+                                               const uint32_t *tab, uint32_t n_out, uint32_t cx, uint32_t lane, const Dest &d)
+{
+    switch (k) {
+    case 1: return entries_dispatch<1, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d);
+    case 2: return entries_dispatch<2, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d);
+    case 3: return entries_dispatch<3, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d);
+    case 4: return entries_dispatch<4, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d);
+    case 5: return entries_dispatch<5, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d);
+    default: return entries_dispatch<6, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d);
+    }
+}
+
 // the steps of one program for one evidence set (b), on the G lanes that own it.
 // Decoding a step costs no memory round trip: the record of a step (header, operand records, observed axes -- the same
 // words for every lane of the warp) is fetched with ONE coalesced load, lane i word i, while the PREVIOUS step runs, and
 // read field by field with warp shuffles; the evidence values of the set sit in registers the same way (lane l of the
 // set holds values 4l .. 4l+3).  Records longer than 32 words and plans with more than 32 observed variables read the
-// rest from memory.  `prog` must be readable 32 words past the last record.  MAX: see ve_fused_max.
-template <int G, int SPW, bool MAX = false>
+// rest from memory.  `prog` must be readable 32 words past the last record.  MAX: see ve_fused_max; MAX and MIXED: see
+// ve_fused_mixed.
+template <int G, int SPW, bool MAX = false, bool MIXED = false>
 __device__ __forceinline__ void run_steps(const uint32_t *__restrict__ prog, const uint32_t *__restrict__ offtab, uint32_t n_steps,
                                           const uint8_t *ev, uint32_t n_obs, double *result, double *zout, uint32_t nb, uint32_t b,
                                           bool live, const SetView<SPW> &v, uint32_t lane, double *s_red, uint8_t *arg = nullptr)
@@ -274,14 +292,8 @@ __device__ __forceinline__ void run_steps(const uint32_t *__restrict__ prog, con
         const uint32_t *tab = offtab + tab_off;
         const bool pairs = (flags & kFusedPairs) != 0;
         double zacc;
-        switch (k) {
-        case 1: zacc = entries_dispatch<1, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        case 2: zacc = entries_dispatch<2, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        case 3: zacc = entries_dispatch<3, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        case 4: zacc = entries_dispatch<4, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        case 5: zacc = entries_dispatch<5, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        default: zacc = entries_dispatch<6, G, SPW, MAX>(v, op, amask, pairs, tab, n_out, cx, lane, d); break;
-        }
+        if (MIXED && !(flags & kFusedMax)) zacc = step_entries<G, SPW, false>(k, v, op, amask, pairs, tab, n_out, cx, lane, d);
+        else zacc = step_entries<G, SPW, MAX>(k, v, op, amask, pairs, tab, n_out, cx, lane, d);
         if (!MAX && (flags & kFusedWantZ) && zout) {      // uniform over the lanes of the set; only single queries ask for it
             double z = zacc;
             if (G <= 32) {
@@ -304,7 +316,7 @@ __device__ __forceinline__ void run_steps(const uint32_t *__restrict__ prog, con
 }
 
 // the evidence sets of a launch, a group of G lanes each
-template <int G, bool MAX>
+template <int G, bool MAX, bool MIXED = false>
 __device__ __forceinline__ void run_sets(const FusedLaunch &p, double *s_red, uint8_t *arg)
 {
     constexpr int SPW = G >= 32 ? 1 : 32 / G;       // sets per warp, interleaved in the warp's slice of the arena
@@ -331,7 +343,7 @@ __device__ __forceinline__ void run_sets(const FusedLaunch &p, double *s_red, ui
         const bool live = b < p.nb;      // lanes of a missing set repeat the last one (they take part in the syncs), stores off
         if (!live) b = p.nb - 1;
         const uint8_t *ev = p.ev ? p.ev + (uint64_t)b * p.n_obs : p.ev_inline;
-        run_steps<G, SPW, MAX>(p.prog, p.offtab, p.n_steps, ev, p.n_obs, p.result, p.z, p.nb, b, live, v, lane, s_red, arg);
+        run_steps<G, SPW, MAX, MIXED>(p.prog, p.offtab, p.n_steps, ev, p.n_obs, p.result, p.z, p.nb, b, live, v, lane, s_red, arg);
     }
 }
 
@@ -347,6 +359,13 @@ template <int G>
 __global__ void __launch_bounds__(kFusedThreads) ve_fused_max(const __grid_constant__ FusedMaxLaunch p)
 {
     run_sets<G, true>(p.f, nullptr, p.arg);
+}
+
+// a MAP program over a batch: kFusedMax steps take the maximum and write their argmax rows, the others sum (fused.hpp)
+template <int G>
+__global__ void __launch_bounds__(kFusedThreads) ve_fused_mixed(const __grid_constant__ FusedMaxLaunch p)
+{
+    run_sets<G, true, true>(p.f, nullptr, p.arg);
 }
 
 // K10 -- TASKS: one launch runs many independent programs of one query, a CTA each.  A mixed plan (hundreds of tiny
@@ -409,6 +428,23 @@ int fused_max_launch(bnpp_ctx *ctx, int G, const FusedMaxLaunch &p)
     }
     static const char *const names[6] = {"ve_fused_max<G=2>", "ve_fused_max<G=4>", "ve_fused_max<G=8>", "ve_fused_max<G=16>",
                                          "ve_fused_max<G=32>", "ve_fused_max<G=128>"};
+    return launch_sets(ctx, G, reinterpret_cast<const void *>(fn), const_cast<FusedMaxLaunch *>(&p), p.f, names);
+}
+
+int fused_mixed_launch(bnpp_ctx *ctx, int G, const FusedMaxLaunch &p)
+{
+    fused_max_fn fn = nullptr;
+    switch (G) {
+    case 2: fn = ve_fused_mixed<2>; break;
+    case 4: fn = ve_fused_mixed<4>; break;
+    case 8: fn = ve_fused_mixed<8>; break;
+    case 16: fn = ve_fused_mixed<16>; break;
+    case 32: fn = ve_fused_mixed<32>; break;
+    case 128: fn = ve_fused_mixed<128>; break;
+    default: break;
+    }
+    static const char *const names[6] = {"ve_fused_mixed<G=2>", "ve_fused_mixed<G=4>", "ve_fused_mixed<G=8>", "ve_fused_mixed<G=16>",
+                                         "ve_fused_mixed<G=32>", "ve_fused_mixed<G=128>"};
     return launch_sets(ctx, G, reinterpret_cast<const void *>(fn), const_cast<FusedMaxLaunch *>(&p), p.f, names);
 }
 

@@ -25,7 +25,7 @@ constexpr int kFusedInlineEv = 256;     // single query: evidence values travel 
 //   [3] out_off   arena offset of the output, or offset into the result buffer (kFusedToResult)
 //   [4] tab_off   first word of this step's operand-offset table [k][n_out] in `offtab`
 //   [5..6] device address of the output (kFusedToGlobal: a later launch of the plan reads it)
-//   [7] kFusedMax: R_s, the first argmax row of the step (MPE plans; 0 otherwise)
+//   [7] kFusedMax: R_s, the first argmax row of the step (MPE / MAP plans; 0 otherwise)
 // then k operand records, 4 words each
 //   [0] kind | nobs << 8     kind 0: intermediate in the arena, 1: resident CPT view
 //   [1] arena offset         | low  32 bits of the CPT's device address
@@ -36,8 +36,9 @@ constexpr uint32_t kFusedToResult = 1u;     // flags
 constexpr uint32_t kFusedWantZ = 2u;
 constexpr uint32_t kFusedToGlobal = 8u;     // the output goes to the device address in header words 5 (low) and 6 (high), dense
 constexpr uint32_t kFusedPairs = 4u;        // cx == 2 and every arena operand holds the eliminated variable at stride 1 on even offsets
-constexpr uint32_t kFusedMax = 16u;         // an eliminating step of an MPE program: the argmax of output entry o for set b
-                                            // goes to byte (R_s + o) * nb + b of the launch's argmax rows (ve_fused_max)
+constexpr uint32_t kFusedMax = 16u;         // a max step of an MPE / MAP program: the argmax of output entry o for set b
+                                            // goes to byte (R_s + o) * nb + b of the launch's argmax rows (ve_fused_max,
+                                            // ve_fused_mixed: there the steps without this flag sum)
 constexpr uint32_t kFusedHeaderWords = 8;
 constexpr uint32_t kFusedOperandWords = 4;
 
@@ -54,7 +55,8 @@ struct FusedLaunch {
 
 // ve_fused_max: the launch of an MPE program -- every step takes the maximum over its eliminated variable (products
 // as in the sum path; the maximum starts at x = 0, a later x replaces it only if strictly greater) and a kFusedMax
-// step writes its argmax bytes to `arg` ([rows][nb], rows of header word 7); result = the value of every set
+// step writes its argmax bytes to `arg` ([rows][nb], rows of header word 7); result = the value of every set.
+// ve_fused_mixed (a MAP program that also sums) takes the same launch: only kFusedMax steps take the maximum.
 struct FusedMaxLaunch {
     FusedLaunch f;
     uint8_t *arg;
@@ -85,5 +87,6 @@ bool fused_valid_g(int G);
 size_t fused_smem_bytes(int G, uint32_t arena);
 int fused_launch(bnpp_ctx *ctx, int G, const FusedLaunch &p);
 int fused_max_launch(bnpp_ctx *ctx, int G, const FusedMaxLaunch &p);
+int fused_mixed_launch(bnpp_ctx *ctx, int G, const FusedMaxLaunch &p);
 
 }  // namespace bnpp

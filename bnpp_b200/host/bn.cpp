@@ -98,6 +98,24 @@ static void execute_mpe()
     cout << ">> Executed in " << uptime << "ms." << endl << endl;
 }
 
+// prompt command `map <id>[, <id>...]`: marginal MAP of those variables under the file's evidence and ordering flags
+static void execute_map(const smatch &m)
+{
+    vector<unsigned> map_vars;
+    const string list = m[1];
+    const regex id("[0-9]+");
+    for (sregex_iterator it(list.begin(), list.end(), id), end; it != end; ++it) map_vars.push_back(stoi(it->str()));
+    double uptime;
+    vector<unsigned> assignment;
+    const double p = model->map(map_vars, evidence, options, assignment, uptime);
+    sort(map_vars.begin(), map_vars.end());
+    cout << ">> MAP = " << p << endl;
+    cout << ">> Assignment =";
+    for (unsigned v : map_vars) cout << " " << v << "=" << assignment[v];
+    cout << endl;
+    cout << ">> Executed in " << uptime << "ms." << endl << endl;
+}
+
 static void execute_marginals()
 {
     double uptime;
@@ -249,6 +267,7 @@ static void prompt()
         {regex("leaves"), [](const smatch &) { print_ids(">> Leaves:", model->leaves()); }},
         {regex("blanket\\s*([0-9]+)"), execute_blanket},
         {regex("width"), [](const smatch &) { execute_width(); }},
+        {regex("map\\s+([0-9]+(\\s*,\\s*[0-9]+)*)"), execute_map},
         {regex("help"), [](const smatch &) { print_help(); }},
     };
     const regex quit("quit");

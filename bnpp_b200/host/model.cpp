@@ -303,6 +303,72 @@ double Model::mpe(const std::unordered_map<unsigned,unsigned> &evidence, std::un
     return host[0];
 }
 
+double Model::map(const std::vector<unsigned> &map_vars, const std::unordered_map<unsigned,unsigned> &evidence,
+                  std::unordered_map<std::string,bool> &options, std::vector<unsigned> &assignment, double &uptime) const
+{
+    Stopwatch sw;
+    std::vector<const Factor*> factors(_factors.begin(), _factors.end());
+    const int nvars = (int)_variables.size();
+    std::vector<unsigned> card;
+    for (const Variable *pv : _variables) card.push_back(pv->size());
+    std::vector<char> in_map(nvars, 0);
+    for (unsigned v : map_vars)
+        if (v < (unsigned)nvars) in_map[v] = 1;
+    std::vector<unsigned> summed, last;
+    for (const Variable *pv : _variables) {
+        const unsigned id = pv->id();
+        if (evidence.find(id) != evidence.end()) continue;
+        if (!in_map[id]) summed.push_back(id);
+    }
+    for (unsigned v : map_vars)
+        if (evidence.find(v) == evidence.end()) last.push_back(v);
+    std::sort(last.begin(), last.end());
+    std::vector<bnpp_scope> scopes(factors.size());
+    std::vector<const double*> tables(factors.size());
+    for (size_t i = 0; i < factors.size(); ++i) {
+        const Domain &d = factors[i]->domain();
+        scopes[i].rank = (int32_t)d.width();
+        scopes[i].var_id = d.ids().data();
+        scopes[i].card = d.cards().data();
+        tables[i] = factors[i]->device_data();
+    }
+    std::vector<uint32_t> obs_var, obs_val;
+    for (const auto &e : evidence) {
+        obs_var.push_back(e.first);
+        obs_val.push_back(e.second);
+    }
+    std::vector<uint32_t> ids(summed.begin(), summed.end());
+    ids.insert(ids.end(), last.begin(), last.end());
+    if (options["min-fill"] || options["weighted-min-fill"] || options["min-degree"]) {
+        int h = 0;
+        if (options["min-degree"]) h = 2;
+        else if (options["weighted-min-fill"]) h = 1;
+        uint32_t n = 0, width = 0;
+        gpu::check(bnpp_elim_order_constrained(nvars, card.data(), (int)factors.size(), scopes.data(), (int)obs_var.size(),
+                                               obs_var.data(), (int)summed.size(), summed.data(), (int)last.size(), last.data(),
+                                               h, ids.data(), &n, &width), "bnpp_elim_order_constrained");
+        ids.resize(n);
+    }
+    std::vector<uint32_t> mv(map_vars.begin(), map_vars.end());
+    bnpp_ctx *ctx = gpu::ctx();
+    bnpp_ve_plan *plan = nullptr;
+    gpu::check(bnpp_map_plan_create(ctx, nvars, card.data(), (int)factors.size(), scopes.data(), (int)obs_var.size(),
+                                    obs_var.data(), (int)mv.size(), mv.data(), (int)ids.size(), ids.data(), &plan),
+               "bnpp_map_plan_create");
+    // [value, assignment as uint32 words]: one buffer, one download
+    double *res = nullptr;
+    gpu::check(bnpp_alloc(ctx, 1 + ((uint64_t)nvars + 1) / 2, &res), "bnpp_alloc");
+    gpu::check(bnpp_mpe_plan_run(plan, tables.data(), obs_val.data(), res, reinterpret_cast<uint32_t *>(res + 1)), "bnpp_mpe_plan_run");
+    std::vector<double> host(1 + ((size_t)nvars + 1) / 2);
+    gpu::check(bnpp_download(ctx, host.data(), res, host.size()), "bnpp_download");
+    bnpp_free(ctx, res);
+    bnpp_ve_plan_destroy(plan);
+    assignment.assign(nvars, 0);
+    std::memcpy(assignment.data(), host.data() + 1, sizeof(unsigned) * nvars);
+    uptime = sw.ms();
+    return host[0];
+}
+
 // ------------------------------------------------------------------------------------------
 // BN
 // ------------------------------------------------------------------------------------------

@@ -60,6 +60,13 @@ public:
     // partition_ve, else variables in id order.  Ties go to the lowest values.
     double mpe(const std::unordered_map<unsigned,unsigned> &evidence, std::unordered_map<std::string,bool> &options,
                std::vector<unsigned> &assignment, double &uptime) const;
+    // Marginal MAP (no reference counterpart): the jointly most probable assignment of the MAP variables `map_vars`
+    // given the evidence, every other unobserved variable summed out, and its value max_{x_M} sum_{x_S} prod_f f(x, e)
+    // (assignment[id]: MAP variables their decoded value, observed ones their evidence, summed ones BNPP_ASSIGN_SUMMED).
+    // The order eliminates the summed variables first: with -mf / -wmf / -md the constrained heuristic order
+    // (bnpp_elim_order_constrained), else each group in id order.  Ties go to the lowest values in decode order.
+    double map(const std::vector<unsigned> &map_vars, const std::unordered_map<unsigned,unsigned> &evidence,
+               std::unordered_map<std::string,bool> &options, std::vector<unsigned> &assignment, double &uptime) const;
 
 protected:
     std::string _name;

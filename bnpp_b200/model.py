@@ -50,6 +50,11 @@ def _declare(L):
     L.bnpp_mpe_plan_run.argtypes = [ctypes.c_void_p, P(ctypes.c_void_p), capi.c_u32p, ctypes.c_void_p, ctypes.c_void_p]
     L.bnpp_mpe_plan_run_batched.argtypes = [ctypes.c_void_p, P(ctypes.c_void_p), ctypes.c_uint32, ctypes.c_uint32,
                                             ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
+    L.bnpp_elim_order_constrained.argtypes = [ctypes.c_int, capi.c_u32p, ctypes.c_int, P(capi.Scope), ctypes.c_int,
+                                              capi.c_u32p, ctypes.c_int, capi.c_u32p, ctypes.c_int, capi.c_u32p, ctypes.c_int,
+                                              capi.c_u32p, capi.c_u32p, capi.c_u32p]
+    L.bnpp_map_plan_create.argtypes = [ctypes.c_void_p, ctypes.c_int, capi.c_u32p, ctypes.c_int, P(capi.Scope), ctypes.c_int,
+                                       capi.c_u32p, ctypes.c_int, capi.c_u32p, ctypes.c_int, capi.c_u32p, P(ctypes.c_void_p)]
     L._ve_declared = True
 
 
@@ -83,6 +88,27 @@ def elim_order(cards, scopes, variables, heuristic, reference_containers=False, 
                            ctypes.byref(n), ctypes.byref(width))
     if rc != 0:
         raise capi.BnppError(rc, "bnpp_elim_order")
+    return list(out[:n.value]), width.value
+
+
+def elim_order_constrained(cards, scopes, first, last, heuristic, reference_containers=False, observed=(), _arr=None,
+                           _cards=None):
+    """the constrained order of marginal MAP -> (order, width): `first` (the summed variables) exactly as `elim_order`
+    orders them, then `last` (the MAP variables) by the same heuristic on the same graph, the fill edges of the first
+    phase in place; width over both phases.  Host only."""
+    L = capi.lib()
+    _declare(L)
+    arr = _arr if _arr is not None else _scopes(scopes, cards)[0]
+    c = _cards if _cards is not None else capi._u32(cards)
+    f, la, ob = capi._u32(first), capi._u32(last), capi._u32(list(observed))
+    out = (ctypes.c_uint32 * max(1, len(first) + len(last)))()
+    width, n = ctypes.c_uint32(), ctypes.c_uint32()
+    rc = L.bnpp_elim_order_constrained(len(cards), ctypes.cast(c, capi.c_u32p), len(scopes), arr, len(observed),
+                                       ctypes.cast(ob, capi.c_u32p), len(first), ctypes.cast(f, capi.c_u32p), len(last),
+                                       ctypes.cast(la, capi.c_u32p), HEUR[heuristic] | (0x100 if reference_containers else 0),
+                                       ctypes.cast(out, capi.c_u32p), ctypes.byref(n), ctypes.byref(width))
+    if rc != 0:
+        raise capi.BnppError(rc, "bnpp_elim_order_constrained")
     return list(out[:n.value]), width.value
 
 
@@ -254,6 +280,36 @@ class MPEPlan(VEPlan):
         """the engine of batched runs: the whole plan in one launch per slice when every step is small (default), or one
         launch per bucket; single runs are always one launch per bucket"""
         super().set_fused(on)
+
+
+class MAPPlan(MPEPlan):
+    """bnpp_map_plan: marginal MAP over the schedule of a VEPlan -- steps eliminating a MAP variable take the maximum
+    (and keep their argmax tables for the decode), every other eliminating step sums.  `order` must eliminate every
+    summed variable before any MAP variable.  Runs as an MPEPlan (run_mpe, run_mpe_batched); a summed variable reports
+    ASSIGN_SUMMED (0xFFFFFFFF; 0xFF in a batch).  ctx.h may be None: a dry plan."""
+
+    def __init__(self, ctx, cards, scopes, observed, order, map_vars=(), _arr=None):
+        self.ctx = ctx
+        L = ctx.L
+        _declare(L)
+        arr, self._keep = (_arr, None) if _arr is not None else _scopes(scopes, cards)
+        self.observed = list(observed)
+        self.map_vars = list(map_vars)
+        self.nvars = len(cards)
+        c, ov, mv, od = capi._u32(cards), capi._u32(self.observed), capi._u32(self.map_vars), capi._u32(order)
+        h = ctypes.c_void_p()
+        ctx.check(L.bnpp_map_plan_create(ctx.h, len(cards), ctypes.cast(c, capi.c_u32p), len(scopes), arr,
+                                         len(self.observed), ctypes.cast(ov, capi.c_u32p), len(self.map_vars),
+                                         ctypes.cast(mv, capi.c_u32p), len(order), ctypes.cast(od, capi.c_u32p),
+                                         ctypes.byref(h)))
+        self.h = h
+        self.result_size = 1
+        vals = [ctypes.c_uint64() for _ in range(5)]
+        ctx.check(L.bnpp_ve_plan_info(h, None, None, None, *[ctypes.byref(v) for v in vals]))
+        self.n_launches, self.union_entries, self.bytes, self.peak_bytes, self.max_step_entries = [v.value for v in vals]
+
+
+ASSIGN_SUMMED = 0xFFFFFFFF
 
 
 class BN:
@@ -434,6 +490,77 @@ class BN:
         assignment = [int(x) for x in host[2:].view(np.uint32)]
         self.last_timing = {"order_ms": (t1 - t0) * 1e3, "plan_ms": (t2 - t1) * 1e3, "run_ms": (t3 - t2) * 1e3}
         return value, assignment, (time.perf_counter() - t0) * 1e3
+
+    def _map_plan(self, map_vars, observed, heuristic):
+        """the MAP plan of (MAP variables, observed ids, heuristic): heuristic None orders the summed variables, then the
+        MAP variables, each in id order; else the constrained heuristic order"""
+        m = sorted(int(v) for v in map_vars)        # a repeated, observed or unknown id: BNPP_EINVAL from the library
+        okey = ("map", tuple(observed), tuple(m), heuristic)
+        order = self._order_cache.get(okey)
+        if order is None:
+            obs, ms = set(observed), set(m)
+            summed = [v for v in range(self.nvars) if v not in obs and v not in ms]
+            if heuristic is None:
+                order = summed + [v for v in m if v not in obs]
+            else:
+                order, _ = elim_order_constrained(self.cards, self.scopes, summed, m, heuristic, observed=sorted(observed),
+                                                  _arr=self._scope_arr, _cards=self._cards_arr)
+            if len(self._order_cache) >= self.MAX_PLANS:
+                self._order_cache.pop(next(iter(self._order_cache)))
+            self._order_cache[okey] = order
+
+        def make(ctx, cards, scopes, obs_, order_, _arr=None):
+            return MAPPlan(ctx, cards, scopes, obs_, order_, map_vars=m, _arr=_arr)
+        return self._cached_plan(("map", tuple(observed), tuple(m), tuple(order)), make, observed, order)
+
+    def map(self, map_vars, evidence=None, heuristic=None):
+        """Marginal MAP (no reference counterpart) -> (value, {v: x_v for v in map_vars}, uptime_ms).
+        value = max over the MAP variables of the sum over every other unobserved variable of the product of every CPT
+        conditioned on the evidence, i.e. P(x_M*, e), not normalised.  Ties go to the lowest values in decode order.
+        The order eliminates the summed variables first (heuristic None: each group in id order; else the constrained
+        heuristic order of `elim_order_constrained`)."""
+        t0 = time.perf_counter()
+        evidence = dict(evidence or {})
+        observed = sorted(evidence)
+        map_vars = [int(v) for v in map_vars]
+        p = self._map_plan(map_vars, observed, heuristic)
+        t1 = time.perf_counter()
+        n = self.nvars
+        if getattr(self, "_mpe_buf", None) is None or self._mpe_buf.numel() != 2 + n:
+            with torch.cuda.stream(self.ctx.torch_stream):
+                self._mpe_buf = torch.empty(2 + n, dtype=torch.int32, device=self._dev.device)
+                self._mpe_host = torch.empty(2 + n, dtype=torch.int32).pin_memory()
+        p.run_mpe(self.table_ptrs, [evidence[v] for v in observed], self._mpe_buf.data_ptr(), self._mpe_buf.data_ptr() + 8)
+        with torch.cuda.stream(self.ctx.torch_stream):
+            self._mpe_host.copy_(self._mpe_buf, non_blocking=True)
+        self.ctx.sync()
+        t2 = time.perf_counter()
+        host = self._mpe_host.numpy()
+        value = float(host[:2].view(np.float64)[0])
+        assignment = host[2:].view(np.uint32)
+        self.last_timing = {"plan_ms": (t1 - t0) * 1e3, "run_ms": (t2 - t1) * 1e3}
+        return value, {v: int(assignment[v]) for v in map_vars}, (time.perf_counter() - t0) * 1e3
+
+    def map_batch(self, map_vars, observed, values, heuristic="mf", host_values=None):
+        """Marginal MAP for a batch of evidence sets sharing the observed ids, the batched counterpart of `map`.
+        observed: sorted variable ids; values: torch.uint8 CUDA tensor [nb][len(observed)] (or host_values, a pinned
+        uint8 tensor, to include the H2D copy).  -> (value [nb] float64, assignment [nvars][nb] uint8), device tensors:
+        a MAP variable's row holds its decoded values, an observed variable's the evidence, a summed variable's 0xFF.
+        Every set equals its single run of the same plan bit for bit.  The tensors are the model's result buffers
+        for MAP batches of nb sets (see `mpe_batch`: synchronise before reading them elsewhere, clone to keep them)."""
+        observed = list(observed)
+        p = self._map_plan([int(v) for v in map_vars], observed, heuristic)
+        with torch.cuda.stream(self.ctx.torch_stream):
+            if host_values is not None:
+                values = host_values.to(self._dev.device, non_blocking=True)
+            nb = values.shape[0]
+            out = self._batch_out.get(("map", nb))
+            if out is None:
+                out = self._batch_out[("map", nb)] = (torch.empty(nb, dtype=torch.float64, device=self._dev.device),
+                                                       torch.empty((self.nvars, nb), dtype=torch.uint8, device=self._dev.device))
+        p.run_mpe_batched(self.table_ptrs, nb, values.data_ptr(), out[0].data_ptr(), out[1].data_ptr())
+        self._keep_alive = values
+        return out
 
     def partition_batch(self, observed, values, heuristic="mf", host_values=None):
         """PR for a batch of evidence sets sharing the observed ids (config 5).

@@ -166,6 +166,15 @@ int bnpp_reduce(bnpp_ctx *ctx, int op, uint64_t n, const double *in_dev, double 
 int bnpp_elim_order(int nvars, const uint32_t *card, int nfac, const bnpp_scope *scopes, int n_obs,
                     const uint32_t *obs_var, int n_vars_to_order, const uint32_t *vars, int heuristic,
                     uint32_t *order_out, uint32_t *n_order_out, uint32_t *width_out);
+/* Constrained elimination order for marginal MAP (no reference counterpart): `first` (the summed
+ * variables) ordered exactly as bnpp_elim_order orders them, then `last` (the MAP variables) ordered
+ * by the same heuristic on the same conditioned graph with the fill edges of the first phase in
+ * place.  heuristic | 0x100 as for bnpp_elim_order.  order_out must hold n_first + n_last ids;
+ * *width_out receives the width over both phases.  Needs no device. */
+int bnpp_elim_order_constrained(int nvars, const uint32_t *card, int nfac, const bnpp_scope *scopes, int n_obs,
+                                const uint32_t *obs_var, int n_first, const uint32_t *first, int n_last,
+                                const uint32_t *last, int heuristic, uint32_t *order_out, uint32_t *n_order_out,
+                                uint32_t *width_out);
 /* Wide-factor sharding over G = 2^g GPUs (SURVEY §8e; no reference counterpart): the g variables of
  * the widest elimination clique that `order` eliminates last.  Every rank then runs the ordinary
  * plan with these variables observed at its rank's values; bnpp_shard_allreduce_sum
@@ -218,22 +227,44 @@ int bnpp_ve_plan_run(bnpp_ve_plan *plan, const double *const *tables_dev, const 
  * BNPP_EINVAL.  bnpp_ve_plan_run / _run_batched / _run_sharded return BNPP_EINVAL on an MPE plan. */
 int bnpp_mpe_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfac, const bnpp_scope *scopes,
                          int n_obs, const uint32_t *obs_var, int n_order, const uint32_t *order, bnpp_ve_plan **out);
+/* Marginal MAP (no reference counterpart): the jointly most probable assignment of the MAP variables
+ * map_var[n_map] given the evidence, every other unobserved variable summed out, and its value
+ * max_{x_M} sum_{x_S} prod_f f(x, e)  -- P(x_M*, e) for a Bayesian network, not normalised.  The steps
+ * are those of bnpp_ve_plan_create for the same order; a step eliminating a MAP variable is a max step
+ * (rule and argmax table of bnpp_product_max_out), every other eliminating step sums.  The argmax
+ * arena, the argmax rows of batches (R_s: the sum of n_out over the MAX steps before s) and the decode
+ * cover the max steps only.  The order must eliminate every summed variable before any MAP variable
+ * (constrained elimination: bnpp_elim_order_constrained), which makes the result exact.  M = every
+ * unobserved variable gives the MPE plan of bnpp_mpe_plan_create; M empty gives the value of
+ * bnpp_ve_plan_run for the same order.  BNPP_EINVAL when a MAP variable is observed, repeated,
+ * >= nvars or has more than 255 values (summed variables may have any), when the order misses an
+ * unobserved variable that some scope mentions, or when it names a MAP variable before a summed one.
+ * ctx may be NULL (a dry plan).  Run it with bnpp_mpe_plan_run / bnpp_mpe_plan_run_batched: a MAP
+ * variable reports its decoded value (0 if no factor mentions it), an observed variable its evidence
+ * value, a summed variable BNPP_ASSIGN_SUMMED in the element type (uint32 0xFFFFFFFF, batch uint8 0xFF). */
+#define BNPP_ASSIGN_SUMMED 0xFFFFFFFFu
+int bnpp_map_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfac, const bnpp_scope *scopes,
+                         int n_obs, const uint32_t *obs_var, int n_map, const uint32_t *map_var, int n_order,
+                         const uint32_t *order, bnpp_ve_plan **out);
+/* run an MPE or MAP plan for one evidence set (see above) */
 int bnpp_mpe_plan_run(bnpp_ve_plan *plan, const double *const *tables_dev, const uint32_t *obs_val,
                       double *value_dev, uint32_t *assignment_dev);
-/* MPE for a BATCH of evidence sets over one MPE plan: ev_dev [nb][n_obs] uint8 as for
+/* MPE or MAP for a BATCH of evidence sets over one MPE or MAP plan: ev_dev [nb][n_obs] uint8 as for
  * bnpp_ve_plan_run_batched; value_dev receives [nb] doubles, assignment_dev [nvars][nb] uint8 (batch
  * fastest).  Every set's value and assignment equal, bit for bit, what bnpp_mpe_plan_run returns for its
  * evidence: the observed variables report the values the set was computed with, a variable no factor
  * mentions reports 0.  A value >= its variable's cardinality is read as 0 (and reported as 0) and raises
  * BNPP_STATUS_BAD_EVIDENCE.  Engines as for batched PR: the whole plan in one launch per slice (K9,
- * ve_fused_max) when fused_info accepts the plan for nb > 1 sets, else one launch per bucket (K8's
- * max-product variants, replayed as a captured graph from the third run with the same buffers on);
+ * ve_fused_max; a MAP plan with both max and summing steps ve_fused_mixed) when fused_info accepts the
+ * plan for nb > 1 sets, else one launch per bucket (K8's max-product variants for max steps, its sum
+ * kernels for the others, replayed as a captured graph from the third run with the same buffers on);
  * bnpp_ve_plan_set_fused(plan, 0) forces K8.  A decode launch per slice, one thread per set, follows.
- * Argmax layout, shared by both engines: eliminating step s (plan order, bnpp_ve_plan_describe) owns the
- * rows [R_s, R_s + n_out_s) of a plan-owned byte scratch, R_s = the sum of n_out over the eliminating steps
- * before it; the argmax of its output entry o for set b of a slice of `slice` sets is at byte
+ * A MAP plan's summed variables report 0xFF.
+ * Argmax layout, shared by both engines: max step s (plan order, bnpp_ve_plan_describe; every eliminating
+ * step of an MPE plan) owns the rows [R_s, R_s + n_out_s) of a plan-owned byte scratch, R_s = the sum of
+ * n_out over the max steps before it; the argmax of its output entry o for set b of a slice of `slice` sets is at byte
  * (R_s + o) * slice + b.  Batches are cut into slices so that the scratch stays within 1 GiB (K8: also its
- * widest intermediate).  A non-MPE plan, an n_obs other than the plan's, a NULL buffer or nb == 0 returns
+ * widest intermediate).  A plan that is neither MPE nor MAP, an n_obs other than the plan's, a NULL buffer or nb == 0 returns
  * BNPP_EINVAL. */
 int bnpp_mpe_plan_run_batched(bnpp_ve_plan *plan, const double *const *tables_dev, uint32_t nb, uint32_t n_obs,
                               const uint8_t *ev_dev, double *value_dev, uint8_t *assignment_dev);
@@ -267,9 +298,10 @@ int bnpp_ve_plan_run_batched(bnpp_ve_plan *plan, const double *const *tables_dev
  * lanes owns an evidence set and walks the bucket loop of code/model.cpp:409-439 with the
  * intermediates of the set in shared memory; results are bit-identical to the launch-per-bucket
  * path.  On by default (environment BNPP_FUSED=0 turns it off for new plans); set_fused(plan, 0)
- * forces one launch per bucket.  On an MPE plan it selects the engine of bnpp_mpe_plan_run_batched
- * only (single MPE runs are always launch-per-bucket), and fused_info / fused_program describe the
- * max-mode program (fused.hpp: kFusedMax steps carry their first argmax row R_s in header word 7).  fused_info: lanes per evidence set a run over nb sets would use
+ * forces one launch per bucket.  On an MPE or MAP plan it selects the engine of bnpp_mpe_plan_run_batched
+ * only (single MPE / MAP runs are always launch-per-bucket), and fused_info / fused_program describe the
+ * max-mode program (fused.hpp: kFusedMax steps carry their first argmax row R_s in header word 7; in a MAP
+ * program exactly the max steps carry the flag).  fused_info: lanes per evidence set a run over nb sets would use
  * (0 = not fused), shared-memory doubles per set, steps in the launch. */
 int bnpp_ve_plan_set_fused(bnpp_ve_plan *plan, int on);
 int bnpp_ve_plan_fused_info(bnpp_ve_plan *plan, uint32_t nb, int32_t *lanes_per_set, uint32_t *arena_doubles,
