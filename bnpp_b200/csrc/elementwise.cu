@@ -103,6 +103,37 @@ int normalize_segments(bnpp_ctx *ctx, double *buf, const uint32_t *off_dev, cons
     return BNPP_OK;
 }
 
+// normalize_segments_kernel for a batch laid out [entries][nb] (batch fastest): one thread per (slice, set), the same
+// index-order sum and true division, so every set's column gets the bits of its own single run.  Neighbouring
+// threads are neighbouring sets of one slice: every read and write of a warp is one contiguous run.
+__global__ void normalize_segments_batched_kernel(double *buf, const uint32_t *__restrict__ off, const uint32_t *__restrict__ size,
+                                                  uint64_t n_items, uint32_t nb)
+{
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_items) return;
+    const uint32_t s = (uint32_t)(t / nb);
+    double *p = buf + (uint64_t)off[s] * nb + (t - (uint64_t)s * nb);
+    const uint32_t m = size[s];
+    if (m == 1) {
+        p[0] = 1.0;
+        return;
+    }
+    double z = 0.0;
+    for (uint32_t i = 0; i < m; ++i) z = __dadd_rn(z, p[(uint64_t)i * nb]);
+    for (uint32_t i = 0; i < m; ++i) p[(uint64_t)i * nb] = __ddiv_rn(p[(uint64_t)i * nb], z);
+}
+
+int normalize_segments_batched(bnpp_ctx *ctx, double *buf, const uint32_t *off_dev, const uint32_t *size_dev, int n, uint32_t nb)
+{
+    if (n <= 0 || nb == 0) return BNPP_OK;
+    const uint64_t items = (uint64_t)n * nb;
+    if ((items + 127) / 128 > 0x7fffffffull) return fail(ctx, BNPP_ETOOBIG, "batched marginals: too many slices x sets");
+    normalize_segments_batched_kernel<<<(unsigned)((items + 127) / 128), 128, 0, ctx->stream>>>(buf, off_dev, size_dev, items, nb);
+    BNPP_CUDA(ctx, cudaGetLastError());
+    ctx->launches++;
+    return BNPP_OK;
+}
+
 static unsigned grid_for(bnpp_ctx *ctx, uint64_t n_items)
 {
     uint64_t b = (n_items + kBlock - 1) / kBlock;

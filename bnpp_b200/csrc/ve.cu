@@ -37,6 +37,7 @@ int contract(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *ou
              double *out_dev, double *z_dev, bool max_mode = false, uint8_t *arg_dev = nullptr);
 int fill(bnpp_ctx *ctx, double *out, uint64_t n, double value);
 int normalize_segments(bnpp_ctx *ctx, double *buf, const uint32_t *off_dev, const uint32_t *size_dev, int n);
+int normalize_segments_batched(bnpp_ctx *ctx, double *buf, const uint32_t *off_dev, const uint32_t *size_dev, int n, uint32_t nb);
 
 struct PlanFactor {
     std::vector<uint32_t> var, card;
@@ -2522,7 +2523,12 @@ static int run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32
                 if (rc != BNPP_OK) return rc;
                 ev = pl->ev_clean;
             }
-            if (!assign_dev) return run_fused(pl, G, tables_dev, nb, ev, nullptr, result_dev, nullptr);
+            if (!assign_dev) {
+                int rc = run_fused(pl, G, tables_dev, nb, ev, nullptr, result_dev, nullptr);
+                if (rc == BNPP_OK && pl->is_mar && pl->normalize)
+                    rc = normalize_segments_batched(ctx, result_dev, pl->mar_off_dev, pl->mar_size_dev, (int)pl->mar_off.size(), nb);
+                return rc;
+            }
             // MPE: slices whose argmax rows fit the scratch, each one ve_fused_max launch and its decode
             const uint32_t slice = batch_slice(pl, nb, false);
             int rc = mpe_batch_prepare(pl, slice);
@@ -2548,9 +2554,12 @@ static int run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32
         key.push_back(assign_dev);
         key.push_back(pl->batch_arg);       // a captured run writes the argmax rows there
     }
+    const bool mar_norm = pl->is_mar && pl->normalize;     // the captured run ends with the batched normaliser
+    key.push_back(reinterpret_cast<const void *>(static_cast<uintptr_t>(mar_norm)));
+    const uint64_t replay_launches = pl->steps.size() + 1 + (mar_norm ? 1 : 0);
     if (pl->batch_exec && key == pl->batch_key) {
         BNPP_CUDA(ctx, cudaGraphLaunch(pl->batch_exec, ctx->stream));
-        ctx->launches += pl->steps.size() + 1;
+        ctx->launches += replay_launches;
         return BNPP_OK;
     }
     if (pl->batch_exec) {
@@ -2570,7 +2579,7 @@ static int run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32
             if (rc == BNPP_OK && e == cudaSuccess && cudaGraphInstantiate(&pl->batch_exec, g, 0) == cudaSuccess) {
                 cudaGraphDestroy(g);
                 BNPP_CUDA(ctx, cudaGraphLaunch(pl->batch_exec, ctx->stream));
-                ctx->launches += pl->steps.size() + 1;
+                ctx->launches += replay_launches;
                 return BNPP_OK;
             }
             if (g) cudaGraphDestroy(g);
@@ -2642,7 +2651,9 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
             if (st.out == -2) {
                 ov = &st.rvar;
                 oc = &st.rcard;
-                dst = result_dev + b0;   // result_size == 1 when slicing
+                // result entry i of set b at result_dev[i * nb + b]: a multi-entry result (a marginals plan) is never
+                // sliced (batch_slice), so there b0 == 0 and cur == nb; a sliced plan's result is one entry, roff 0
+                dst = result_dev + (uint64_t)st.roff * nb + b0;
             } else {
                 const PlanFactor &of = pl->f[st.out];
                 ov = &of.var;
@@ -2662,10 +2673,13 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
         }
         for (double *p : owned)
             if (p) bnpp_free(ctx, p);
-        if (pl->steps.empty() || pl->steps.back().out != -2) rc = fill(ctx, result_dev + b0, cur, 1.0);
+        if (!pl->is_mar && (pl->steps.empty() || pl->steps.back().out != -2)) rc = fill(ctx, result_dev + b0, cur, 1.0);
         if (rc == BNPP_OK && assign_dev) rc = mpe_decode_batch_launch(pl, nb, b0, cur, evt + b0, nb, 1, assign_dev);
     }
     bnpp_free(ctx, evt_store);
+    // inside the run, hence inside its captured graph: a replay normalises too
+    if (rc == BNPP_OK && pl->is_mar && pl->normalize)
+        rc = normalize_segments_batched(ctx, result_dev, pl->mar_off_dev, pl->mar_size_dev, (int)pl->mar_off.size(), nb);
     return rc;
 }
 

@@ -279,9 +279,10 @@ int bnpp_ve_plan_result_size(const bnpp_ve_plan *plan, uint64_t *n);
 int bnpp_mar_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfac, const bnpp_scope *scopes, int n_obs,
                          const uint32_t *obs_var, int n_order, const uint32_t *order, bnpp_ve_plan **out);
 int bnpp_mar_plan_layout(const bnpp_ve_plan *plan, int nvars, uint32_t *off, uint32_t *size, uint64_t *total);
-/* A marginals plan normalises every slice at the end of a run.  set_normalize(plan, 0) leaves the slices
- * unnormalised (P(v, evidence) -- what a sharded run sums over the ranks before it normalises,
- * bnpp_b200_nccl.h); bnpp_mar_plan_normalize then normalises a result buffer in place. */
+/* A marginals plan normalises every slice at the end of a run, single or batched.  set_normalize(plan, 0)
+ * leaves the slices unnormalised (P(v, evidence) -- what a sharded run sums over the ranks before it
+ * normalises, bnpp_b200_nccl.h); bnpp_mar_plan_normalize then normalises the result buffer of a SINGLE
+ * run in place (it does not know a batch's [result_size][nb] layout). */
 int bnpp_ve_plan_set_normalize(bnpp_ve_plan *plan, int on);
 int bnpp_mar_plan_normalize(bnpp_ve_plan *plan, double *result_dev);
 
@@ -290,7 +291,12 @@ int bnpp_mar_plan_normalize(bnpp_ve_plan *plan, double *result_dev);
  * result_dev receives [result_size][nb] doubles, batch fastest (PR: one double per set).
  * One launch per bucket for the whole batch; CPTs are shared, never copied per set.
  * n_obs must equal the plan's; a value >= its variable's cardinality is treated as 0 and raises
- * BNPP_STATUS_BAD_EVIDENCE (bnpp_ctx_status). */
+ * BNPP_STATUS_BAD_EVIDENCE (bnpp_ctx_status).
+ * A marginals plan: entry i of the layout (bnpp_mar_plan_layout) for set b at result_dev[i * nb + b], and
+ * each set's column equals, bit for bit, what bnpp_ve_plan_run returns for its evidence -- normalised
+ * slices (NaN where P(evidence) = 0, as 0/0 in the single run), 1.0 in the one-entry slices.  With
+ * set_normalize(plan, 0) the slices of more than one entry hold the single run's unnormalised values
+ * and the one-entry slices are not written. */
 int bnpp_ve_plan_run_batched(bnpp_ve_plan *plan, const double *const *tables_dev, uint32_t nb, uint32_t n_obs,
                              const uint8_t *ev_dev, double *result_dev);
 /* K9 -- a plan whose elimination steps are all small (every union table <= 2^14 entries: the
