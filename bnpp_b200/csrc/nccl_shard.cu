@@ -1,5 +1,5 @@
-// The cross-shard sum-out of wide-factor sharding: one NCCL all-reduce (fp64 sum) of the ranks'
-// results over NVLink / NVSwitch.  See include/bnpp_b200_nccl.h.
+// The cross-shard steps of wide-factor sharding: one NCCL all-reduce (fp64 sum) of the ranks' results over NVLink /
+// NVSwitch, or for MPE / MAP one all-gather of their (value, assignment) records.  See include/bnpp_b200_nccl.h.
 #include <nccl.h>
 
 #include "../../include/bnpp_b200_nccl.h"
@@ -69,4 +69,43 @@ extern "C" int bnpp_ve_plan_run_sharded(bnpp_ctx *ctx, bnpp_ve_plan *plan, void 
     }
     if (is_mar) return bnpp_normalize(ctx, n, result_dev, z_dev, 0.0, result_dev);     // / sum of the Z_r: true division
     return BNPP_OK;
+}
+
+// MPE / MAP of one sharded network: the cross-shard step of a max is a max, and the winner's assignment must travel
+// with its value.  NCCL has no max-loc, so every rank gathers every rank's (value, assignment) record and one small
+// kernel of the core library picks the winner -- the same on every rank, since all of them see the same records.
+extern "C" int bnpp_mpe_plan_run_sharded(bnpp_ctx *ctx, bnpp_ve_plan *plan, void *nccl_comm, const double *const *tables_dev,
+                                         const uint32_t *obs_val, double *value_dev, uint32_t *assignment_dev)
+{
+    if (!ctx || !plan || !nccl_comm || !value_dev || !assignment_dev) return BNPP_EINVAL;
+    uint32_t nvars = 0;
+    if (bnpp_mpe_plan_nvars(plan, &nvars) != BNPP_OK) {
+        ctx->last_error = "bnpp_mpe_plan_run_sharded: not an MPE or MAP plan";
+        return BNPP_EINVAL;
+    }
+    ncclComm_t comm = static_cast<ncclComm_t>(nccl_comm);
+    int rank = 0, world = 0;
+    ncclResult_t r = ncclCommUserRank(comm, &rank);
+    if (r == ncclSuccess) r = ncclCommCount(comm, &world);
+    if (r != ncclSuccess) {
+        ctx->last_error = std::string("ncclCommUserRank / ncclCommCount: ") + ncclGetErrorString(r);
+        return BNPP_ECUDA;
+    }
+    const uint64_t stride = (2ull + nvars + 1) & ~1ull;       // even: every record's value stays 8-byte aligned
+    double *buf = nullptr;
+    int rc = bnpp_alloc(ctx, (uint64_t)world * stride / 2, &buf);
+    if (rc != BNPP_OK) return rc;
+    uint32_t *records = reinterpret_cast<uint32_t *>(buf);
+    uint32_t *mine = records + (uint64_t)rank * stride;
+    rc = bnpp_mpe_plan_run(plan, tables_dev, obs_val, reinterpret_cast<double *>(mine), mine + 2);
+    if (rc == BNPP_OK) {
+        r = ncclAllGather(mine, records, stride, ncclUint32, comm, ctx->stream);
+        if (r != ncclSuccess) {
+            ctx->last_error = std::string("ncclAllGather: ") + ncclGetErrorString(r);
+            rc = BNPP_ECUDA;
+        }
+    }
+    if (rc == BNPP_OK) rc = bnpp_mpe_shard_select(ctx, (uint32_t)world, nvars, records, value_dev, assignment_dev);
+    const int rc_free = bnpp_free(ctx, buf);
+    return rc != BNPP_OK ? rc : rc_free;
 }

@@ -138,6 +138,60 @@ __global__ void mpe_decode(const __grid_constant__ MpeDecodeParams p)
     if (p.set_one) *p.value = 1.0;
 }
 
+// Max-loc over the ranks of a sharded MPE / MAP run (bnpp_mpe_shard_select): record r = words [r * stride, + stride),
+// its value (a double, words 0-1) and assignment (words 2..).  Candidates are ordered by: a number beats a NaN, a
+// larger value beats a smaller one, then the lower rank -- a total order, so the strided scan and the tree give the
+// winner of the sequential rule (start at rank 0, a later rank replaces it only if strictly greater) in any grouping,
+// except that the sequential rule keeps rank 0 when its value is a NaN: that case is checked last.
+constexpr int kSelectThreads = 256;
+
+__device__ __forceinline__ double record_value(const uint32_t *rec)
+{
+    return __hiloint2double((int)rec[1], (int)rec[0]);
+}
+
+__device__ __forceinline__ bool select_beats(double v, uint32_t r, double bv, uint32_t br)
+{
+    if (r == UINT32_MAX) return false;
+    if (br == UINT32_MAX) return true;
+    const bool n = isnan(v), bn = isnan(bv);
+    if (n != bn) return bn;
+    if (!n && v != bv) return v > bv;
+    return r < br;
+}
+
+__global__ void __launch_bounds__(kSelectThreads) mpe_shard_select(const uint32_t *rec, uint32_t nranks, uint32_t nvars,
+                                                                   uint64_t stride, double *value, uint32_t *assign)
+{
+    __shared__ double s_v[kSelectThreads / 32];
+    __shared__ uint32_t s_r[kSelectThreads / 32];
+    double bv = 0.0;
+    uint32_t br = UINT32_MAX;
+    for (uint32_t r = threadIdx.x; r < nranks; r += blockDim.x) {
+        const double v = record_value(rec + r * stride);
+        if (select_beats(v, r, bv, br)) bv = v, br = r;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double v = __shfl_down_sync(0xffffffffu, bv, o);
+        const uint32_t r = __shfl_down_sync(0xffffffffu, br, o);
+        if (select_beats(v, r, bv, br)) bv = v, br = r;
+    }
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    if (lane == 0) s_v[w] = bv, s_r[w] = br;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int i = 1; i < (int)(blockDim.x >> 5); ++i)
+            if (select_beats(s_v[i], s_r[i], bv, br)) bv = s_v[i], br = s_r[i];
+        if (isnan(record_value(rec))) br = 0;
+        s_r[0] = br;
+    }
+    __syncthreads();
+    const uint32_t *win = rec + s_r[0] * stride;
+    if (threadIdx.x == 0) *value = record_value(win);
+    for (uint32_t v = threadIdx.x; v < nvars; v += blockDim.x) assign[v] = win[2 + v];
+}
+
 // MPE / MAP decode of a batch (bnpp_mpe_plan_run_batched): one thread per set of a slice walks the records of mpe_decode with
 // the FIRST ARGMAX ROW of the step in words 1-2: the argmax of output entry o of a step for set t of the slice is
 // arg[(row + o) * cur + t].  The records are the same for every set, so the threads of a warp always touch one
@@ -2173,6 +2227,30 @@ int bnpp_mpe_plan_run(bnpp_ve_plan *pl, const double *const *tables_dev, const u
     if (!pl) return BNPP_EINVAL;
     if (!pl->is_mpe || !assignment_dev) return fail(pl->ctx, BNPP_EINVAL, "bnpp_mpe_plan_run: not an MPE plan, or no assignment buffer");
     return run_plan(pl, tables_dev, obs_val, value_dev, nullptr, assignment_dev);
+}
+
+int bnpp_mpe_plan_nvars(const bnpp_ve_plan *pl, uint32_t *nvars)
+{
+    if (!pl || !pl->is_mpe || !nvars) return BNPP_EINVAL;
+    *nvars = pl->mpe_nvars;
+    return BNPP_OK;
+}
+
+int bnpp_mpe_shard_select(bnpp_ctx *ctx, uint32_t nranks, uint32_t nvars, const uint32_t *records_dev, double *value_dev,
+                          uint32_t *assignment_dev)
+{
+    if (!ctx) return BNPP_EINVAL;
+    if (nranks == 0 || nvars == 0 || !records_dev || !value_dev || !assignment_dev)
+        return fail(ctx, BNPP_EINVAL, "bnpp_mpe_shard_select: no ranks, no variables or a NULL buffer");
+    const uint64_t stride = (2ull + nvars + 1) & ~1ull;
+    mpe_shard_select<<<1, kSelectThreads, 0, ctx->stream>>>(records_dev, nranks, nvars, stride, value_dev, assignment_dev);
+    BNPP_CUDA(ctx, cudaGetLastError());
+    ctx->launches++;
+    ctx->last_desc = nullptr;
+    ctx->last_kernel = "mpe_shard_select";
+    ctx->last_grid = 1;
+    ctx->last_block = kSelectThreads;
+    return BNPP_OK;
 }
 
 // assign_dev != NULL: an MPE run (result_dev is the value)

@@ -455,13 +455,22 @@ class BN:
         self.last_timing = {"order_ms": (t1 - t0) * 1e3, "plan_ms": (t2 - t1) * 1e3, "run_ms": (t3 - t2) * 1e3}
         return z1, (time.perf_counter() - t0) * 1e3
 
-    def mpe(self, evidence=None, heuristic=None):
+    def mpe(self, evidence=None, heuristic=None, comm=None):
         """Most probable explanation (no reference counterpart) -> (value, assignment list, uptime_ms).
         value = max over the unobserved variables of the product of every CPT conditioned on the evidence, i.e.
         P(x*, e), not normalised; assignment[v] is the evidence value of an observed v.  Ties go to the lowest values.
-        The order is the one `partition` uses (heuristic None: variables in id order)."""
+        The order is the one `partition` uses (heuristic None: variables in id order).
+        comm (a nccl.ShardComm over all ranks): the network is sharded over the ranks exactly as `partition` shards it,
+        every rank maximises over its slab, and the ranks' values and assignments are all-gathered and the best one kept
+        on the device (bnpp_mpe_plan_run_sharded); every rank returns the same answer, the shard variables at the
+        winning rank's values.  The ranks form their products in another order than one GPU does, so the value agrees
+        with the unsharded query to rounding, and under exactly tied maxima the lowest rank wins, which can give another
+        assignment than one GPU.  Batches (`mpe_batch`) are sharded by contiguous slices and need no collective."""
         t0 = time.perf_counter()
         evidence = dict(evidence or {})
+        sharded = comm is not None and comm.world > 1
+        if sharded:
+            evidence, _ = self.shard(evidence, heuristic, comm)
         observed = sorted(evidence)
         okey = (tuple(observed), heuristic)
         order = self._order_cache.get(okey)
@@ -480,7 +489,11 @@ class BN:
             with torch.cuda.stream(self.ctx.torch_stream):
                 self._mpe_buf = torch.empty(2 + n, dtype=torch.int32, device=self._dev.device)
                 self._mpe_host = torch.empty(2 + n, dtype=torch.int32).pin_memory()
-        p.run_mpe(self.table_ptrs, [evidence[v] for v in observed], self._mpe_buf.data_ptr(), self._mpe_buf.data_ptr() + 8)
+        if sharded:
+            comm.run_mpe_sharded(p, self.table_ptrs, [evidence[v] for v in observed], self._mpe_buf.data_ptr(),
+                                 self._mpe_buf.data_ptr() + 8)
+        else:
+            p.run_mpe(self.table_ptrs, [evidence[v] for v in observed], self._mpe_buf.data_ptr(), self._mpe_buf.data_ptr() + 8)
         with torch.cuda.stream(self.ctx.torch_stream):
             self._mpe_host.copy_(self._mpe_buf, non_blocking=True)
         self.ctx.sync()
@@ -491,10 +504,9 @@ class BN:
         self.last_timing = {"order_ms": (t1 - t0) * 1e3, "plan_ms": (t2 - t1) * 1e3, "run_ms": (t3 - t2) * 1e3}
         return value, assignment, (time.perf_counter() - t0) * 1e3
 
-    def _map_plan(self, map_vars, observed, heuristic):
-        """the MAP plan of (MAP variables, observed ids, heuristic): heuristic None orders the summed variables, then the
-        MAP variables, each in id order; else the constrained heuristic order"""
-        m = sorted(int(v) for v in map_vars)        # a repeated, observed or unknown id: BNPP_EINVAL from the library
+    def _map_order(self, m, observed, heuristic):
+        """the elimination order of a MAP query (m: sorted MAP variables): heuristic None orders the summed variables,
+        then the MAP variables, each in id order; else the constrained heuristic order"""
         okey = ("map", tuple(observed), tuple(m), heuristic)
         order = self._order_cache.get(okey)
         if order is None:
@@ -508,29 +520,70 @@ class BN:
             if len(self._order_cache) >= self.MAX_PLANS:
                 self._order_cache.pop(next(iter(self._order_cache)))
             self._order_cache[okey] = order
+        return order
+
+    def _map_plan(self, map_vars, observed, heuristic):
+        """the MAP plan of (MAP variables, observed ids, heuristic), over the order of `_map_order`"""
+        m = sorted(int(v) for v in map_vars)        # a repeated, observed or unknown id: BNPP_EINVAL from the library
+        order = self._map_order(m, observed, heuristic)
 
         def make(ctx, cards, scopes, obs_, order_, _arr=None):
             return MAPPlan(ctx, cards, scopes, obs_, order_, map_vars=m, _arr=_arr)
         return self._cached_plan(("map", tuple(observed), tuple(m), tuple(order)), make, observed, order)
 
-    def map(self, map_vars, evidence=None, heuristic=None):
+    def map_shard(self, map_vars, evidence, heuristic, comm):
+        """wide-factor sharding of a marginal MAP query: the log2(world) MAP variables of the widest elimination clique
+        of the UNSHARDED query's constrained order that it eliminates last (sharding.pick_max_shard_vars: ValueError
+        unless there are that many and they are binary), observed at this rank's values
+        -> (evidence incl. shard values, shard vars)"""
+        from . import sharding
+        g = (comm.world - 1).bit_length()
+        if (1 << g) != comm.world:
+            raise ValueError("wide-factor sharding needs a power-of-two number of ranks")
+        m = sorted(int(v) for v in map_vars)
+        observed = sorted(evidence)
+        key = ("map", tuple(observed), tuple(m), heuristic, g)
+        shard_vars = self._shard_cache.get(key)
+        if shard_vars is None:
+            order = self._map_order(m, observed, heuristic)
+            live = self.conditioned_scopes(set(evidence))
+            shard_vars = self._shard_cache[key] = sharding.pick_max_shard_vars(live, order, g, self.cards, m)
+        full = dict(evidence)
+        full.update(sharding.shard_evidence(shard_vars, comm.rank))
+        return full, shard_vars
+
+    def map(self, map_vars, evidence=None, heuristic=None, comm=None):
         """Marginal MAP (no reference counterpart) -> (value, {v: x_v for v in map_vars}, uptime_ms).
         value = max over the MAP variables of the sum over every other unobserved variable of the product of every CPT
         conditioned on the evidence, i.e. P(x_M*, e), not normalised.  Ties go to the lowest values in decode order.
         The order eliminates the summed variables first (heuristic None: each group in id order; else the constrained
-        heuristic order of `elim_order_constrained`)."""
+        heuristic order of `elim_order_constrained`).
+        comm (a nccl.ShardComm over all ranks): sharded like `mpe`, but the shard variables are MAP variables of the
+        widest clique of the constrained order (`map_shard`): maximising a rank's max-of-sums over the ranks is exact
+        only for maximised shard variables.  Every rank runs the MAP plan over the other MAP variables with the shard
+        variables observed, and returns the same answer; the shard variables report the winning rank's values.  Ties
+        and rounding as for `mpe`.  Batches (`map_batch`) are sharded by contiguous slices and need no collective."""
         t0 = time.perf_counter()
         evidence = dict(evidence or {})
-        observed = sorted(evidence)
         map_vars = [int(v) for v in map_vars]
-        p = self._map_plan(map_vars, observed, heuristic)
+        sharded = comm is not None and comm.world > 1
+        rank_vars = map_vars
+        if sharded:
+            evidence, shard_vars = self.map_shard(map_vars, evidence, heuristic, comm)
+            rank_vars = [v for v in map_vars if v not in shard_vars]
+        observed = sorted(evidence)
+        p = self._map_plan(rank_vars, observed, heuristic)
         t1 = time.perf_counter()
         n = self.nvars
         if getattr(self, "_mpe_buf", None) is None or self._mpe_buf.numel() != 2 + n:
             with torch.cuda.stream(self.ctx.torch_stream):
                 self._mpe_buf = torch.empty(2 + n, dtype=torch.int32, device=self._dev.device)
                 self._mpe_host = torch.empty(2 + n, dtype=torch.int32).pin_memory()
-        p.run_mpe(self.table_ptrs, [evidence[v] for v in observed], self._mpe_buf.data_ptr(), self._mpe_buf.data_ptr() + 8)
+        if sharded:
+            comm.run_mpe_sharded(p, self.table_ptrs, [evidence[v] for v in observed], self._mpe_buf.data_ptr(),
+                                 self._mpe_buf.data_ptr() + 8)
+        else:
+            p.run_mpe(self.table_ptrs, [evidence[v] for v in observed], self._mpe_buf.data_ptr(), self._mpe_buf.data_ptr() + 8)
         with torch.cuda.stream(self.ctx.torch_stream):
             self._mpe_host.copy_(self._mpe_buf, non_blocking=True)
         self.ctx.sync()

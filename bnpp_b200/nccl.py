@@ -1,7 +1,8 @@
 """The path's one collective through the product's own C ABI (include/bnpp_b200_nccl.h).
 
 `ShardComm` owns an ncclComm_t (one rank per GPU) and sums a device buffer over all ranks with
-bnpp_shard_allreduce_sum -- the cross-shard sum-out of wide-factor sharding.  The unique id
+bnpp_shard_allreduce_sum -- the cross-shard sum-out of wide-factor sharding -- or, for MPE and marginal MAP, gathers
+every rank's value and assignment and keeps the best (bnpp_mpe_plan_run_sharded).  The unique id
 travels over torch.distributed (plumbing); the reduction itself does not go through torch.
 """
 import ctypes
@@ -47,6 +48,18 @@ class ShardComm:
                                                       capi.c_u32p, ctypes.c_void_p, ctypes.c_void_p]
         self.ctx.check(self.lib.bnpp_ve_plan_run_sharded(self.ctx.h, plan.h, self.comm, tp, ctypes.cast(ov, capi.c_u32p),
                                                          ctypes.c_void_p(result_ptr), ctypes.c_void_p(z_ptr) if z_ptr else None))
+
+    def run_mpe_sharded(self, plan, table_ptrs, obs_val, value_ptr, assignment_ptr):
+        """bnpp_mpe_plan_run_sharded: this rank's slab of an MPE or MAP plan, then the all-gather of every rank's value
+        and assignment and the max-loc over them; every rank receives the winner's (value_ptr: device double,
+        assignment_ptr: device uint32 [nvars]).  Asynchronous."""
+        tp = (ctypes.c_void_p * max(1, len(table_ptrs)))(*table_ptrs)
+        ov = capi._u32(obs_val)
+        self.lib.bnpp_mpe_plan_run_sharded.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                                       ctypes.POINTER(ctypes.c_void_p), capi.c_u32p, ctypes.c_void_p,
+                                                       ctypes.c_void_p]
+        self.ctx.check(self.lib.bnpp_mpe_plan_run_sharded(self.ctx.h, plan.h, self.comm, tp, ctypes.cast(ov, capi.c_u32p),
+                                                          ctypes.c_void_p(value_ptr), ctypes.c_void_p(assignment_ptr)))
 
     def allreduce_sum(self, ptr, n):
         """in place, on the context's stream"""

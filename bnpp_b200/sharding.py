@@ -4,7 +4,9 @@
 * one wide factor: the log2(G) variables of the widest elimination clique that the order
   eliminates LAST become shard variables.  With the canonical VE layout they are the
   leading axes of every wide table, so fixing them to the bits of a rank selects that
-  rank's slab; summing them out across shards is one all-reduce of the partition.
+  rank's slab; summing them out across shards is one all-reduce of the partition.  For MPE and
+  marginal MAP they must be maximised variables, and maximising them out is one all-gather of every
+  rank's (value, assignment) and a max-loc.
 """
 
 
@@ -17,6 +19,26 @@ def pick_shard_vars(scopes, order, g):
     """the g variables of the widest elimination clique that `order` eliminates last"""
     if g <= 0:
         return []
+    return widest_clique(scopes, order)[-g:]
+
+
+def pick_max_shard_vars(scopes, order, g, cards, max_vars):
+    """shard variables of a query that maximises over `max_vars` (MPE: every unobserved variable; marginal MAP: the MAP
+    variables): the g variables of `max_vars` in the widest elimination clique of `order` that it eliminates last.
+    Taking the max over the ranks of each rank's max over the other MAP variables of a sum over the summed ones is
+    exact only when the shard variables are maximised, so a summed variable is never one.  ValueError when the widest
+    clique holds fewer than g of them or one of the g is not binary."""
+    if g <= 0:
+        return []
+    mx = set(max_vars)
+    picked = [v for v in widest_clique(scopes, order) if v in mx][-g:]
+    if len(picked) != g or any(int(cards[v]) != 2 for v in picked):
+        raise ValueError("no %d binary MAP shard variables in the widest clique" % g)
+    return picked
+
+
+def widest_clique(scopes, order):
+    """the variables of the widest elimination clique of `order` (the first one found), in elimination order"""
     rank = {v: i for i, v in enumerate(order)}
     buckets = {v: [] for v in order}
     for sc in scopes:
@@ -33,7 +55,7 @@ def pick_shard_vars(scopes, order, g):
         u.discard(v)
         if u:
             buckets[min(u, key=rank.get)].append(u)
-    return sorted(best_u, key=rank.get)[-g:]
+    return sorted(best_u, key=rank.get)
 
 
 def shard_evidence(shard_vars, rank, cards=None):

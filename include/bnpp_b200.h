@@ -224,7 +224,8 @@ int bnpp_ve_plan_run(bnpp_ve_plan *plan, const double *const *tables_dev, const 
  * run: assignment_dev[nvars] receives one uint32 per variable id: the evidence value for an
  * observed variable, 0 for a variable no factor mentions; value_dev one double.  Zero-probability
  * evidence gives value 0 and the lowest values.  An evidence value out of range returns
- * BNPP_EINVAL.  bnpp_ve_plan_run / _run_batched / _run_sharded return BNPP_EINVAL on an MPE plan. */
+ * BNPP_EINVAL.  bnpp_ve_plan_run / _run_batched / _run_sharded return BNPP_EINVAL on an MPE plan; one network sharded
+ * over several GPUs runs with bnpp_mpe_plan_run_sharded of bnpp_b200_nccl.h. */
 int bnpp_mpe_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfac, const bnpp_scope *scopes,
                          int n_obs, const uint32_t *obs_var, int n_order, const uint32_t *order, bnpp_ve_plan **out);
 /* Marginal MAP (no reference counterpart): the jointly most probable assignment of the MAP variables
@@ -249,6 +250,17 @@ int bnpp_map_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfa
 /* run an MPE or MAP plan for one evidence set (see above) */
 int bnpp_mpe_plan_run(bnpp_ve_plan *plan, const double *const *tables_dev, const uint32_t *obs_val,
                       double *value_dev, uint32_t *assignment_dev);
+/* the nvars an MPE or MAP plan was created with (the length of its assignment); BNPP_EINVAL for any other plan */
+int bnpp_mpe_plan_nvars(const bnpp_ve_plan *plan, uint32_t *nvars);
+/* Max-loc over the ranks of a sharded MPE or MAP query (bnpp_mpe_plan_run_sharded, bnpp_b200_nccl.h), one block of one
+ * launch (kernel mpe_shard_select).  records_dev holds nranks records of stride = 2 + nvars rounded up to an even number
+ * of uint32 words; rank r's starts at word r * stride: its value (a double, words 0-1, 8-byte aligned) and its assignment
+ * (nvars uint32, words 2..) -- what bnpp_mpe_plan_run writes.  The winner is the largest value; equal values keep the
+ * lowest rank and a NaN never replaces a number (the rule of bnpp_product_max_out over the ranks: rank 0 first, a later
+ * rank replaces it only if strictly greater).  Its value goes to value_dev, its assignment to assignment_dev[nvars].
+ * Asynchronous on the context's stream.  nranks == 0, nvars == 0 or a NULL pointer returns BNPP_EINVAL. */
+int bnpp_mpe_shard_select(bnpp_ctx *ctx, uint32_t nranks, uint32_t nvars, const uint32_t *records_dev, double *value_dev,
+                          uint32_t *assignment_dev);
 /* MPE or MAP for a BATCH of evidence sets over one MPE or MAP plan: ev_dev [nb][n_obs] uint8 as for
  * bnpp_ve_plan_run_batched; value_dev receives [nb] doubles, assignment_dev [nvars][nb] uint8 (batch
  * fastest).  Every set's value and assignment equal, bit for bit, what bnpp_mpe_plan_run returns for its
