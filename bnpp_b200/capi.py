@@ -30,6 +30,7 @@ EXPORTS = [
     "bnpp_sampler_create", "bnpp_sampler_destroy", "bnpp_sampler_logical", "bnpp_sampler_likelihood",
     "bnpp_product_max_out", "bnpp_mpe_plan_create", "bnpp_mpe_plan_run", "bnpp_mpe_plan_run_batched",
     "bnpp_elim_order_constrained", "bnpp_map_plan_create", "bnpp_mpe_plan_nvars", "bnpp_mpe_shard_select",
+    "bnpp_ve_plan_windows",
 ]
 
 

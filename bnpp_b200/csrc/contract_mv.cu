@@ -31,6 +31,7 @@
 #include "common.cuh"
 #include "contract.hpp"
 #include "contract_mv.hpp"
+#include "chain.hpp"
 
 extern "C" int bnpp_alloc(bnpp_ctx *ctx, uint64_t n_doubles, double **dptr);
 extern "C" int bnpp_free(bnpp_ctx *ctx, double *dptr);
@@ -192,6 +193,7 @@ struct MvKnobs {
     uint32_t staged = 1;
     uint32_t staged_tma = 1;
     uint32_t staged_async = 1;
+    uint32_t chain_depth = kChainDefaultDepth;      // levels of a ve.cu window (contract_chain); 0 or 1 = no windows
     MvKnobs()
     {
         const char *e = getenv("BNPP_MV_MIN_ENTRIES");
@@ -202,6 +204,8 @@ struct MvKnobs {
         if (e && e[0] == '0') staged_tma = 0;
         e = getenv("BNPP_STAGED_ASYNC");
         if (e && e[0] == '0') staged_async = 0;
+        e = getenv("BNPP_CHAIN_DEPTH");
+        if (e) chain_depth = (uint32_t)atoi(e);
     }
 };
 static MvKnobs &knobs()
@@ -213,6 +217,7 @@ static MvKnobs &knobs()
 uint64_t mv_min_entries() { return knobs().min_entries; }
 bool mv_staged_enabled() { return knobs().staged != 0; }
 bool staged_tma_enabled() { return knobs().staged_tma != 0; }
+uint32_t chain_depth_knob() { return knobs().chain_depth; }
 bool staged_async_enabled() { return knobs().staged_async != 0; }
 
 static uint32_t mv_emax(int k)
@@ -436,6 +441,7 @@ extern "C" int bnpp_tuning_set(const char *key, uint64_t value)
     else if (!strcmp(key, "mv_staged")) bnpp::knobs().staged = (uint32_t)value;
     else if (!strcmp(key, "staged_tma")) bnpp::knobs().staged_tma = (uint32_t)value;
     else if (!strcmp(key, "staged_async")) bnpp::knobs().staged_async = (uint32_t)value;
+    else if (!strcmp(key, "chain_depth")) bnpp::knobs().chain_depth = (uint32_t)value;
     else return BNPP_EINVAL;
     return BNPP_OK;
 }
@@ -448,6 +454,7 @@ extern "C" int bnpp_tuning_get(const char *key, uint64_t *value)
     else if (!strcmp(key, "mv_staged")) *value = bnpp::knobs().staged;
     else if (!strcmp(key, "staged_tma")) *value = bnpp::knobs().staged_tma;
     else if (!strcmp(key, "staged_async")) *value = bnpp::knobs().staged_async;
+    else if (!strcmp(key, "chain_depth")) *value = bnpp::knobs().chain_depth;
     else return BNPP_EINVAL;
     return BNPP_OK;
 }

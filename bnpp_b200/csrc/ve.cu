@@ -27,6 +27,7 @@
 #include <vector>
 
 #include "batched.hpp"
+#include "chain.hpp"
 #include "common.cuh"
 #include "contract.hpp"
 #include "elim_order.hpp"
@@ -38,6 +39,7 @@ int contract(bnpp_ctx *ctx, int k, const bnpp_operand *ops, const bnpp_scope *ou
 int fill(bnpp_ctx *ctx, double *out, uint64_t n, double value);
 int normalize_segments(bnpp_ctx *ctx, double *buf, const uint32_t *off_dev, const uint32_t *size_dev, int n);
 int normalize_segments_batched(bnpp_ctx *ctx, double *buf, const uint32_t *off_dev, const uint32_t *size_dev, int n, uint32_t nb);
+uint32_t chain_depth_knob();
 
 struct PlanFactor {
     std::vector<uint32_t> var, card;
@@ -330,6 +332,24 @@ struct bnpp_ve_plan {
     std::vector<cudaEvent_t> ev;
     std::vector<float> step_ms;
     std::vector<std::string> step_kernel;
+    // K11 -- WINDOWS (chain.hpp): runs of wide binary eliminations, each one contract_chain launch with its
+    // intermediates in registers.  Steps [a, b) of the plan; the steps stay in the plan (the batched engines, the
+    // emulator of the tests and bnpp_ve_plan_describe see them one by one), only the single-query run fuses them.
+    struct Window {
+        int a = 0, b = 0;
+        int head = -1, out = -1;                        // PlanFactor ids
+        int side[bnpp::kChainMaxLevels][bnpp::kChainMaxSides];
+        int m = 0, add[bnpp::kChainMaxLevels] = {0, 0, 0, 0};
+        const void *fn = nullptr;
+        unsigned grid = 0;                              // resolved by the first run (occupancy)
+        bnpp::ChainParams p;                            // pointers patched per run
+        uint64_t bytes = 0, entries = 0;
+        std::string name;
+    };
+    uint32_t chain_depth = 0;               // bnpp_tuning_set("chain_depth") at plan creation; <= 1: no windows
+    std::vector<Window> windows;
+    std::vector<int> window_at;             // per step: the window that STARTS here, or -1
+    std::vector<int> launch_first;          // first step of every launch of a single run without task groups
 };
 
 using namespace bnpp;
@@ -531,18 +551,33 @@ void build_exec(bnpp_ve_plan *pl)
     pl->arena_off.assign(pl->f.size(), 0);
     std::vector<std::pair<uint64_t, uint64_t>> free_list;   // (offset, size)
     uint64_t top = 0;
+    // first fit; `avoid`: regions the block must not overlap (the head and side tables a window's launch reads while
+    // it writes its last level's output)
+    std::vector<std::pair<uint64_t, uint64_t>> avoid;                 // (offset, end)
+    auto clear_of = [&](uint64_t off, uint64_t n) {
+        for (auto &a : avoid)
+            if (off < a.second && a.first < off + n) return a.second;      // the first end to try next
+        return uint64_t(0);
+    };
     auto take = [&](uint64_t n) {
         n = (n + gran - 1) / gran * gran;
-        for (size_t i = 0; i < free_list.size(); ++i)
-            if (free_list[i].second >= n) {
-                const uint64_t off = free_list[i].first;
-                free_list[i].first += n;
-                free_list[i].second -= n;
-                if (!free_list[i].second) free_list.erase(free_list.begin() + i);
-                return off;
-            }
-        const uint64_t off = top;
-        top += n;
+        for (size_t i = 0; i < free_list.size(); ++i) {
+            const uint64_t lo = free_list[i].first, hi = lo + free_list[i].second;
+            uint64_t off = lo;
+            for (uint64_t e; off + n <= hi && (e = clear_of(off, n));) off = (e + gran - 1) / gran * gran;
+            if (off + n > hi) continue;
+            free_list.erase(free_list.begin() + i);
+            if (off + n < hi) free_list.insert(free_list.begin() + i, {off + n, hi - off - n});
+            if (lo < off) free_list.insert(free_list.begin() + i, {lo, off - lo});
+            return off;
+        }
+        uint64_t off = top;
+        for (uint64_t e; (e = clear_of(off, n));) off = (e + gran - 1) / gran * gran;
+        if (top < off) {
+            free_list.push_back({top, off - top});
+            std::sort(free_list.begin(), free_list.end());
+        }
+        top = off + n;
         return off;
     };
     auto give = [&](uint64_t off, uint64_t n) {
@@ -565,6 +600,16 @@ void build_exec(bnpp_ve_plan *pl)
     const bool leveled = pl->step_level.size() == pl->steps.size();
     for (size_t s = 0; s < pl->steps.size(); ++s) {
         const PlanStep &st = pl->steps[s];
+        avoid.clear();
+        for (const auto &w : pl->windows)
+            if ((int)s == w.b - 1) {
+                auto add = [&](int id) {
+                    if (pl->f[id].src < 0) avoid.push_back({pl->arena_off[id], pl->arena_off[id] + (pl->f[id].size + gran - 1) / gran * gran});
+                };
+                add(w.head);
+                for (int j = 0; j < w.m; ++j)
+                    for (int q = 0; q < w.p.lv[j].k; ++q) add(w.side[j][q]);
+            }
         if (st.out >= 0) pl->arena_off[st.out] = take(pl->f[st.out].size);
         pl->arena_doubles = std::max(pl->arena_doubles, top);
         for (int id : st.operands)
@@ -1302,6 +1347,276 @@ void build_segments(bnpp_ve_plan *pl)
                 std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tb2).count());
 }
 
+// ---- K11: windows (chain.hpp) ---------------------------------------------------------------------------------
+// A LINK joins step s to step t when t is the only reader of s's output, neither is the result step nor wants Z, t
+// eliminates the innermost axis of s's output, t's union has >= kChainMinUnion entries, every variable of both steps
+// is binary and every other operand of t (a SIDE) has <= kChainMaxSide entries.  A window is a chain of links
+// s0 -> t1 -> ... -> tm (2 <= m <= chain_depth) whose head -- s0's output -- holds the m eliminated variables as its
+// m fastest axes; it is cut where a level's tile would exceed kChainTile doubles, where a variable a level adds would
+// be eliminated inside the window, and where the shape has no contract_chain instantiation.  Plans with max steps
+// (MPE / MAP) form none.
+constexpr uint64_t kChainMinUnion = 1ull << 20;
+constexpr uint64_t kChainMaxSide = 1ull << 16;
+
+// stride of variable v in factor pf (0: absent); dense factors are row-major over (var, card)
+int64_t factor_stride(const PlanFactor &pf, uint32_t v)
+{
+    int64_t dense = 1;
+    for (size_t i = pf.var.size(); i-- > 0;) {
+        const int64_t st = pf.stride.empty() ? dense : pf.stride[i];
+        if (pf.var[i] == v) return st;
+        dense *= pf.card[i];
+    }
+    return 0;
+}
+
+// rest index -> offset, as bit-fields: rest bit b is variable rest[b]
+bool chain_fields(const PlanFactor &pf, const std::vector<uint32_t> &rest, Field *f, uint8_t &nf)
+{
+    nf = 0;
+    for (size_t b = 0; b < rest.size();) {
+        const int64_t st = factor_stride(pf, rest[b]);
+        if (!st) { ++b; continue; }
+        size_t len = 1;
+        while (b + len < rest.size() && factor_stride(pf, rest[b + len]) == (st << len)) ++len;
+        if (nf == kChainMaxFields || st > UINT32_MAX) return false;
+        f[nf++] = Field{(uint32_t)((1ull << len) - 1), (uint32_t)st, (uint32_t)b};
+        b += len;
+    }
+    return true;
+}
+
+// the window of head `head` over the levels `lv` (plan step indices) -> w, or false when it has no kernel
+bool chain_shape(const bnpp_ve_plan *pl, int head, const std::vector<int> &lv, bnpp_ve_plan::Window &w)
+{
+    const int m = (int)lv.size();
+    const PlanFactor &H = pl->f[head];
+    const int nh = (int)H.var.size();
+    if (m < 2 || m > kChainMaxLevels || nh < m || !H.stride.empty()) return false;
+    std::vector<uint32_t> rest;                     // rest bit b -> variable (bit 0 = the fastest rest axis)
+    for (int b = nh - m - 1; b >= 0; --b) rest.push_back(H.var[b]);
+    const uint64_t n_items = H.size >> m;
+    if (n_items % chain_chunk_items(m) || n_items > UINT32_MAX) return false;
+    w = bnpp_ve_plan::Window();
+    w.m = m;
+    w.head = head;
+    memset(&w.p, 0, sizeof w.p);
+    w.p.n_items = (uint32_t)n_items;
+    std::vector<uint32_t> added;                    // new variables, in order of addition
+    std::vector<int> sides_seen;
+    int in = head, nb = 0;
+    w.bytes = 8 * H.size;
+    for (int j = 0; j < m; ++j) {
+        const PlanStep &st = pl->steps[lv[j]];
+        if (st.elim != (int64_t)H.var[nh - 1 - j] || st.out < 0) return false;
+        // union bits: the eliminated variable, the head's later tile variables, the added ones
+        std::vector<uint32_t> ub;
+        for (int i = j; i < m; ++i) ub.push_back(H.var[nh - 1 - i]);
+        ub.insert(ub.end(), added.begin(), added.end());
+        ChainLevel &L = w.p.lv[j];
+        int hpos = -1, k = 0;
+        for (size_t q = 0; q < st.operands.size(); ++q) {
+            const int id = st.operands[q];
+            if (id == in && hpos < 0) { hpos = (int)q; continue; }
+            if (k == kChainMaxSides) return false;
+            w.side[j][k++] = id;
+        }
+        if (hpos < 0) return false;
+        // the kernel multiplies (s0 * s1) * h: a three-operand step lists its operands by size (fold_small), the head last
+        if (k == 2 && hpos != 2) return false;
+        L.k = (uint8_t)k;
+        int add = 0;
+        for (int q = 0; q < k; ++q)
+            for (uint32_t v : pl->f[w.side[j][q]].var)
+                if (std::find(ub.begin(), ub.end(), v) == ub.end() && std::find(rest.begin(), rest.end(), v) == rest.end()) {
+                    ub.push_back(v);
+                    added.push_back(v);
+                    ++add;
+                }
+        if (add > kChainMaxAdd) return false;
+        const int inb = m - j + nb, outb = inb - 1 + add;
+        if (inb > 4 || outb > 4 || (int)ub.size() != inb + add) return false;
+        w.add[j] = add;
+        nb += add;
+        for (int q = 0; q < k; ++q) {
+            const PlanFactor &S = pl->f[w.side[j][q]];
+            for (size_t b = 0; b < ub.size(); ++b) {
+                const int64_t sv = factor_stride(S, ub[b]);
+                if (sv > UINT32_MAX) return false;
+                L.s[q].us[b] = (uint32_t)sv;
+            }
+            if (!chain_fields(S, rest, L.s[q].f, L.s[q].nf)) return false;
+            if (std::find(sides_seen.begin(), sides_seen.end(), w.side[j][q]) == sides_seen.end()) {
+                sides_seen.push_back(w.side[j][q]);
+                w.bytes += 8 * S.size;
+            }
+        }
+        // the step's output must be exactly (later tile variables, rest, added): what the next level reads
+        const PlanFactor &O = pl->f[st.out];
+        if (O.var.size() != ub.size() - 1 + rest.size()) return false;
+        w.entries += st.union_entries;
+        in = st.out;
+    }
+    const PlanFactor &O = pl->f[in];
+    if (O.size > UINT32_MAX || !O.stride.empty()) return false;
+    for (size_t i = 0; i < added.size(); ++i) w.p.os[i] = (uint32_t)factor_stride(O, added[i]);
+    if (!chain_fields(O, rest, w.p.of, w.p.onf)) return false;
+    w.out = in;
+    w.bytes += 8 * O.size;
+    w.fn = chain_kernel(m, w.add);
+    if (!w.fn) return false;
+    w.name = chain_name(m, w.add);
+    return true;
+}
+
+void set_launches(bnpp_ve_plan *pl)
+{
+    const size_t ns = pl->steps.size();
+    if (pl->window_at.size() != ns) pl->window_at.assign(ns, -1);
+    pl->launch_first.clear();
+    uint64_t bytes = 0;
+    for (size_t s = 0; s < ns; ++s) {
+        pl->launch_first.push_back((int)s);
+        if (pl->window_at[s] >= 0) {
+            const auto &w = pl->windows[pl->window_at[s]];
+            bytes += w.bytes;
+            s = (size_t)w.b - 1;
+        } else {
+            bytes += pl->steps[s].bytes;
+        }
+    }
+    pl->bytes = bytes;
+}
+
+// Find the windows and move the steps that sit between a window's levels (the producers of its side tables among
+// them) ahead of its first level, so every window is a contiguous run of the step list.  Any topological order gives
+// the same numbers (operand lists are untouched), and no step between the levels reads a level's output (each has
+// one reader, the next level), so the new order is topological.  The arena is laid out again over it.
+void form_windows(bnpp_ve_plan *pl)
+{
+    if (pl->runs || pl->arena || pl->batch_runs || !pl->offtab_host.empty()) return;
+    const size_t ns = pl->steps.size();
+    pl->windows.clear();
+    pl->window_at.assign(ns, -1);
+    bool any_max = false;
+    for (const PlanStep &st : pl->steps) any_max |= st.max;
+    if (pl->is_mpe || pl->is_mar || any_max || pl->chain_depth < 2 || ns < 3) {
+        set_launches(pl);
+        return;
+    }
+    std::vector<int> producer(pl->f.size(), -1), nread(pl->f.size(), 0), reader(pl->f.size(), -1);
+    for (size_t s = 0; s < ns; ++s) {
+        const PlanStep &st = pl->steps[s];
+        if (st.out >= 0) producer[st.out] = (int)s;
+        std::vector<int> seen;
+        for (int id : st.operands)
+            if (std::find(seen.begin(), seen.end(), id) == seen.end()) {
+                seen.push_back(id);
+                nread[id]++;
+                reader[id] = (int)s;
+            }
+    }
+    auto binary = [&](const PlanStep &st) {
+        for (int id : st.operands)
+            for (uint32_t c : pl->f[id].card)
+                if (c != 2) return false;
+        return true;
+    };
+    auto link = [&](int s) {        // the step s links to, or -1
+        const PlanStep &a = pl->steps[s];
+        if (a.out < 0 || a.want_z || nread[a.out] != 1 || pl->f[a.out].var.empty()) return -1;
+        const int t = reader[a.out];
+        const PlanStep &b = pl->steps[t];
+        if (b.out < 0 || b.want_z || b.elim < 0 || b.union_entries < kChainMinUnion) return -1;
+        if (pl->f[a.out].var.back() != (uint32_t)b.elim || !binary(a) || !binary(b)) return -1;
+        for (int id : b.operands)
+            if (id != a.out && pl->f[id].size > kChainMaxSide) return -1;
+        return t;
+    };
+    std::vector<int> order(ns), pos(ns);
+    for (size_t i = 0; i < ns; ++i) order[i] = pos[i] = (int)i;
+    std::vector<std::pair<int, bnpp_ve_plan::Window>> found;     // (first level, window) by plan step index
+    for (size_t at = 0; at < ns; ++at) {
+        const int t1 = order[at];
+        int s0 = -1;
+        for (int id : pl->steps[t1].operands)
+            if (pl->f[id].src < 0 && producer[id] >= 0 && link(producer[id]) == t1) s0 = producer[id];
+        if (s0 < 0) continue;
+        std::vector<int> lv{t1};
+        while ((uint32_t)lv.size() < std::min<uint32_t>(pl->chain_depth, kChainMaxLevels)) {
+            const int t = link(lv.back());
+            if (t < 0) break;
+            lv.push_back(t);
+        }
+        bnpp_ve_plan::Window w;
+        while (lv.size() >= 2 && !chain_shape(pl, pl->steps[s0].out, lv, w)) lv.pop_back();
+        if (lv.size() < 2) continue;
+        // [at, pos(tm)]: the steps between the levels first (in their order), then the levels
+        std::vector<int> between, span(order.begin() + at, order.begin() + pos[lv.back()] + 1);
+        for (int s : span)
+            if (std::find(lv.begin(), lv.end(), s) == lv.end()) between.push_back(s);
+        size_t q = at;
+        for (int s : between) order[q++] = s;
+        for (int s : lv) order[q++] = s;
+        for (size_t i = at; i < q; ++i) pos[order[i]] = (int)i;
+        found.push_back({t1, w});
+        at = q - 1;
+    }
+    if (found.empty()) {
+        set_launches(pl);
+        return;
+    }
+    // re-order the steps (and their levels / tasks) and renumber what refers to step indices
+    std::vector<PlanStep> steps;
+    steps.reserve(ns);
+    const bool leveled = pl->step_level.size() == ns && pl->step_task.size() == ns;
+    std::vector<int> level, task;
+    for (size_t j = 0; j < ns; ++j) {
+        steps.push_back(std::move(pl->steps[order[j]]));
+        if (leveled) {
+            level.push_back(pl->step_level[order[j]]);
+            task.push_back(pl->step_task[order[j]] >= 0 ? pos[pl->step_task[order[j]]] : -1);
+        }
+    }
+    pl->steps = std::move(steps);
+    if (leveled) {
+        pl->step_level = std::move(level);
+        pl->step_task = std::move(task);
+    }
+    pl->window_at.assign(ns, -1);
+    for (auto &fw : found) {
+        bnpp_ve_plan::Window &w = fw.second;
+        w.a = pos[fw.first];
+        w.b = w.a + w.m;
+        pl->window_at[w.a] = (int)pl->windows.size();
+        pl->windows.push_back(w);
+    }
+    for (PlanFactor &pf : pl->f) pf.last_use = -1;
+    for (size_t i = 0; i < ns; ++i)
+        for (int id : pl->steps[i].operands) pl->f[id].last_use = (int)i;
+    // every factor keeps its per-step lifetime (the step-by-step engines and the emulator of the tests run them so);
+    // build_exec places a window's last output clear of the head and side tables its launch reads meanwhile
+    pl->arena_doubles = 0;
+    build_exec(pl);
+    if (leveled) {
+        pl->peak_bytes = 8 * pl->arena_doubles;         // what build_levels reports: the arena of level-wide lifetimes
+    } else {
+        // the live intermediates at their peak, as create_plan counts them, over the new order
+        uint64_t live = 0;
+        pl->peak_bytes = 0;
+        for (size_t i = 0; i < ns; ++i) {
+            const PlanStep &st = pl->steps[i];
+            if (st.out >= 0) live += 8 * pl->f[st.out].size;
+            pl->peak_bytes = std::max(pl->peak_bytes, live);
+            for (int id : st.operands)
+                if (pl->f[id].src < 0 && pl->f[id].last_use == (int)i) live -= 8 * pl->f[id].size;
+        }
+    }
+    pl->exec.clear();
+    pl->exec_planned.clear();
+    set_launches(pl);
+}
+
 // device copies of the task programs; addresses inside them (CPT tables, arena slots) patched when they moved
 int upload_tasks(bnpp_ve_plan *pl, const double *const *tables_dev)
 {
@@ -1480,6 +1795,7 @@ static int create_plan(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_
     pl->obs_card.assign(n_obs, 0);
     pl->fused_mode = fused_default_on() ? 1 : 0;
     pl->segments_mode = segments_default_mode();
+    pl->chain_depth = mpe_card ? 0u : chain_depth_knob();
 
     std::map<uint32_t, int> obs_index;
     for (int i = 0; i < n_obs; ++i) obs_index[obs_var[i]] = i;
@@ -1565,6 +1881,7 @@ static int create_plan(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_
         }
     }
     if (pl->segments_mode) build_levels(pl);
+    form_windows(pl);
     if (getenv("BNPP_TIMING")) {
         auto ms = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
             return std::chrono::duration<double, std::milli>(b - a).count();
@@ -1878,7 +2195,7 @@ int bnpp_ve_plan_info(const bnpp_ve_plan *pl, int32_t *result_rank, uint32_t *re
         if (result_var) result_var[i] = pl->result_var[i];
         if (result_card) result_card[i] = pl->result_card[i];
     }
-    if (n_launches) *n_launches = pl->steps.size();
+    if (n_launches) *n_launches = pl->windows.empty() ? pl->steps.size() : pl->launch_first.size();     // a window is one launch
     if (union_entries) *union_entries = pl->union_entries;
     if (algorithmic_bytes) *algorithmic_bytes = pl->bytes;
     if (peak_bytes) *peak_bytes = pl->peak_bytes;
@@ -2012,6 +2329,7 @@ int bnpp_ve_plan_set_segments(bnpp_ve_plan *pl, int on, uint32_t max_steps)
     if (on && (!pl->levels_built || max_steps != pl->segments_max_steps)) {
         pl->segments_max_steps = max_steps;
         build_levels(pl);       // re-orders the steps; refused (the plan keeps its tasks) once the plan has run
+        form_windows(pl);
     }
     return BNPP_OK;
 }
@@ -2060,9 +2378,21 @@ int bnpp_ve_plan_launches(bnpp_ve_plan *pl, uint64_t *launches, uint32_t *groups
     if (!pl->segments_built) build_segments(pl);
     uint64_t covered = 0;
     for (const auto &g : pl->groups) covered += (uint64_t)(g.b - g.a);
+    for (const auto &w : pl->windows) covered += (uint64_t)(w.b - w.a - 1);
     if (launches) *launches = pl->steps.size() - covered + pl->groups.size();
     if (groups) *groups = (uint32_t)pl->groups.size();
-    if (levels) *levels = pl->step_level.empty() ? 0u : (uint32_t)(pl->step_level.back() + 1);
+    if (levels) *levels = pl->step_level.empty() ? 0u : (uint32_t)(*std::max_element(pl->step_level.begin(), pl->step_level.end()) + 1);
+    return BNPP_OK;
+}
+
+int bnpp_ve_plan_windows(const bnpp_ve_plan *pl, uint32_t cap, uint32_t *n, uint32_t *first_step, uint32_t *n_steps)
+{
+    if (!pl || !n) return BNPP_EINVAL;
+    *n = (uint32_t)pl->windows.size();
+    for (uint32_t i = 0; i < *n && i < cap; ++i) {
+        if (first_step) first_step[i] = (uint32_t)pl->windows[i].a;
+        if (n_steps) n_steps[i] = (uint32_t)(pl->windows[i].b - pl->windows[i].a);
+    }
     return BNPP_OK;
 }
 
@@ -2095,17 +2425,27 @@ int bnpp_ve_plan_fused_program(bnpp_ve_plan *pl, uint32_t nb, uint32_t *prog, ui
 int bnpp_ve_plan_step_stats(bnpp_ve_plan *pl, uint64_t n, float *ms, uint64_t *bytes, uint64_t *entries, int32_t *k)
 {
     if (!pl) return BNPP_EINVAL;
+    // one row per launch of a single run: a window is one row (its bytes: head + sides + output; its entries: the
+    // union entries of its steps)
+    const size_t ns = pl->steps.size();
+    const bool win = !pl->windows.empty() && pl->window_at.size() == ns;
+    auto launch_end = [&](size_t s) -> size_t { return win && pl->window_at[s] >= 0 ? (size_t)pl->windows[pl->window_at[s]].b : s + 1; };
     if (pl->profiling && !pl->ev.empty()) {
-        BNPP_CUDA(pl->ctx, cudaEventSynchronize(pl->ev[pl->steps.size()]));
-        pl->step_ms.resize(pl->steps.size());
-        for (size_t s = 0; s < pl->steps.size(); ++s)
-            BNPP_CUDA(pl->ctx, cudaEventElapsedTime(&pl->step_ms[s], pl->ev[s], pl->ev[s + 1]));
+        BNPP_CUDA(pl->ctx, cudaEventSynchronize(pl->ev[ns]));
+        pl->step_ms.clear();
+        for (size_t s = 0; s < ns; s = launch_end(s)) {
+            float t = 0.0f;
+            BNPP_CUDA(pl->ctx, cudaEventElapsedTime(&t, pl->ev[s], pl->ev[launch_end(s)]));
+            pl->step_ms.push_back(t);
+        }
     }
-    for (size_t s = 0; s < pl->steps.size() && s < n; ++s) {
-        if (ms) ms[s] = s < pl->step_ms.size() ? pl->step_ms[s] : 0.0f;
-        if (bytes) bytes[s] = pl->steps[s].bytes;
-        if (entries) entries[s] = pl->steps[s].union_entries;
-        if (k) k[s] = (int32_t)pl->steps[s].operands.size();
+    size_t row = 0;
+    for (size_t s = 0; s < ns && row < n; s = launch_end(s), ++row) {
+        const bool w = win && pl->window_at[s] >= 0;
+        if (ms) ms[row] = row < pl->step_ms.size() ? pl->step_ms[row] : 0.0f;
+        if (bytes) bytes[row] = w ? pl->windows[pl->window_at[s]].bytes : pl->steps[s].bytes;
+        if (entries) entries[row] = w ? pl->windows[pl->window_at[s]].entries : pl->steps[s].union_entries;
+        if (k) k[row] = (int32_t)pl->steps[s].operands.size();
     }
     return BNPP_OK;
 }
@@ -2113,6 +2453,7 @@ int bnpp_ve_plan_step_stats(bnpp_ve_plan *pl, uint64_t n, float *ms, uint64_t *b
 int bnpp_ve_plan_step_kernel(const bnpp_ve_plan *pl, uint64_t step, char *name, size_t name_len)
 {
     if (!pl || !name || !name_len) return BNPP_EINVAL;
+    if (!pl->windows.empty()) step = step < pl->launch_first.size() ? (uint64_t)pl->launch_first[step] : UINT64_MAX;   // row = launch
     const std::string s = step < pl->step_kernel.size() ? pl->step_kernel[step] : std::string();
     strncpy(name, s.c_str(), name_len - 1);
     name[name_len - 1] = 0;
@@ -2383,6 +2724,50 @@ static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uin
                 s = (size_t)g.b - 1;
                 continue;
             }
+            if (!pl->windows.empty() && pl->window_at[s] >= 0) {
+                // K11: a window of binary eliminations, one contract_chain launch
+                bnpp_ve_plan::Window &w = pl->windows[pl->window_at[s]];
+                if (pl->profiling) cudaEventRecord(pl->ev[s], ctx->stream);
+                if (!w.grid) {
+                    const int occ = chain_occupancy(w.fn);
+                    if (occ <= 0) return fail(ctx, BNPP_ECUDA, "contract_chain: no occupancy");
+                    const uint64_t chunks = w.p.n_items / (uint64_t)chain_chunk_items(w.m);
+                    w.grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>(chunks, (uint64_t)occ * ctx->sm_count));
+                }
+                ChainParams now = w.p;
+                now.head = ptr[w.head];
+                now.out = pl->arena + pl->arena_off[w.out];
+                for (int j = 0; j < w.m; ++j)
+                    for (int q = 0; q < now.lv[j].k; ++q) now.lv[j].s[q].p = ptr[w.side[j][q]];
+                bool moved = fresh || now.head != w.p.head || now.out != w.p.out;
+                for (int j = 0; j < w.m; ++j)
+                    for (int q = 0; q < now.lv[j].k; ++q) moved = moved || now.lv[j].s[q].p != w.p.lv[j].s[q].p;
+                w.p = now;
+                ++n_launched;
+                void *args[1] = {&w.p};
+                if (!(graphed && pl->use_graph)) {
+                    BNPP_CUDA(ctx, cudaLaunchKernel(w.fn, dim3(w.grid), dim3(kBlock), args, 0, ctx->stream));
+                    ctx->launches++;
+                    ctx->last_desc = nullptr;
+                    ctx->last_kernel = w.name;
+                    ctx->last_grid = w.grid;
+                    ctx->last_block = kBlock;
+                } else if (moved) {
+                    cudaKernelNodeParams kp;
+                    memset(&kp, 0, sizeof kp);
+                    kp.func = const_cast<void *>(w.fn);
+                    kp.gridDim = dim3(w.grid);
+                    kp.blockDim = dim3(kBlock);
+                    kp.kernelParams = args;
+                    cudaError_t e;
+                    if (fresh) e = cudaGraphAddKernelNode(&pl->nodes[s], pl->graph, prev ? &prev : nullptr, prev ? 1 : 0, &kp);
+                    else e = cudaGraphExecKernelNodeSetParams(pl->graph_exec, pl->nodes[s], &kp);
+                    if (e != cudaSuccess) return cuda_fail(ctx, e, "CUDA graph node (contract_chain)");
+                }
+                if (fresh) prev = pl->nodes[s];
+                s = (size_t)w.b - 1;
+                continue;
+            }
             const PlanStep &st = pl->steps[s];
             if (pl->profiling) cudaEventRecord(pl->ev[s], ctx->stream);
             const double *in[kMaxK];
@@ -2456,6 +2841,7 @@ static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uin
         if (pl->profiling) {
             pl->step_kernel.resize(pl->steps.size());
             for (size_t s = 0; s < pl->steps.size(); ++s) pl->step_kernel[s] = pl->exec[s] ? pl->exec[s]->name() : std::string();
+            for (const auto &w : pl->windows) pl->step_kernel[w.a] = w.name;
         }
     }
     if (rc == BNPP_OK && pl->is_mar && pl->normalize)

@@ -89,7 +89,10 @@ int bnpp_last_launch(const bnpp_ctx *ctx, char *name, size_t name_len, uint32_t 
  *                      of its contiguous runs (contract_staged_bulk); 0 = element-wise cp.async (contract_staged)
  *   "staged_async"   : 1 (default) = in that kernel the other operands are prefetched too (cp.async, a ring of stages)
  *                      when their micro-tiles are at most two values; 0 = loaded into registers chunk by chunk
- * Unknown keys return BNPP_EINVAL.  Environment BNPP_MV_MIN_ENTRIES / BNPP_MV_EMAX / BNPP_STAGED_TMA / BNPP_STAGED_ASYNC seed the defaults. */
+ *   "chain_depth"    : levels of a window of a VE plan (runs of wide binary eliminations as one contract_chain launch,
+ *                      intermediates in registers), read when a plan is created; default 4; 0 or 1 = no windows
+ * Unknown keys return BNPP_EINVAL.  Environment BNPP_MV_MIN_ENTRIES / BNPP_MV_EMAX / BNPP_STAGED_TMA / BNPP_STAGED_ASYNC /
+ * BNPP_CHAIN_DEPTH seed the defaults. */
 int bnpp_tuning_set(const char *key, uint64_t value);
 int bnpp_tuning_get(const char *key, uint64_t *value);
 
@@ -347,6 +350,8 @@ int bnpp_ve_plan_set_segments(bnpp_ve_plan *plan, int on, uint32_t max_steps);
 int bnpp_ve_plan_segments(bnpp_ve_plan *plan, uint32_t cap, uint32_t *n, uint32_t *first_step, uint32_t *end_step,
                           int32_t *lanes, uint32_t *arena_doubles);
 int bnpp_ve_plan_launches(bnpp_ve_plan *plan, uint64_t *launches, uint32_t *groups, uint32_t *levels);
+/* windows of a VE plan (one contract_chain launch each): the first step and the number of steps of each */
+int bnpp_ve_plan_windows(const bnpp_ve_plan *plan, uint32_t cap, uint32_t *n, uint32_t *first_step, uint32_t *n_steps);
 int bnpp_ve_plan_segment_program(bnpp_ve_plan *plan, uint32_t segment, uint32_t *prog, uint64_t prog_cap, uint64_t *prog_words,
                                  uint32_t *offtab, uint64_t tab_cap, uint64_t *tab_words);
 /* per-launch CUDA-event timing for roofline reports: enable, run, then read
