@@ -52,6 +52,8 @@ struct ChainParams {
 
 // the kernel for m levels adding add[j] variables at level j; nullptr when the shape has no instantiation
 const void *chain_kernel(int m, const int *add);
+// one launch of a window's kernel `fn` on the context's stream; bnpp_last_launch reports it as `name`
+int chain_launch(bnpp_ctx *ctx, const void *fn, unsigned grid, const ChainParams &p, const std::string &name);
 // blocks per SM the kernel reaches with kBlock threads (0 on error)
 int chain_occupancy(const void *fn);
 std::string chain_name(int m, const int *add);

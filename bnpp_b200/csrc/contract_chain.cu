@@ -197,6 +197,18 @@ const void *chain_kernel(int m, const int *add)
     return chain_table(code, std::make_integer_sequence<int, kChainCodes>());
 }
 
+int chain_launch(bnpp_ctx *ctx, const void *fn, unsigned grid, const ChainParams &p, const std::string &name)
+{
+    void *args[1] = {const_cast<ChainParams *>(&p)};
+    BNPP_CUDA(ctx, cudaLaunchKernel(fn, dim3(grid), dim3(kBlock), args, 0, ctx->stream));
+    ctx->launches++;
+    ctx->last_desc = nullptr;
+    ctx->last_kernel = name;
+    ctx->last_grid = grid;
+    ctx->last_block = kBlock;
+    return BNPP_OK;
+}
+
 int chain_occupancy(const void *fn)
 {
     int n = 0;

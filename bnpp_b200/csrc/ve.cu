@@ -356,6 +356,23 @@ using namespace bnpp;
 
 namespace {
 
+// device buffer of `count` elements of T, rounded up to whole doubles; *out is set only on success
+template <class T>
+int dev_alloc(bnpp_ctx *ctx, size_t count, T **out)
+{
+    double *store = nullptr;
+    const int rc = bnpp_alloc(ctx, (count * sizeof(T) + sizeof(double) - 1) / sizeof(double), &store);
+    if (rc == BNPP_OK) *out = static_cast<T *>(static_cast<void *>(store));
+    return rc;
+}
+
+template <class T>
+void dev_free(bnpp_ctx *ctx, T *&p)
+{
+    if (p) bnpp_free(ctx, static_cast<double *>(static_cast<void *>(p)));
+    p = nullptr;
+}
+
 uint64_t table_size(const std::vector<uint32_t> &card)
 {
     uint64_t n = 1;
@@ -627,6 +644,20 @@ void build_exec(bnpp_ve_plan *pl)
     // (the descriptors themselves -- 4 KB each -- are allocated by the first launch-per-bucket run: a plan that
     // runs fused never needs them)
     pl->exec_ok = true;
+}
+
+// bytes of the live intermediates at their peak over the step order (an intermediate lives from its step to its last reader)
+uint64_t live_peak(const bnpp_ve_plan *pl)
+{
+    uint64_t live = 0, peak = 0;
+    for (size_t s = 0; s < pl->steps.size(); ++s) {
+        const PlanStep &st = pl->steps[s];
+        if (st.out >= 0) live += 8 * pl->f[st.out].size;
+        peak = std::max(peak, live);
+        for (int id : st.operands)
+            if (pl->f[id].src < 0 && pl->f[id].last_use == (int)s) live -= 8 * pl->f[id].size;
+    }
+    return peak;
 }
 
 // resolve the launch of step s against stand-in pointers that carry only the guaranteed alignment
@@ -1134,11 +1165,9 @@ bool step_is_small(const PlanStep &st)
 
 void free_tasks(bnpp_ve_plan *pl)
 {
-    if (pl->tasks_prog_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->tasks_prog_dev));
-    if (pl->tasks_tab_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->tasks_tab_dev));
-    if (pl->tasks_rec_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->tasks_rec_dev));
-    pl->tasks_prog_dev = pl->tasks_tab_dev = nullptr;
-    pl->tasks_rec_dev = nullptr;
+    dev_free(pl->ctx, pl->tasks_prog_dev);
+    dev_free(pl->ctx, pl->tasks_tab_dev);
+    dev_free(pl->ctx, pl->tasks_rec_dev);
     pl->tasks_uploaded = false;
     pl->tasks_prog.clear();
     pl->tasks_tab_words = 0;
@@ -1148,6 +1177,45 @@ void free_tasks(bnpp_ve_plan *pl)
     pl->groups.clear();
     pl->group_at.clear();
     pl->segments_built = false;
+}
+
+// Puts step order[j] at position j, with its level and task (a task root renumbered to its new position) when the plan
+// is levelled.  Any topological order gives the same numbers: operand lists are untouched.  The arena is laid out
+// again over the new order (around the plan's windows as they stand); the launches resolved for the old order and
+// the K9 program are dropped.
+void reorder_steps(bnpp_ve_plan *pl, const std::vector<int> &order)
+{
+    const size_t ns = pl->steps.size();
+    const bool leveled = pl->step_level.size() == ns && pl->step_task.size() == ns;
+    std::vector<int> pos(ns);
+    for (size_t j = 0; j < ns; ++j) pos[order[j]] = (int)j;
+    std::vector<PlanStep> steps;
+    steps.reserve(ns);
+    std::vector<int> level, task;
+    for (size_t j = 0; j < ns; ++j) {
+        steps.push_back(std::move(pl->steps[order[j]]));
+        if (leveled) {
+            level.push_back(pl->step_level[order[j]]);
+            task.push_back(pl->step_task[order[j]] >= 0 ? pos[pl->step_task[order[j]]] : -1);
+        }
+    }
+    pl->steps = std::move(steps);
+    if (leveled) {
+        pl->step_level = std::move(level);
+        pl->step_task = std::move(task);
+    }
+    for (PlanFactor &pf : pl->f) pf.last_use = -1;
+    for (size_t i = 0; i < ns; ++i)
+        for (int id : pl->steps[i].operands) pl->f[id].last_use = (int)i;
+    pl->arena_doubles = 0;
+    build_exec(pl);
+    // a levelled plan reports its arena (level-wide lifetimes), any other the live intermediates, as create_plan does
+    pl->peak_bytes = leveled ? 8 * pl->arena_doubles : live_peak(pl);
+    pl->exec.clear();
+    pl->exec_planned.clear();
+    dev_free(pl->ctx, pl->fused.prog_dev);
+    dev_free(pl->ctx, pl->fused.offtab_dev);
+    pl->fused = FusedProgram();
 }
 
 // Tasks and levels.  The steps of a plan form a DAG (a tree for PR plans).  A small step absorbs the tasks of its
@@ -1222,39 +1290,17 @@ void build_levels(bnpp_ve_plan *pl)
         root[i] = parent[i] >= 0 ? root[parent[i]] : (int)i;
         if (parent[i] >= 0) level[i] = level[root[i]];
     }
-    std::vector<size_t> order(ns);
-    for (size_t i = 0; i < ns; ++i) order[i] = i;
-    std::stable_sort(order.begin(), order.end(), [&](size_t x, size_t y) {
+    std::vector<int> order(ns);
+    for (size_t i = 0; i < ns; ++i) order[i] = (int)i;
+    std::stable_sort(order.begin(), order.end(), [&](int x, int y) {
         if (level[x] != level[y]) return level[x] < level[y];
         if (small[x] != small[y]) return small[x] > small[y];         // the level's tasks first, then its wide steps
         if (small[x] && root[x] != root[y]) return root[x] < root[y];
         return x < y;
     });
-    std::vector<PlanStep> steps;
-    steps.reserve(ns);
-    std::vector<int> new_index(ns, -1);
-    pl->step_level.assign(ns, 0);
-    pl->step_task.assign(ns, -1);
-    for (size_t j = 0; j < ns; ++j) {
-        new_index[order[j]] = (int)j;
-        pl->step_level[j] = level[order[j]];
-    }
-    for (size_t j = 0; j < ns; ++j) {
-        pl->step_task[j] = small[order[j]] ? new_index[root[order[j]]] : -1;
-        steps.push_back(std::move(pl->steps[order[j]]));
-    }
-    pl->steps = std::move(steps);
-    for (PlanFactor &pf : pl->f) pf.last_use = -1;
-    for (size_t i = 0; i < ns; ++i)
-        for (int id : pl->steps[i].operands) pl->f[id].last_use = (int)i;
-    pl->arena_doubles = 0;
-    build_exec(pl);
-    pl->peak_bytes = 8 * pl->arena_doubles;
-    pl->exec.clear();
-    pl->exec_planned.clear();
-    if (pl->fused.prog_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->fused.prog_dev));
-    if (pl->fused.offtab_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->fused.offtab_dev));
-    pl->fused = FusedProgram();
+    pl->step_level = level;
+    pl->step_task = root;       // -1 for wide steps
+    reorder_steps(pl, order);
 }
 
 // the step program of every task, the groups (one ve_tasks launch each), and all programs in one buffer
@@ -1566,23 +1612,9 @@ void form_windows(bnpp_ve_plan *pl)
         set_launches(pl);
         return;
     }
-    // re-order the steps (and their levels / tasks) and renumber what refers to step indices
-    std::vector<PlanStep> steps;
-    steps.reserve(ns);
-    const bool leveled = pl->step_level.size() == ns && pl->step_task.size() == ns;
-    std::vector<int> level, task;
-    for (size_t j = 0; j < ns; ++j) {
-        steps.push_back(std::move(pl->steps[order[j]]));
-        if (leveled) {
-            level.push_back(pl->step_level[order[j]]);
-            task.push_back(pl->step_task[order[j]] >= 0 ? pos[pl->step_task[order[j]]] : -1);
-        }
-    }
-    pl->steps = std::move(steps);
-    if (leveled) {
-        pl->step_level = std::move(level);
-        pl->step_task = std::move(task);
-    }
+    // the windows in the new step order first: the arena is laid out around them.  Every factor keeps its per-step
+    // lifetime (the step-by-step engines and the emulator of the tests run them so); build_exec places a window's last
+    // output clear of the head and side tables its launch reads meanwhile
     pl->window_at.assign(ns, -1);
     for (auto &fw : found) {
         bnpp_ve_plan::Window &w = fw.second;
@@ -1591,29 +1623,7 @@ void form_windows(bnpp_ve_plan *pl)
         pl->window_at[w.a] = (int)pl->windows.size();
         pl->windows.push_back(w);
     }
-    for (PlanFactor &pf : pl->f) pf.last_use = -1;
-    for (size_t i = 0; i < ns; ++i)
-        for (int id : pl->steps[i].operands) pl->f[id].last_use = (int)i;
-    // every factor keeps its per-step lifetime (the step-by-step engines and the emulator of the tests run them so);
-    // build_exec places a window's last output clear of the head and side tables its launch reads meanwhile
-    pl->arena_doubles = 0;
-    build_exec(pl);
-    if (leveled) {
-        pl->peak_bytes = 8 * pl->arena_doubles;         // what build_levels reports: the arena of level-wide lifetimes
-    } else {
-        // the live intermediates at their peak, as create_plan counts them, over the new order
-        uint64_t live = 0;
-        pl->peak_bytes = 0;
-        for (size_t i = 0; i < ns; ++i) {
-            const PlanStep &st = pl->steps[i];
-            if (st.out >= 0) live += 8 * pl->f[st.out].size;
-            pl->peak_bytes = std::max(pl->peak_bytes, live);
-            for (int id : st.operands)
-                if (pl->f[id].src < 0 && pl->f[id].last_use == (int)i) live -= 8 * pl->f[id].size;
-        }
-    }
-    pl->exec.clear();
-    pl->exec_planned.clear();
+    reorder_steps(pl, order);
     set_launches(pl);
 }
 
@@ -1634,14 +1644,11 @@ int upload_tasks(bnpp_ve_plan *pl, const double *const *tables_dev)
         }
     }
     if (!pl->tasks_prog_dev) {
-        double *p0 = nullptr, *p1 = nullptr, *p2 = nullptr;
-        int rc = bnpp_alloc(ctx, pl->tasks_prog.size() / 2 + 18, &p0);      // the kernel prefetches 32 words past a record
-        if (rc == BNPP_OK) rc = bnpp_alloc(ctx, pl->tasks_tab_words / 2 + 2, &p1);
-        if (rc == BNPP_OK) rc = bnpp_alloc(ctx, pl->tasks_rec.size() * 2 + 2, &p2);
+        // the program last: it marks the three as allocated
+        int rc = dev_alloc(ctx, pl->tasks_tab_words + 4, &pl->tasks_tab_dev);
+        if (rc == BNPP_OK) rc = dev_alloc(ctx, pl->tasks_rec.size() + 1, &pl->tasks_rec_dev);
+        if (rc == BNPP_OK) rc = dev_alloc(ctx, pl->tasks_prog.size() + 36, &pl->tasks_prog_dev);  // the kernel prefetches 32 words past a record
         if (rc != BNPP_OK) return rc;
-        pl->tasks_prog_dev = reinterpret_cast<uint32_t *>(p0);
-        pl->tasks_tab_dev = reinterpret_cast<uint32_t *>(p1);
-        pl->tasks_rec_dev = reinterpret_cast<TaskRecord *>(p2);
         // the tables are gathered straight into the pinned ring (one copy to the device); too large for it: task by task
         if (uint32_t *stage = static_cast<uint32_t *>(stage_reserve(ctx, pl->tasks_tab_words * sizeof(uint32_t)))) {
             for (size_t i = 0; i < pl->segs.size(); ++i)
@@ -1705,19 +1712,15 @@ int run_fused(bnpp_ve_plan *pl, FusedProgram &fp, int G, const double *const *ta
             fp.slot_addr[i] = a;
         }
         if (!fp.prog_dev) {
-            double *store = nullptr;
-            const int rc = bnpp_alloc(ctx, fp.prog.size() / 2 + 18, &store);      // the kernel prefetches 32 words past a record
+            const int rc = dev_alloc(ctx, fp.prog.size() + 36, &fp.prog_dev);      // the kernel prefetches 32 words past a record
             if (rc != BNPP_OK) return rc;
-            fp.prog_dev = reinterpret_cast<uint32_t *>(store);
         }
         // stream-ordered after any launch still reading the previous contents; the pageable source is staged before the call returns
         BNPP_CUDA(ctx, cudaMemcpyAsync(fp.prog_dev, fp.prog.data(), fp.prog.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
     }
     if (!fp.offtab_uploaded) {
-        double *store = nullptr;
-        const int rc = bnpp_alloc(ctx, fp.offtab.size() / 2 + 2, &store);
+        const int rc = dev_alloc(ctx, fp.offtab.size() + 4, &fp.offtab_dev);
         if (rc != BNPP_OK) return rc;
-        fp.offtab_dev = reinterpret_cast<uint32_t *>(store);
         if (!fp.offtab.empty())
             BNPP_CUDA(ctx, cudaMemcpyAsync(fp.offtab_dev, fp.offtab.data(), fp.offtab.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
         fp.offtab_uploaded = true;
@@ -1780,6 +1783,36 @@ extern "C" {
 
 static int mpe_finish(bnpp_ve_plan *pl, int nvars, int n_obs, const uint32_t *obs_var, const std::vector<char> *is_map);
 
+// What every plan starts with: the plan, the elimination time of every ordered variable in `rank`, and the input tables
+// as evidence-reduced views; no plan when the order or a scope is bad.
+static int plan_prelude(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_obs, const uint32_t *obs_var, int n_order,
+                        const uint32_t *order, bnpp_ve_plan *&plan, RankMap &rank)
+{
+    plan = nullptr;
+    bnpp_ve_plan *pl = new bnpp_ve_plan();
+    pl->ctx = ctx;
+    pl->n_inputs = nfac;
+    pl->n_obs = n_obs;
+    pl->obs_card.assign(n_obs, 0);
+    pl->fused_mode = fused_default_on() ? 1 : 0;
+    pl->segments_mode = segments_default_mode();
+    std::map<uint32_t, int> obs_index;
+    for (int i = 0; i < n_obs; ++i) obs_index[obs_var[i]] = i;
+    for (int i = 0; i < n_order; ++i) {
+        if (rank.count(order[i]) || obs_index.count(order[i])) {
+            delete pl;
+            return fail(ctx, BNPP_EINVAL, "elimination order repeats a variable or names an observed one");
+        }
+        rank.set(order[i], (uint64_t)i);
+    }
+    if (int rc = add_inputs(pl, nfac, scopes, obs_index, rank)) {
+        delete pl;
+        return fail(ctx, rc, "bad factor scope");
+    }
+    plan = pl;
+    return BNPP_OK;
+}
+
 // the bucket schedule of bnpp_ve_plan_create; mpe_card != NULL: an MPE plan over that many variables (bnpp_mpe_plan_create),
 // or with is_map (per variable id, 1 = a MAP variable) a MAP plan (bnpp_map_plan_create)
 static int create_plan(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_obs, const uint32_t *obs_var, int n_order,
@@ -1788,31 +1821,11 @@ static int create_plan(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_
 {
     if (!out || nfac < 0 || n_obs < 0 || n_order < 0) return BNPP_EINVAL;   // ctx == NULL: a dry plan (inspect, never run)
     *out = nullptr;
-    bnpp_ve_plan *pl = new bnpp_ve_plan();
-    pl->ctx = ctx;
-    pl->n_inputs = nfac;
-    pl->n_obs = n_obs;
-    pl->obs_card.assign(n_obs, 0);
-    pl->fused_mode = fused_default_on() ? 1 : 0;
-    pl->segments_mode = segments_default_mode();
-    pl->chain_depth = mpe_card ? 0u : chain_depth_knob();
-
-    std::map<uint32_t, int> obs_index;
-    for (int i = 0; i < n_obs; ++i) obs_index[obs_var[i]] = i;
-    RankMap rank;           // elimination time; kept variables after all eliminated ones
-    for (int i = 0; i < n_order; ++i) {
-        if (rank.count(order[i]) || obs_index.count(order[i])) {
-            delete pl;
-            return fail(ctx, BNPP_EINVAL, "elimination order repeats a variable or names an observed one");
-        }
-        rank.set(order[i], (uint64_t)i);
-    }
-
     const auto tc0 = std::chrono::steady_clock::now();
-    if (int rc = add_inputs(pl, nfac, scopes, obs_index, rank)) {
-        delete pl;
-        return fail(ctx, rc, "bad factor scope");
-    }
+    bnpp_ve_plan *pl;
+    RankMap rank;           // elimination time; kept variables after all eliminated ones
+    if (int rc = plan_prelude(ctx, nfac, scopes, n_obs, obs_var, n_order, order, pl, rank)) return rc;
+    pl->chain_depth = mpe_card ? 0u : chain_depth_knob();
     if (mpe_card) {
         // MPE eliminates every unobserved variable; its argmax tables are uint8 (MAP: those of the MAP variables)
         for (const PlanFactor &pf : pl->f)
@@ -1862,15 +1875,8 @@ static int create_plan(bnpp_ctx *ctx, int nfac, const bnpp_scope *scopes, int n_
     }
 
     // statistics: bytes, and the peak of live intermediates
-    uint64_t live = 0;
-    for (size_t s = 0; s < pl->steps.size(); ++s) {
-        const PlanStep &st = pl->steps[s];
-        pl->bytes += st.bytes;
-        if (st.out >= 0) live += 8 * pl->f[st.out].size;
-        pl->peak_bytes = std::max(pl->peak_bytes, live);
-        for (int id : st.operands)
-            if (pl->f[id].src < 0 && pl->f[id].last_use == (int)s) live -= 8 * pl->f[id].size;
-    }
+    for (const PlanStep &st : pl->steps) pl->bytes += st.bytes;
+    pl->peak_bytes = live_peak(pl);
     const auto tc2 = std::chrono::steady_clock::now();
     build_exec(pl);
     const auto tc3 = std::chrono::steady_clock::now();
@@ -2018,28 +2024,10 @@ int bnpp_mar_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfa
 {
     if (!out || nvars < 0 || nfac < 0 || n_obs < 0 || n_order < 0) return BNPP_EINVAL;   // ctx == NULL: a dry plan
     *out = nullptr;
-    bnpp_ve_plan *pl = new bnpp_ve_plan();
-    pl->ctx = ctx;
-    pl->n_inputs = nfac;
-    pl->n_obs = n_obs;
-    pl->obs_card.assign(n_obs, 0);
-    pl->fused_mode = fused_default_on() ? 1 : 0;
-    pl->segments_mode = segments_default_mode();
-    pl->is_mar = true;
-    std::map<uint32_t, int> obs_index;
-    for (int i = 0; i < n_obs; ++i) obs_index[obs_var[i]] = i;
+    bnpp_ve_plan *pl;
     RankMap rank;
-    for (int i = 0; i < n_order; ++i) {
-        if (rank.count(order[i]) || obs_index.count(order[i])) {
-            delete pl;
-            return fail(ctx, BNPP_EINVAL, "elimination order repeats a variable or names an observed one");
-        }
-        rank.set(order[i], (uint64_t)i);
-    }
-    if (int rc = add_inputs(pl, nfac, scopes, obs_index, rank)) {
-        delete pl;
-        return fail(ctx, rc, "bad factor scope");
-    }
+    if (int rc = plan_prelude(ctx, nfac, scopes, n_obs, obs_var, n_order, order, pl, rank)) return rc;
+    pl->is_mar = true;
     for (const PlanFactor &pf : pl->f)
         for (uint32_t v : pf.var)
             if (rank.at(v) >= (uint64_t)n_order) {
@@ -2108,28 +2096,18 @@ int bnpp_mar_plan_create(bnpp_ctx *ctx, int nvars, const uint32_t *card, int nfa
     pl->result_card.clear();
     pl->result_size = total;
 
-    uint64_t live = 0;
-    for (size_t s = 0; s < pl->steps.size(); ++s) {
-        const PlanStep &st = pl->steps[s];
-        pl->bytes += st.bytes;
-        if (st.out >= 0) live += 8 * pl->f[st.out].size;
-        pl->peak_bytes = std::max(pl->peak_bytes, live);
-        for (int id : st.operands)
-            if (pl->f[id].src < 0 && pl->f[id].last_use == (int)s) live -= 8 * pl->f[id].size;
-    }
+    for (const PlanStep &st : pl->steps) pl->bytes += st.bytes;
+    pl->peak_bytes = live_peak(pl);
     build_exec(pl);
     if (pl->segments_mode) build_levels(pl);
     if (!ctx) {
         *out = pl;
         return BNPP_OK;
     }
-    double *store = nullptr;
-    int rc = bnpp_alloc(ctx, (uint64_t)nvars + 2, &store);   // 2 * nvars uint32
-    if (rc != BNPP_OK) {
+    if (int rc = dev_alloc(ctx, 2 * (size_t)nvars + 4, &pl->mar_off_dev)) {     // the offsets, then the sizes
         delete pl;
         return rc;
     }
-    pl->mar_off_dev = reinterpret_cast<uint32_t *>(store);
     pl->mar_size_dev = pl->mar_off_dev + nvars;
     if (nvars) {
         cudaMemcpyAsync(pl->mar_off_dev, pl->mar_off.data(), sizeof(uint32_t) * nvars, cudaMemcpyHostToDevice, ctx->stream);
@@ -2162,25 +2140,24 @@ int bnpp_ve_plan_destroy(bnpp_ve_plan *pl)
     }
     if (pl->graph_exec) cudaGraphExecDestroy(pl->graph_exec);
     if (pl->graph) cudaGraphDestroy(pl->graph);
-    if (pl->arena) bnpp_free(pl->ctx, pl->arena);
-    if (pl->arg_arena) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->arg_arena));
-    if (pl->decode_rec_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->decode_rec_dev));
-    if (pl->obs_val_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->obs_val_dev));
-    if (pl->batch_rec_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->batch_rec_dev));
-    if (pl->batch_arg) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->batch_arg));
+    dev_free(pl->ctx, pl->arena);
+    dev_free(pl->ctx, pl->arg_arena);
+    dev_free(pl->ctx, pl->decode_rec_dev);
+    dev_free(pl->ctx, pl->obs_val_dev);
+    dev_free(pl->ctx, pl->batch_rec_dev);
+    dev_free(pl->ctx, pl->batch_arg);
     for (auto &d : pl->exec)
         if (d) {
             contract_release(pl->ctx, *d);
             if (pl->ctx && pl->ctx->last_desc == d.get()) pl->ctx->last_desc = nullptr;      // bnpp_last_launch must not follow a pointer into a dead plan
         }
     free_tasks(pl);
-    if (pl->fused.prog_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->fused.prog_dev));
-    if (pl->fused.offtab_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->fused.offtab_dev));
-    if (pl->mar_off_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->mar_off_dev));
-    if (pl->obs_card_dev) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->obs_card_dev));
-    if (pl->ev_clean) bnpp_free(pl->ctx, reinterpret_cast<double *>(pl->ev_clean));
-    for (uint32_t *t : pl->offtab_dev)
-        if (t) bnpp_free(pl->ctx, reinterpret_cast<double *>(t));
+    dev_free(pl->ctx, pl->fused.prog_dev);
+    dev_free(pl->ctx, pl->fused.offtab_dev);
+    dev_free(pl->ctx, pl->mar_off_dev);
+    dev_free(pl->ctx, pl->obs_card_dev);
+    dev_free(pl->ctx, pl->ev_clean);
+    for (uint32_t *&t : pl->offtab_dev) dev_free(pl->ctx, t);
     delete pl;
     return BNPP_OK;
 }
@@ -2491,7 +2468,7 @@ static int run_dynamic(bnpp_ve_plan *pl, const std::vector<const double *> &ptr_
             os.rank = (int32_t)of.var.size();
             os.var_id = of.var.data();
             os.card = of.card.data();
-            rc = bnpp_alloc(ctx, of.size, &owned[st.out]);
+            rc = dev_alloc(ctx, of.size, &owned[st.out]);
             if (rc != BNPP_OK) break;
             dst = owned[st.out];
             ptr[st.out] = dst;
@@ -2504,13 +2481,9 @@ static int run_dynamic(bnpp_ve_plan *pl, const std::vector<const double *> &ptr_
             pl->step_kernel[s] = ctx->last_kernel;   // set by contract() below
         }
         for (int id : st.operands)
-            if (owned[id] && pl->f[id].last_use == (int)s) {
-                bnpp_free(ctx, owned[id]);
-                owned[id] = nullptr;
-            }
+            if (pl->f[id].last_use == (int)s) dev_free(ctx, owned[id]);
     }
-    for (double *p : owned)
-        if (p) bnpp_free(ctx, p);
+    for (double *&p : owned) dev_free(ctx, p);
     return rc;
 }
 
@@ -2520,10 +2493,8 @@ static int mpe_decode_prepare(bnpp_ve_plan *pl, const uint32_t *obs_val, double 
 {
     bnpp_ctx *ctx = pl->ctx;
     if (!pl->decode_rec_dev && !pl->decode_rec.empty()) {
-        double *store = nullptr;
-        int rc = bnpp_alloc(ctx, (pl->decode_rec.size() + 1) / 2, &store);
+        const int rc = dev_alloc(ctx, pl->decode_rec.size(), &pl->decode_rec_dev);
         if (rc != BNPP_OK) return rc;
-        pl->decode_rec_dev = reinterpret_cast<uint32_t *>(store);
         BNPP_CUDA(ctx, cudaMemcpyAsync(pl->decode_rec_dev, pl->decode_rec.data(), 4 * pl->decode_rec.size(),
                                        cudaMemcpyHostToDevice, ctx->stream));
     }
@@ -2541,15 +2512,44 @@ static int mpe_decode_prepare(bnpp_ve_plan *pl, const uint32_t *obs_val, double 
         for (uint32_t i = 0; i < p.n_obs; ++i) p.obs_val[i] = obs_val[i];
     } else {
         if (!pl->obs_val_dev) {
-            double *store = nullptr;
-            int rc = bnpp_alloc(ctx, (p.n_obs + 1) / 2, &store);
+            const int rc = dev_alloc(ctx, p.n_obs, &pl->obs_val_dev);
             if (rc != BNPP_OK) return rc;
-            pl->obs_val_dev = reinterpret_cast<uint32_t *>(store);
         }
         BNPP_CUDA(ctx, cudaMemcpyAsync(pl->obs_val_dev, obs_val, 4ull * p.n_obs, cudaMemcpyHostToDevice, ctx->stream));
         p.obs_val_dev = pl->obs_val_dev;
     }
     return BNPP_OK;
+}
+
+constexpr unsigned kDecodeThreads = 32;
+
+// the decode as a launch of its own; bnpp_last_launch keeps reporting the plan's last step
+static int decode_launch(bnpp_ve_plan *pl)
+{
+    bnpp_ctx *ctx = pl->ctx;
+    mpe_decode<<<1, kDecodeThreads, 0, ctx->stream>>>(pl->decode);
+    BNPP_CUDA(ctx, cudaGetLastError());
+    ctx->launches++;
+    return BNPP_OK;
+}
+
+// one kernel run of the replay graph: a new node after `prev` while the graph is being built (it becomes `prev`), else
+// the instantiated node's parameters set again
+static cudaError_t graph_node(bnpp_ve_plan *pl, cudaGraphNode_t &node, cudaGraphNode_t &prev, const void *fn, unsigned grid,
+                              unsigned block, unsigned smem, void *params)
+{
+    void *args[1] = {params};
+    cudaKernelNodeParams kp;
+    memset(&kp, 0, sizeof kp);
+    kp.func = const_cast<void *>(fn);
+    kp.gridDim = dim3(grid);
+    kp.blockDim = dim3(block);
+    kp.sharedMemBytes = smem;
+    kp.kernelParams = args;
+    if (pl->graph_exec) return cudaGraphExecKernelNodeSetParams(pl->graph_exec, node, &kp);
+    const cudaError_t e = cudaGraphAddKernelNode(&node, pl->graph, prev ? &prev : nullptr, prev ? 1 : 0, &kp);
+    prev = node;
+    return e;
 }
 
 static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uint32_t *obs_val, double *result_dev,
@@ -2628,10 +2628,8 @@ static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uin
     if (ev_inline && !pl->is_mpe) fused_g = fused_pick(pl, 1);
     if (pl->is_mpe) {
         if (!pl->arg_arena && pl->arg_bytes) {
-            double *store = nullptr;
-            rc = bnpp_alloc(ctx, (pl->arg_bytes + 7) / 8, &store);
+            rc = dev_alloc(ctx, pl->arg_bytes, &pl->arg_arena);
             if (rc != BNPP_OK) return rc;
-            pl->arg_arena = reinterpret_cast<uint8_t *>(store);
         }
         rc = mpe_decode_prepare(pl, obs_val, result_dev, assign_dev);
         if (rc != BNPP_OK) return rc;
@@ -2644,15 +2642,11 @@ static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uin
         rc = run_fused(pl, fused_g, tables_dev, 1, nullptr, obs_val, result_dev, z_dev);
     } else if (!pl->exec_ok || !aligned32) {
         rc = run_dynamic(pl, ptr, result_dev, z_dev);
-        if (rc == BNPP_OK && pl->is_mpe) {
-            mpe_decode<<<1, 32, 0, ctx->stream>>>(pl->decode);
-            BNPP_CUDA(ctx, cudaGetLastError());
-            ctx->launches++;
-        }
+        if (rc == BNPP_OK && pl->is_mpe) rc = decode_launch(pl);
     } else {
         if (!pl->arena && pl->arena_doubles) {
             const auto t_a0 = std::chrono::steady_clock::now();
-            rc = bnpp_alloc(ctx, pl->arena_doubles, &pl->arena);
+            rc = dev_alloc(ctx, pl->arena_doubles, &pl->arena);
             if (rc != BNPP_OK) return rc;
             if (getenv("BNPP_TIMING"))
                 fprintf(stderr, "bnpp timing: arena of %.1f MB allocated in %.3f ms\n", pl->arena_doubles * 8e-6,
@@ -2707,20 +2701,9 @@ static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uin
                 if (!(graphed && pl->use_graph)) {
                     rc = tasks_launch(ctx, g.launch, g.grid, g.smem);
                 } else if (changed) {
-                    void *args[1] = {&g.launch};
-                    cudaKernelNodeParams kp;
-                    memset(&kp, 0, sizeof kp);
-                    kp.func = const_cast<void *>(tasks_kernel());
-                    kp.gridDim = dim3(g.grid);
-                    kp.blockDim = dim3(kFusedThreads);
-                    kp.sharedMemBytes = g.smem;
-                    kp.kernelParams = args;
-                    cudaError_t e;
-                    if (fresh) e = cudaGraphAddKernelNode(&pl->nodes[s], pl->graph, prev ? &prev : nullptr, prev ? 1 : 0, &kp);
-                    else e = cudaGraphExecKernelNodeSetParams(pl->graph_exec, pl->nodes[s], &kp);
+                    const cudaError_t e = graph_node(pl, pl->nodes[s], prev, tasks_kernel(), g.grid, kFusedThreads, g.smem, &g.launch);
                     if (e != cudaSuccess) return cuda_fail(ctx, e, "CUDA graph node (tasks)");
                 }
-                if (fresh) prev = pl->nodes[s];
                 s = (size_t)g.b - 1;
                 continue;
             }
@@ -2744,27 +2727,12 @@ static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uin
                     for (int q = 0; q < now.lv[j].k; ++q) moved = moved || now.lv[j].s[q].p != w.p.lv[j].s[q].p;
                 w.p = now;
                 ++n_launched;
-                void *args[1] = {&w.p};
                 if (!(graphed && pl->use_graph)) {
-                    BNPP_CUDA(ctx, cudaLaunchKernel(w.fn, dim3(w.grid), dim3(kBlock), args, 0, ctx->stream));
-                    ctx->launches++;
-                    ctx->last_desc = nullptr;
-                    ctx->last_kernel = w.name;
-                    ctx->last_grid = w.grid;
-                    ctx->last_block = kBlock;
+                    rc = chain_launch(ctx, w.fn, w.grid, w.p, w.name);
                 } else if (moved) {
-                    cudaKernelNodeParams kp;
-                    memset(&kp, 0, sizeof kp);
-                    kp.func = const_cast<void *>(w.fn);
-                    kp.gridDim = dim3(w.grid);
-                    kp.blockDim = dim3(kBlock);
-                    kp.kernelParams = args;
-                    cudaError_t e;
-                    if (fresh) e = cudaGraphAddKernelNode(&pl->nodes[s], pl->graph, prev ? &prev : nullptr, prev ? 1 : 0, &kp);
-                    else e = cudaGraphExecKernelNodeSetParams(pl->graph_exec, pl->nodes[s], &kp);
+                    const cudaError_t e = graph_node(pl, pl->nodes[s], prev, w.fn, w.grid, kBlock, 0, &w.p);
                     if (e != cudaSuccess) return cuda_fail(ctx, e, "CUDA graph node (contract_chain)");
                 }
-                if (fresh) prev = pl->nodes[s];
                 s = (size_t)w.b - 1;
                 continue;
             }
@@ -2792,38 +2760,16 @@ static int run_plan(bnpp_ve_plan *pl, const double *const *tables_dev, const uin
             for (size_t q = 0; q < st.operands.size(); ++q) h.in[q] = in[q];
             h.out = dst;
             h.z = z;
-            void *args[1];
-            args[0] = d.params();
-            cudaKernelNodeParams kp;
-            memset(&kp, 0, sizeof kp);
-            kp.func = const_cast<void *>(d.fn);
-            kp.gridDim = dim3(d.grid);
-            kp.blockDim = dim3(kBlock);
-            kp.sharedMemBytes = d.smem;
-            kp.kernelParams = args;
-            cudaError_t e;
-            if (fresh) e = cudaGraphAddKernelNode(&pl->nodes[s], pl->graph, prev ? &prev : nullptr, prev ? 1 : 0, &kp);
-            else e = cudaGraphExecKernelNodeSetParams(pl->graph_exec, pl->nodes[s], &kp);
+            const cudaError_t e = graph_node(pl, pl->nodes[s], prev, d.fn, d.grid, kBlock, d.smem, d.params());
             if (e != cudaSuccess) return cuda_fail(ctx, e, "CUDA graph node");
-            if (fresh) prev = pl->nodes[s];
         }
         if (pl->is_mpe && rc == BNPP_OK) {
             ++n_launched;
             if (!(graphed && pl->use_graph)) {
-                mpe_decode<<<1, 32, 0, ctx->stream>>>(pl->decode);
-                BNPP_CUDA(ctx, cudaGetLastError());
-                ctx->launches++;
+                rc = decode_launch(pl);
             } else {
-                void *args[1] = {&pl->decode};
-                cudaKernelNodeParams kp;
-                memset(&kp, 0, sizeof kp);
-                kp.func = reinterpret_cast<void *>(mpe_decode);
-                kp.gridDim = dim3(1);
-                kp.blockDim = dim3(32);
-                kp.kernelParams = args;
-                cudaError_t e;
-                if (fresh) e = cudaGraphAddKernelNode(&pl->decode_node, pl->graph, prev ? &prev : nullptr, prev ? 1 : 0, &kp);
-                else e = cudaGraphExecKernelNodeSetParams(pl->graph_exec, pl->decode_node, &kp);
+                const cudaError_t e = graph_node(pl, pl->decode_node, prev, reinterpret_cast<const void *>(mpe_decode), 1,
+                                                 kDecodeThreads, 0, &pl->decode);
                 if (e != cudaSuccess) return cuda_fail(ctx, e, "CUDA graph node (MPE decode)");
             }
         }
@@ -2902,22 +2848,17 @@ static int mpe_batch_prepare(bnpp_ve_plan *pl, uint32_t slice)
 {
     bnpp_ctx *ctx = pl->ctx;
     if (!pl->batch_rec_dev && !pl->batch_rec.empty()) {
-        double *store = nullptr;
-        const int rc = bnpp_alloc(ctx, (pl->batch_rec.size() + 1) / 2, &store);
+        const int rc = dev_alloc(ctx, pl->batch_rec.size(), &pl->batch_rec_dev);
         if (rc != BNPP_OK) return rc;
-        pl->batch_rec_dev = reinterpret_cast<uint32_t *>(store);
         BNPP_CUDA(ctx, cudaMemcpyAsync(pl->batch_rec_dev, pl->batch_rec.data(), 4 * pl->batch_rec.size(), cudaMemcpyHostToDevice,
                                        ctx->stream));
     }
     const uint64_t need = pl->arg_rows * slice;
     if (need > pl->batch_arg_bytes) {
-        if (pl->batch_arg) bnpp_free(ctx, reinterpret_cast<double *>(pl->batch_arg));
-        pl->batch_arg = nullptr;
+        dev_free(ctx, pl->batch_arg);
         pl->batch_arg_bytes = 0;
-        double *store = nullptr;
-        const int rc = bnpp_alloc(ctx, (need + 7) / 8, &store);
+        const int rc = dev_alloc(ctx, need, &pl->batch_arg);
         if (rc != BNPP_OK) return rc;
-        pl->batch_arg = reinterpret_cast<uint8_t *>(store);
         pl->batch_arg_bytes = need;
     }
     return BNPP_OK;
@@ -2958,10 +2899,8 @@ static int run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32
     if ((int)n_obs != pl->n_obs) return fail(ctx, BNPP_EINVAL, "batched VE: n_obs differs from the plan's");
     if (n_obs && !ev_dev) return fail(ctx, BNPP_EINVAL, "batched VE: evidence matrix missing");
     if (n_obs && !pl->obs_card_dev) {
-        double *store = nullptr;
-        const int rc = bnpp_alloc(ctx, n_obs / 2 + 2, &store);
+        const int rc = dev_alloc(ctx, n_obs + 4, &pl->obs_card_dev);
         if (rc != BNPP_OK) return rc;
-        pl->obs_card_dev = reinterpret_cast<uint32_t *>(store);
         std::vector<uint32_t> c(pl->obs_card);
         for (uint32_t &v : c)
             if (!v) v = 256;        // a variable no factor mentions: any byte is harmless
@@ -2976,11 +2915,9 @@ static int run_batched(bnpp_ve_plan *pl, const double *const *tables_dev, uint32
             if (n_obs) {
                 const uint64_t need = (uint64_t)nb * n_obs;
                 if (pl->ev_clean_bytes < need) {
-                    if (pl->ev_clean) bnpp_free(ctx, reinterpret_cast<double *>(pl->ev_clean));
-                    double *store = nullptr;
-                    const int rc = bnpp_alloc(ctx, need / 8 + 2, &store);
+                    dev_free(ctx, pl->ev_clean);
+                    const int rc = dev_alloc(ctx, need + 16, &pl->ev_clean);
                     if (rc != BNPP_OK) return rc;
-                    pl->ev_clean = reinterpret_cast<uint8_t *>(store);
                     pl->ev_clean_bytes = need;
                 }
                 const int rc = sanitize_evidence_launch(ctx, ev_dev, pl->ev_clean, nb, n_obs, pl->obs_card_dev, false);
@@ -3083,10 +3020,9 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
         for (uint32_t d = 0; d == 0 || (d < 4 && (max_base >> (8 * d))); ++d) digit_obs[i].push_back({1ll << (8 * d), (int)n_cols++});
     }
     // evidence columns contiguous over the sets: every thread of a warp then reads neighbouring bytes
-    double *evt_store = nullptr;
-    rc = bnpp_alloc(ctx, ((uint64_t)nb * (n_cols ? n_cols : 1) + 7) / 8 + 1, &evt_store);
+    uint8_t *evt = nullptr;
+    rc = dev_alloc(ctx, (uint64_t)nb * (n_cols ? n_cols : 1) + 8, &evt);
     if (rc != BNPP_OK) return rc;
-    uint8_t *evt = reinterpret_cast<uint8_t *>(evt_store);
     if (pl->offtab_host.size() != pl->steps.size()) {
         pl->offtab_host.assign(pl->steps.size(), std::vector<uint32_t>());
         pl->offtab_dev.assign(pl->steps.size(), nullptr);
@@ -3122,7 +3058,7 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
                 const PlanFactor &of = pl->f[st.out];
                 ov = &of.var;
                 oc = &of.card;
-                rc = bnpp_alloc(ctx, of.size * cur, &owned[st.out]);
+                rc = dev_alloc(ctx, of.size * cur, &owned[st.out]);
                 if (rc != BNPP_OK) break;
                 dst = owned[st.out];
             }
@@ -3130,17 +3066,13 @@ static int run_batched_once(bnpp_ve_plan *pl, const double *const *tables_dev, u
             rc = contract_batched_step(ctx, (int)st.operands.size(), ops, *ov, *oc, st.elim, cur, evt + b0, nb, n_cols, dst,
                                        &pl->offtab_host[s], &pl->offtab_dev[s], arg);
             for (int id : st.operands)
-                if (owned[id] && pl->f[id].last_use == (int)s) {
-                    bnpp_free(ctx, owned[id]);
-                    owned[id] = nullptr;
-                }
+                if (pl->f[id].last_use == (int)s) dev_free(ctx, owned[id]);
         }
-        for (double *p : owned)
-            if (p) bnpp_free(ctx, p);
+        for (double *&p : owned) dev_free(ctx, p);
         if (!pl->is_mar && (pl->steps.empty() || pl->steps.back().out != -2)) rc = fill(ctx, result_dev + b0, cur, 1.0);
         if (rc == BNPP_OK && assign_dev) rc = mpe_decode_batch_launch(pl, nb, b0, cur, evt + b0, nb, 1, assign_dev);
     }
-    bnpp_free(ctx, evt_store);
+    dev_free(ctx, evt);
     // inside the run, hence inside its captured graph: a replay normalises too
     if (rc == BNPP_OK && pl->is_mar && pl->normalize)
         rc = normalize_segments_batched(ctx, result_dev, pl->mar_off_dev, pl->mar_size_dev, (int)pl->mar_off.size(), nb);
